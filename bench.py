@@ -1,7 +1,11 @@
 """bench.py -- rollout env-steps/s and CEM-iteration latency of the B200-native CEM planner.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--global-batch G]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--global-batch G] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step returned (the new mean and covariance, the per-sample costs, thetadot
+and theta) as DIR/<name>.npy in float32.  The inputs are fixed constants and PRNGKey(0), so two builds run with the same
+arguments can be compared array for array.
 
 One "step" = one full CEM iteration of the planner hot path (sample -> projection filter ->
 Bernstein evaluation -> T-step rollout of every sample -> cost -> elite top-k [+ NCCL all-gather
@@ -203,6 +207,28 @@ def cpu_baseline_record():
 
 
 # ---------------------------------------------------------------------------------------------- GPU arm
+DUMP_BYTES = 60 * 10 ** 6          # array data of --dump-outputs: under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, whole, per_sample):
+    """Write `whole` and `per_sample` (name -> numpy array; the latter with one row per sample) as out_dir/<name>.npy.  When
+    they exceed DUMP_BYTES, only a fixed, seeded subset of the sample rows is written, and its row indices as sample_rows.npy.
+    Returns {name: shape} of what was written."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = dict(whole)
+    n = len(next(iter(per_sample.values())))
+    row_bytes = sum(a.nbytes for a in per_sample.values()) // n
+    room = DUMP_BYTES - sum(a.nbytes for a in whole.values())
+    if row_bytes * n > room:
+        rows = np.sort(np.random.default_rng(0).choice(n, room // (row_bytes + 8), replace=False))
+        per_sample = {k: a[rows] for k, a in per_sample.items()}
+        out["sample_rows"] = rows.astype(np.float64)
+    out.update(per_sample)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    return {k: list(a.shape) for k, a in out.items()}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -213,7 +239,11 @@ def main():
     ap.add_argument("--global-batch", type=int, default=0, help="strong scaling: this many samples over all GPUs (BASELINE config 5: 65536)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config5", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (rank 0's samples when sharded; --impl ours only)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs is not None:
+        ap.error("--dump-outputs writes the outputs of --impl ours; the reference arm has none to write")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -255,24 +285,30 @@ def main():
         return [float(v) for v in out.cpu()]
 
     def timed(fn, k):
-        evs = []
-        for _ in range(k):
+        """Event times of k calls of fn, and what the last call returned (earlier results are dropped at once, so the
+        allocator sees the same pattern in every step)."""
+        evs, last = [], None
+        for i in range(k):
             flush.fill_(1.0)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            fn()
+            if i == k - 1:
+                last = fn()
+            else:
+                fn()
             b.record()
             evs.append((a, b))
         torch.cuda.synchronize(dev)
-        return [a.elapsed_time(b) for a, b in evs]
+        return [a.elapsed_time(b) for a, b in evs], last
 
     z6 = torch.zeros(6, device=dev)
     q0 = torch.as_tensor(Q0, dtype=torch.float32, device=dev)
     tp = torch.as_tensor(TP, dtype=torch.float32, device=dev)
     tr = torch.as_tensor(TR, dtype=torch.float32, device=dev)
 
-    def measure(Bg, with_e2e, with_kernel):
-        """Device-resident CEM iteration (+ optionally the public-API tick and the rollout kernel alone) at global batch Bg."""
+    def measure(Bg, with_e2e, with_kernel, with_outputs=False):
+        """Device-resident CEM iteration (+ optionally the public-API tick and the rollout kernel alone) at global batch Bg.
+        with_outputs: also return, on the host, what the last timed iteration computed."""
         Bl = Bg // world
         with contextlib.redirect_stdout(io.StringIO()):
             pl = cem_planner(num_dof=6, num_batch=Bg, num_steps=T, timestep=DT, maxiter_cem=1, num_elite=ELITE, w_pos=W_POS, w_rot=W_ROT,
@@ -293,9 +329,16 @@ def main():
             device_step()
         barrier()
         l0 = lib.cemk_launch_count(h)
-        ms = timed(device_step, args.steps)
+        ms, last = timed(device_step, args.steps)
         barrier()
         res = {"pl": pl, "Bl": Bl, "launches": lib.cemk_launch_count(h) - l0, "ms_all": [round(v, 4) for v in ms]}
+        if with_outputs:
+            carry, (cost, cost_g, cost_r, cost_c, thetadot, theta) = last
+            host = lambda t: t.detach().float().cpu().numpy()
+            res["outputs"] = ({"xi_mean": host(carry[4]), "xi_cov": host(carry[5])},
+                              {n: host(t) for n, t in (("cost", cost), ("cost_g", cost_g), ("cost_r", cost_r), ("cost_c", cost_c),
+                                                       ("thetadot", thetadot), ("theta", theta))})
+        del last
         res["tot_ms"] = max_over_ranks(sum(ms))
         res["value"] = Bg * T * args.steps / (res["tot_ms"] * 1e-3)
         if with_e2e:
@@ -327,7 +370,7 @@ def main():
 
             for _ in range(2):
                 rollout_only()
-            res["roll_ms"] = float(np.mean(timed(rollout_only, max(3, args.steps))))
+            res["roll_ms"] = float(np.mean(timed(rollout_only, args.steps)[0]))
             res["roll_ms_by_rank"] = all_ranks(res["roll_ms"])
             # this rank's own event time per iteration (includes its wait inside the all-gather for the slowest rank)
             res["iter_ms_by_rank"] = all_ranks(sum(ms) / args.steps)
@@ -339,7 +382,7 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    main_res = measure(Bg_main, True, True)
+    main_res = measure(Bg_main, True, True, with_outputs=args.dump_outputs is not None and rank == 0)
     c5 = None
     if not args.no_config5 and args.global_batch == 0 and B_CONFIG5 % world == 0:
         c5 = measure(B_CONFIG5, False, False)
@@ -419,6 +462,8 @@ def main():
                            "ms_per_step": c5["tot_ms"] / args.steps, "scaling": "strong", "gpu_launches": int(c5["launches"])}
     if not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_baseline_record()
+    if args.dump_outputs is not None:
+        line["dumped_outputs"] = dump_outputs(args.dump_outputs, *main_res["outputs"])
     print(json.dumps(line))
     shutdown()
 

@@ -1,7 +1,7 @@
 """Ready-made hook for the day a real MJX oracle is available (SURVEY.md section 8c).
 
 `mujoco`, `mujoco.mjx` and `jax` cannot be installed in this environment, so every test here is
-skipped; with them importable (and the reference checkout at /root/reference) the tests compare
+skipped; with them importable (and MANIPULATOR_MUJOCO_REFERENCE naming a checkout of the upstream project) the tests compare
   * the MJCF compiler's constants against `mujoco.MjModel`,
   * the C oracle's rollout against `jax.vmap(lax.scan(mjx.step))` exactly as the reference planner
     builds it (mjx_planner.py:251-274),
@@ -15,8 +15,10 @@ mujoco = pytest.importorskip("mujoco")
 jax = pytest.importorskip("jax")
 mjx = pytest.importorskip("mujoco.mjx")
 
-REF_XML = "/root/reference/sampling_based_planner/ur5e_hande_mjx/scene.xml"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_XML), reason="reference checkout not present")
+REFERENCE = os.environ.get("MANIPULATOR_MUJOCO_REFERENCE", "")
+REF_XML = os.path.join(REFERENCE, "sampling_based_planner", "ur5e_hande_mjx", "scene.xml")
+pytestmark = pytest.mark.skipif(not REFERENCE or not os.path.exists(REF_XML),
+                                reason="needs the upstream checkout named by MANIPULATOR_MUJOCO_REFERENCE")
 
 
 @pytest.fixture(scope="module")

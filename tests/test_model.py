@@ -11,7 +11,11 @@ from manipulator_mujoco_b200 import kmodel as KM
 from manipulator_mujoco_b200.mjcf import compile_mjcf, host_kinematics, host_mass_matrix
 
 IDS = json.load(open(os.path.join(GOLDEN, "scene_ids.json")))
-REF_XML = "/root/reference/sampling_based_planner/ur5e_hande_mjx/scene.xml"
+# checkout of the upstream project alinjar1996/manipulator_mujoco: its MJCF files are not part of this repository, so the
+# tests that compile them run only where MANIPULATOR_MUJOCO_REFERENCE names such a checkout
+REFERENCE = os.environ.get("MANIPULATOR_MUJOCO_REFERENCE", "")
+REF_XML = os.path.join(REFERENCE, "sampling_based_planner", "ur5e_hande_mjx", "scene.xml")
+NO_REFERENCE = "needs the upstream checkout named by MANIPULATOR_MUJOCO_REFERENCE"
 
 
 def test_counts_and_ids(mc):
@@ -35,7 +39,7 @@ def test_forward_kinematics_pins(mc):
     np.testing.assert_allclose(xquat[mc.body_id("hande")], IDS["xquat_hande_at_init_pos"], atol=1e-5)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_XML), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not REFERENCE or not os.path.exists(REF_XML), reason=NO_REFERENCE)
 def test_packaged_constants_match_the_xml(mc):
     fresh = compile_mjcf(REF_XML)
     for k, v in fresh.d.items():
@@ -186,11 +190,11 @@ def test_from_mjmodel_reproduces_the_compiled_model(mc):
     np.testing.assert_allclose(a, b, rtol=0, atol=1e-6)
 
 
-SCENE_B = "/root/reference/universal_robots_ur5e/scene_mjx.xml"
-DUAL_ARM = "/root/reference/universal_robots_ur5e/dual_arm_scene.xml"
+SCENE_B = os.path.join(REFERENCE, "universal_robots_ur5e", "scene_mjx.xml")
+DUAL_ARM = os.path.join(REFERENCE, "universal_robots_ur5e", "dual_arm_scene.xml")
 
 
-@pytest.mark.skipif(not os.path.exists(SCENE_B), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not REFERENCE or not os.path.exists(SCENE_B), reason=NO_REFERENCE)
 def test_scene_b_loads_with_the_counts_of_the_survey(tmp_path):
     """universal_robots_ur5e/scene_mjx.xml (the file BASELINE.json names; the planner itself loads scene A): slide joints of the
     two Hand-E fingers, their joint equality and fixed tendon, two contact excludes, one free box.  Counts: SURVEY.md A.3."""
@@ -236,7 +240,7 @@ def test_scene_b_loads_with_the_counts_of_the_survey(tmp_path):
         KM.build_kmodel(mb, 0.05)
 
 
-@pytest.mark.skipif(not os.path.exists(DUAL_ARM), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not REFERENCE or not os.path.exists(DUAL_ARM), reason=NO_REFERENCE)
 def test_dual_arm_scene_loads_and_is_refused_by_the_kernel():
     """universal_robots_ur5e/dual_arm_scene.xml (BASELINE config 4, an extension: the reference planner cannot load it either,
     SURVEY.md finding 0.4 / A.4): 12 hinges, 12 position servos, implicitfast, cylinder end-effector geoms, keyframe `home`."""

@@ -1,7 +1,7 @@
 """Generate the committed golden fixtures under tests/golden/ from the reference checkout.
 
-Run in the build container (needs /root/reference; the GPU box never reads it):
-    python tools/make_golden.py
+Needs a checkout of the upstream project alinjar1996/manipulator_mujoco; the tests only read what this writes:
+    MANIPULATOR_MUJOCO_REFERENCE=<checkout> python tools/make_golden.py
 Produces
   bernstein.npz        P, Pdot, Pddot of the reference's own bernstein_coeff_ordern_new for the
                        horizons used by the tests (imported from the reference, not restated);
@@ -17,7 +17,7 @@ import sys
 
 import numpy as np
 
-REF = "/root/reference/sampling_based_planner"
+REF = os.path.join(os.environ["MANIPULATOR_MUJOCO_REFERENCE"], "sampling_based_planner")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden")
 
 
