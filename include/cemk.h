@@ -11,7 +11,12 @@
  *     reference method), kernels are enqueued on `stream` (a cudaStream_t passed as void*) and the
  *     call returns without synchronising;
  *   - one handle per device, not thread-safe per handle;
- *   - B = num_batch (samples on this GPU), T = num_steps, NV = 66 = num_dof(6) * 11 coefficients.
+ *   - B = num_batch (samples on this GPU), T = num_steps, nd = num_dof (cemk_set_dof, default 6),
+ *     nc = Bernstein coefficients per DOF (cemk_set_order, default 11), NV = nvar = nd * nc decision variables.
+ *     "66", "30" and "6T" in the shapes below are NV, 5 nd and nd T at the defaults.
+ *   - The planner algebra (sampling, projection, elite selection, mean / covariance) runs at any
+ *     1 <= nd <= 12 and 4 <= nc <= 16 (NV <= 192).  The rollout (cemk_rollout_cost, cemk_tick_record)
+ *     models the 6-DOF arm of the KModel only and returns CEMK_ERR_ARG on a handle with nd != 6.
  */
 #ifndef CEMK_H
 #define CEMK_H
@@ -40,8 +45,12 @@ int cemk_destroy(cemk_handle* h);
 /* Update the rollout snapshot (qpos0 / warm0 / qvel0 of the KModel) after construction. */
 int cemk_set_model(cemk_handle* h, const void* kmodel, int kmodel_bytes);
 
+/* Degrees of freedom of the planner algebra, 1 <= nd <= 12 (cem_planner(num_dof=nd); default 6, the UR5e of the KModel).
+ * nvar = nd nc.  Call before cemk_set_horizon (it discards the horizon tables). */
+int cemk_set_dof(cemk_handle* h, int ndof);
+
 /* Bernstein coefficients per DOF, nc = order + 1 (mjx_planner.py:40 calls bernstein_coeff_ordern_new(10, ...), i.e. nc = 11, the
- * default; SURVEY.md 8 f.4: arbitrary order n).  4 <= nc <= 16; nvar = 6 nc is the width of every xi / mean / cov / elite array
+ * default; SURVEY.md 8 f.4: arbitrary order n).  4 <= nc <= 16; nvar = nd nc is the width of every xi / mean / cov / elite array
  * below ("66" in their descriptions is the default nvar).  Call before cemk_set_horizon (it discards the horizon tables). */
 int cemk_set_order(cemk_handle* h, int ncoef);
 
@@ -64,7 +73,7 @@ int cemk_jax_normal(cemk_handle* h, unsigned key0, unsigned key1, int original, 
                     unsigned count, float* out, void* stream);
 
 /* compute_projection_filter (mjx_planner.py:234-249) + Bernstein evaluation (mjx_planner.py:348):
- *   xi[B][66], state_term[B][30] -> xi_f[B][66]; thetadot[B][6*T] (index dof*T + t) when non-null. */
+ *   xi[B][NV], state_term[B][5 nd] -> xi_f[B][NV]; thetadot[B][nd*T] (index dof*T + t) when non-null. */
 int cemk_project(cemk_handle* h, int B, int maxiter_projection, const float* xi, const float* state_term, float* xi_f,
                  float* thetadot, void* stream);
 

@@ -40,6 +40,7 @@ _SIGS = {
     "cemk_create": ([_vp, _i, _i, C.POINTER(_vp)], _i),
     "cemk_destroy": ([_vp], _i),
     "cemk_set_model": ([_vp, _vp, _i], _i),
+    "cemk_set_dof": ([_vp, _i], _i),
     "cemk_set_order": ([_vp, _i], _i),
     "cemk_set_horizon": ([_vp, _i, _vp, _vp, _vp, _vp], _i),
     "cemk_sample": ([_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp], _i),

@@ -1,13 +1,13 @@
 // cemk.cu -- sm_100a kernels + the C ABI declared in include/cemk.h.
 //
 // Kernels (one per stage of cem_planner.cem_iter, reference mjx_planner.py:337-362):
-//   k_jax_normal / k_chol66 / k_sample            compute_xi_samples       (:313-316)
+//   k_jax_normal / k_chol66 | k_chol_wide / k_sample   compute_xi_samples  (:313-316)
 //   k_project                compute_projection_filter + A_thetadot @ xi   (:181-249, :348)
 //   k_rollout                vmap(scan(mjx.step)) + compute_cost_batch     (:251-303)   <- hot kernel
 //   k_cost_batch             compute_cost_batch on materialised trajectories (:277-303)
 //   k_rank_select (n <= 8192) | k_make_keys / k_bitonic* / k_finish_sort / k_pack_sorted     compute_ellite_samples   (:306-310)
 //   k_merge_lists            the same selection over the per-rank sorted lists of several GPUs
-//   k_mean_cov | k_mc_partial + k_mc_finish (k >= 1024)                    compute_mean_cov (:326-335)
+//   k_mean_cov | k_mc_partial[_wide] + k_mc_finish (k >= 1024)             compute_mean_cov (:326-335)
 //   k_tick_record            what compute_cem keeps of an iteration        (:390-404)
 // The rollout core lives in rollout_core.h (shared with the CPU emulation used by the no-GPU tests).
 #include <cuda_runtime.h>
@@ -19,10 +19,12 @@
 #include "rollout_core.h"
 
 // Bernstein order n (mjx_planner.py:40 hard-codes 10; SURVEY 8 f.4 asks for order n): ncoef = n + 1 coefficients per DOF,
-// nvar = 6 ncoef decision variables, chosen per handle by cemk_set_order (default 11 / 66).
+// nvar = ndof ncoef decision variables, chosen per handle by cemk_set_dof / cemk_set_order (default 6 DOF x 11 = 66).  The
+// planner algebra runs at any ndof <= MAXDOF; the rollout models the 6-DOF (KM_NL) arm only.
 #define MINCOEF 4
 #define MAXCOEF 16
-#define MAXVAR (KM_NL * MAXCOEF)
+#define MAXDOF 12
+#define MAXVAR (MAXDOF * MAXCOEF)      // 192
 #ifndef ROLLOUT_WARPS
 #define ROLLOUT_WARPS 14      // warps per CTA (28 samples with two samples per warp: all the shared memory of an SM); they
                               // step in lockstep (STEP_ALIGN) to share the instruction cache
@@ -55,7 +57,7 @@ struct DevGuard {
 struct cemk_handle {
   int device;
   KModel* d_model;
-  int ncoef, nvar;                 // Bernstein coefficients per DOF, decision variables (6 ncoef)
+  int ndof, ncoef, nvar;           // DOF of the planner algebra, Bernstein coefficients per DOF, decision variables (ndof ncoef)
   int T;
   float* d_G;      // [3][T][11]
   float* d_K;      // Kpp[ncoef^2] Kpe[ncoef*5] bounds[3]
@@ -169,12 +171,14 @@ static_assert(((sizeof(KModel) + 15) & ~size_t(15)) + ROLLOUT_WARPS * GPW * size
 // one pass applies the panel's CHOL_NB updates to every trailing element -- the same operations on the same operands in
 // the same order per element as the column-at-a-time loop (bit-identical, 33 us), with the long per-column trailing
 // sweep off the barrier chain.  (A left-looking variant with four lanes per row dot product was slower: 43 us.)
+// N = largest n of the instantiation: k_chol66 (n <= 96, the matrix in static shared memory) and k_chol_wide (n <= 192, the
+// matrix in dynamic shared memory: 148 KB at 192).  Both run this body with the same operations in the same order.
 #define CHOL_NB 8
-#define CHOL_KU ((MAXVAR + 15) / 16)
-static_assert(CHOL_NB == 8, "k_chol66 deals the panel columns with threadIdx.x & 7");
-__global__ void __launch_bounds__(256) k_chol66(int n, const float* __restrict__ cov, float* __restrict__ L) {
-  __shared__ float A[MAXVAR][MAXVAR + 1];
-  __shared__ float P[MAXVAR];
+#define CHOL_SMALL_N 96
+static_assert(CHOL_NB == 8, "chol_body deals the panel columns with threadIdx.x & 7");
+template <int N>
+__device__ __forceinline__ void chol_body(int n, const float* __restrict__ cov, float* __restrict__ L, float (*A)[N + 1], float* P) {
+  constexpr int KU = (N + 15) / 16, RM = (N + 31) / 32;   // trailing elements of a row per thread; panel rows per thread
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   for (int i = ty; i < n; i += 16)
     for (int j = tx; j < n; j += 16) A[i][j] = cov[i * n + j] + (i == j ? 0.003f : 0.f);
@@ -183,13 +187,13 @@ __global__ void __launch_bounds__(256) k_chol66(int n, const float* __restrict__
   for (int j0 = 0; j0 < n - 1; j0 += CHOL_NB) {
     const int je = j0 + CHOL_NB < n ? j0 + CHOL_NB : n;
     for (int j = j0; j < je && j < n - 1; ++j) {
-      // every load of the step is issued before the first dependent instruction (rows i0, i0 + 32, i0 + 64)
+      // every load of the step is issued before the first dependent instruction (rows i0, i0 + 32, ...)
       const int k = j + 1 + pc, i0 = j + 1 + pr;
       const bool kon = k < je;
       const float ajj = A[j][j], akj = kon ? A[k][j] : 0.f;
-      float aij[3], aik[3]; bool on[3];
+      float aij[RM], aik[RM]; bool on[RM];
 #pragma unroll
-      for (int m = 0; m < 3; ++m) {
+      for (int m = 0; m < RM; ++m) {
         const int i = i0 + 32 * m;
         on[m] = kon && i < n && k <= i;
         aij[m] = on[m] ? A[i][j] : 0.f; aik[m] = on[m] ? A[i][k] : 0.f;
@@ -198,7 +202,7 @@ __global__ void __launch_bounds__(256) k_chol66(int n, const float* __restrict__
                                                          //  kernels spell out IEEE division / sqrt / exp so the flag does not touch them)
       if (threadIdx.x == 0) P[j] = p;
 #pragma unroll
-      for (int m = 0; m < 3; ++m) {
+      for (int m = 0; m < RM; ++m) {
         const float s = aij[m] * p;
         aik[m] -= s * akj;
         if (on[m]) A[i0 + 32 * m][k] = aik[m];
@@ -213,10 +217,10 @@ __global__ void __launch_bounds__(256) k_chol66(int n, const float* __restrict__
         float ai[CHOL_NB];
 #pragma unroll
         for (int q = 0; q < CHOL_NB; ++q) ai[q] = A[i][j0 + q] * pp[q];
-        // up to CHOL_KU elements of row i per thread, their CHOL_NB-long chains interleaved
-        float a[CHOL_KU], ak[CHOL_KU][CHOL_NB]; bool on[CHOL_KU];
+        // up to KU elements of row i per thread, their CHOL_NB-long chains interleaved
+        float a[KU], ak[KU][CHOL_NB]; bool on[KU];
 #pragma unroll
-        for (int u = 0; u < CHOL_KU; ++u) {
+        for (int u = 0; u < KU; ++u) {
           const int k = je + tx + 16 * u;
           on[u] = k <= i;
           a[u] = on[u] ? A[i][k] : 0.f;
@@ -226,9 +230,9 @@ __global__ void __launch_bounds__(256) k_chol66(int n, const float* __restrict__
 #pragma unroll
         for (int q = 0; q < CHOL_NB; ++q)
 #pragma unroll
-          for (int u = 0; u < CHOL_KU; ++u) a[u] -= ai[q] * ak[u][q];
+          for (int u = 0; u < KU; ++u) a[u] -= ai[q] * ak[u][q];
 #pragma unroll
-        for (int u = 0; u < CHOL_KU; ++u) if (on[u]) A[i][je + tx + 16 * u] = a[u];
+        for (int u = 0; u < KU; ++u) if (on[u]) A[i][je + tx + 16 * u] = a[u];
       }
     }
     __syncthreads();
@@ -239,6 +243,16 @@ __global__ void __launch_bounds__(256) k_chol66(int n, const float* __restrict__
       L[i * n + j] = j > i ? 0.f : (i == j ? d : __fdiv_rn(A[i][j], d));
     }
 }
+__global__ void __launch_bounds__(256) k_chol66(int n, const float* __restrict__ cov, float* __restrict__ L) {
+  __shared__ float A[CHOL_SMALL_N][CHOL_SMALL_N + 1];
+  __shared__ float P[CHOL_SMALL_N];
+  chol_body<CHOL_SMALL_N>(n, cov, L, A, P);
+}
+__global__ void __launch_bounds__(256) k_chol_wide(int n, const float* __restrict__ cov, float* __restrict__ L) {
+  extern __shared__ float chol_sm[];                     // A[MAXVAR][MAXVAR + 1], P[MAXVAR]
+  chol_body<MAXVAR>(n, cov, L, reinterpret_cast<float (*)[MAXVAR + 1]>(chol_sm), chol_sm + MAXVAR * (MAXVAR + 1));
+}
+static size_t chol_wide_smem() { return sizeof(float) * ((size_t)MAXVAR * (MAXVAR + 1) + MAXVAR); }
 // xi[b][i] = mean[i] + sum_{j<=i} L[i][j] z[b][j] (the sum runs j = 0 .. i in this order).  One CTA per SAMPLE_TILE
 // consecutive samples: L and the tile's draws in shared memory, a warp works on one row i for different samples (L[i][j]
 // is a broadcast, the triangular trip count is uniform in the warp), results leave through a shared tile so that the
@@ -372,13 +386,16 @@ constexpr int kProjUnroll = PROJ_UNROLL;
 #define PROJ_MINB 3
 #endif
 // NC = Bernstein coefficients per DOF (order + 1), a template parameter so that the iterates stay in registers; a basis
-// row is padded to PC = 4 ceil(NC / 4) floats.
-template <int NC>
-__global__ void __launch_bounds__(32 * PROJ_WARPS, NC <= 11 ? PROJ_MINB : 1) k_project(int B, int T, int iters, const float* __restrict__ G,
+// row is padded to PC = 4 ceil(NC / 4) floats.  nd = DOF per sample: B nd problems, xi / xi_f rows of nd NC, state_term rows of
+// 5 nd, thetadot rows of nd T.  ND = KM_NL fixes it at compile time (the product path, the code the 6-DOF build always had);
+// ND = 0 takes it from `ndof` at run time (any other DOF count; the per-problem arithmetic is the same).
+template <int NC, int ND>
+__global__ void __launch_bounds__(32 * PROJ_WARPS, NC <= 11 ? PROJ_MINB : 1) k_project(int B, int ndof, int T, int iters, const float* __restrict__ G,
                                                               const float* __restrict__ Kc, const float* __restrict__ xi,
                                                               const float* __restrict__ state_term, float* __restrict__ xi_f,
                                                               float* __restrict__ thetadot) {
-  constexpr int PC = (NC + 3) / 4 * 4, NV = KM_NL * NC, KPAD = (5 * NC + 3 + 3) / 4 * 4;
+  constexpr int PC = (NC + 3) / 4 * 4, KPAD = (5 * NC + 3 + 3) / 4 * 4;
+  const int nd = ND ? ND : ndof, NV = nd * NC;
   extern __shared__ __align__(16) float sm[];
   float* sG = sm;                        // [3][T][PC]
   float* sKpp = sm + 3 * T * PC;         // [NC][PC]
@@ -400,9 +417,9 @@ __global__ void __launch_bounds__(32 * PROJ_WARPS, NC <= 11 ? PROJ_MINB : 1) k_p
 #define PROJ_SRC(q) ((lane & ~(PROJ_SLICES - 1)) | (q))
 #endif
   int prob = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * PROJ_PPW + pl;
-  const bool act = prob < B * 6;         // idle lanes still take part in the shuffles
-  if (!act) prob = B * 6 - 1;
-  const int b = prob / 6, d = prob % 6;
+  const bool act = prob < B * nd;        // idle lanes still take part in the shuffles
+  if (!act) prob = B * nd - 1;
+  const int b = prob / nd, d = prob % nd;
   const float* Kpe = sK; const float* bnd = sK + 5 * NC;
   float* myxs = sP + threadIdx.x;
   float* mycst = sP + NC * blockDim.x + threadIdx.x;
@@ -424,7 +441,7 @@ __global__ void __launch_bounds__(32 * PROJ_WARPS, NC <= 11 ? PROJ_MINB : 1) k_p
 #pragma unroll
     for (int k = 0; k < NC; ++k) { myxs[k * cs] = xi[(size_t)b * NV + d * NC + k]; mylam[k * cs] = 0.f; x[k] = 0.f; rh[k] = 0.f; }
 #pragma unroll
-    for (int k = 0; k < 5; ++k) beq[k] = state_term[(size_t)b * 30 + k * 6 + d];
+    for (int k = 0; k < 5; ++k) beq[k] = state_term[(size_t)b * 5 * nd + k * nd + d];
 #pragma unroll
     for (int i = 0; i < NC; ++i) { float s = 0.f; for (int k = 0; k < 5; ++k) s += Kpe[i * 5 + k] * beq[k]; mycst[i * cs] = s; }
   }
@@ -470,7 +487,7 @@ __global__ void __launch_bounds__(32 * PROJ_WARPS, NC <= 11 ? PROJ_MINB : 1) k_p
   }
   if (thetadot) {
     const float* Gv = sG;    // Pdot
-    float* out = thetadot + (size_t)b * 6 * T + (size_t)d * T;
+    float* out = thetadot + (size_t)b * nd * T + (size_t)d * T;
     for (int t = slice; t < T; t += PROJ_SLICES) {
       float g[NC];
       rowp(Gv + t * PC, g);
@@ -486,9 +503,9 @@ static int project_smem(int T, int threads) {
   constexpr int PC = (NC + 3) / 4 * 4, KPAD = (5 * NC + 3 + 3) / 4 * 4;
   return (3 * T * PC + NC * PC + KPAD + 3 * NC * threads) * (int)sizeof(float);
 }
-// warps per CTA: PROJ_WARPS when the problems fill the GPU, fewer (more CTAs) for small batches
-static int project_warps(int B) {
-  const int warps = (B * 6 + PROJ_PPW - 1) / PROJ_PPW;
+// warps per CTA: PROJ_WARPS when the nprob = B ndof problems fill the GPU, fewer (more CTAs) for small batches
+static int project_warps(int nprob) {
+  const int warps = (nprob + PROJ_PPW - 1) / PROJ_PPW;
   const int w = (warps + 148 * PROJ_MINB - 1) / (148 * PROJ_MINB);
   return w < 1 ? 1 : (w > PROJ_WARPS ? PROJ_WARPS : w);
 }
@@ -853,12 +870,14 @@ __global__ void __launch_bounds__(MC_THREADS) k_mean_cov(int NVAR, int k, const 
 #define MC_PAD 16                       // the number of blocks is padded to a multiple (zero blocks): no remainder loop in the sums
 static int mc_blocks(int k) { return ((k + MC_EB - 1) / MC_EB + MC_PAD - 1) / MC_PAD * MC_PAD; }
 static size_t mc_stride(int nvar) { return 1 + (size_t)nvar + (size_t)nvar * (nvar + 1) / 2; }
-__global__ void __launch_bounds__(256) k_mc_partial(int NVAR, int k, const float* __restrict__ cost, const float* __restrict__ xi,
-                                                    const float* __restrict__ mean_prev, float lamda, float* __restrict__ part) {
-  __shared__ float red[256];
-  __shared__ float sw[MC_EB];
-  __shared__ float sd[MC_EB][MAXVAR + 1];          // x - a
-  __shared__ float swd[MC_EB][MAXVAR + 1];         // w (x - a)
+// The elite tiles x - a and w (x - a) of a block, rows of LD floats: k_mc_partial keeps them in static shared memory
+// (LD = 97, nvar <= 96), k_mc_partial_wide in dynamic shared memory (LD = 193, nvar <= 192: 49 KB, above the static limit).
+#define MC_LD_SMALL (CHOL_SMALL_N + 1)
+#define MC_LD_WIDE (MAXVAR + 1)
+template <int LD>
+__device__ __forceinline__ void mc_partial_body(int NVAR, int k, const float* __restrict__ cost, const float* __restrict__ xi,
+                                                const float* __restrict__ mean_prev, float lamda, float* __restrict__ part,
+                                                float* red, float* sw, float (*sd)[LD], float (*swd)[LD]) {
   const int tid = threadIdx.x, e0 = blockIdx.x * MC_EB, ne = k - e0 < MC_EB ? (k - e0 > 0 ? k - e0 : 0) : MC_EB;
   const int npair = NVAR * (NVAR + 1) / 2;
   float* P = part + (size_t)blockIdx.x * (1 + NVAR + npair);
@@ -889,16 +908,35 @@ __global__ void __launch_bounds__(256) k_mc_partial(int NVAR, int k, const float
     P[1 + NVAR + p] = t;
   }
 }
-// grid = nvar CTAs (covariance row r = blockIdx.x, entries c <= r and their mirror images), 128 threads
-__global__ void __launch_bounds__(128) k_mc_finish(int NVAR, int nblk, const float* __restrict__ part, const float* __restrict__ mean_prev,
+__global__ void __launch_bounds__(256) k_mc_partial(int NVAR, int k, const float* __restrict__ cost, const float* __restrict__ xi,
+                                                    const float* __restrict__ mean_prev, float lamda, float* __restrict__ part) {
+  __shared__ float red[256];
+  __shared__ float sw[MC_EB];
+  __shared__ float sd[MC_EB][MC_LD_SMALL];         // x - a
+  __shared__ float swd[MC_EB][MC_LD_SMALL];        // w (x - a)
+  mc_partial_body<MC_LD_SMALL>(NVAR, k, cost, xi, mean_prev, lamda, part, red, sw, sd, swd);
+}
+__global__ void __launch_bounds__(256) k_mc_partial_wide(int NVAR, int k, const float* __restrict__ cost, const float* __restrict__ xi,
+                                                         const float* __restrict__ mean_prev, float lamda, float* __restrict__ part) {
+  __shared__ float red[256];
+  __shared__ float sw[MC_EB];
+  extern __shared__ float mc_tiles[];              // sd, swd [MC_EB][MC_LD_WIDE]
+  float (*sd)[MC_LD_WIDE] = reinterpret_cast<float (*)[MC_LD_WIDE]>(mc_tiles);
+  mc_partial_body<MC_LD_WIDE>(NVAR, k, cost, xi, mean_prev, lamda, part, red, sw, sd, sd + MC_EB);
+}
+static size_t mc_wide_smem() { return sizeof(float) * 2 * MC_EB * MC_LD_WIDE; }
+// grid = nvar CTAs (covariance row r = blockIdx.x, entries c <= r and their mirror images), THREADS > nvar threads
+// (128 for nvar <= 127, 256 above)
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS) k_mc_finish(int NVAR, int nblk, const float* __restrict__ part, const float* __restrict__ mean_prev,
                                                    const float* __restrict__ cov_prev, float am, float ac, float* __restrict__ mean_out,
                                                    float* __restrict__ cov_out) {
   __shared__ float sdelta[MAXVAR], sD[MAXVAR], sS2[MAXVAR], sW;
   const int tid = threadIdx.x, r = blockIdx.x, npair = NVAR * (NVAR + 1) / 2;
   const size_t stride = 1 + (size_t)NVAR + npair;
-  // one pass over the blocks: thread t < nvar adds S1[t] and S2[r][t]; thread 127 adds S0 (nvar <= 96)
+  // one pass over the blocks: thread t < nvar adds S1[t] and S2[r][t]; thread THREADS - 1 adds S0
   {
-    const bool w = tid == 127, on = tid < NVAR, lo = on && tid <= r;
+    const bool w = tid == THREADS - 1, on = tid < NVAR, lo = on && tid <= r;
     const float* p1 = part + (w ? 0 : 1 + (on ? tid : 0));
     const float* p2 = part + 1 + NVAR + (size_t)r * (r + 1) / 2 + (lo ? tid : 0);
     float s1 = 0.f, s2 = 0.f;
@@ -944,9 +982,23 @@ __global__ void __launch_bounds__(256) k_fma_peak(float* out, int iters, float a
 }
 
 // ================================================================================================ C ABI
+// block sums of the blocked mean / covariance update, sized for the handle's nvar (19 MB at nvar = 192, 2.3 MB at 66)
+static int mc_alloc(cemk_handle* h) {
+  if (h->d_mc) { CK(cudaFree(h->d_mc)); h->d_mc = nullptr; }
+  CK(cudaMalloc(&h->d_mc, sizeof(float) * mc_blocks(MC_BLOCKED_MAXK) * mc_stride(h->nvar)));
+  return CEMK_OK;
+}
+// the rollout models the KM_NL-DOF arm of the KModel; a handle planning for another DOF count cannot feed it
+static int rollout_dof_check(const cemk_handle* h, const char* fn) {
+  if (h->ndof == KM_NL) return CEMK_OK;
+  snprintf(g_err, sizeof g_err, "%s: DOF mismatch: the rollout models a %d-DOF arm, this handle plans for %d DOF (cemk_set_dof)",
+           fn, KM_NL, h->ndof);
+  return CEMK_ERR_ARG;
+}
+
 extern "C" {
 
-int cemk_version(void) { return 1; }
+int cemk_version(void) { return 2; }
 const char* cemk_last_error(void) { return g_err; }
 int cemk_sizeof_kmodel(void) { return (int)sizeof(KModel); }
 
@@ -958,7 +1010,7 @@ int cemk_create(const void* kmodel, int kmodel_bytes, int device, cemk_handle** 
     return set_err(CEMK_ERR_MODEL, "cemk_create: unsupported topology");
   DevGuard guard(device);
   cemk_handle* h = new cemk_handle();
-  h->device = device; h->ncoef = 11; h->nvar = KM_NL * 11; h->T = 0; h->d_G = nullptr; h->d_K = nullptr; h->launches = 0; h->d_flags = nullptr; h->flags_cap = 0; h->force_rerun = 0; h->cta_samples = 0; h->d_prevd = nullptr; h->prevd_cap = 0; h->d_ovf = nullptr;
+  h->device = device; h->ndof = KM_NL; h->ncoef = 11; h->nvar = KM_NL * 11; h->T = 0; h->d_G = nullptr; h->d_K = nullptr; h->launches = 0; h->d_flags = nullptr; h->flags_cap = 0; h->force_rerun = 0; h->cta_samples = 0; h->d_prevd = nullptr; h->prevd_cap = 0; h->d_ovf = nullptr;
   { cudaDeviceProp prop; CK(cudaGetDeviceProperties(&prop, device)); h->num_sms = prop.multiProcessorCount; }
   CK(cudaMalloc(&h->d_model, sizeof(KModel)));
   CK(cudaMemcpy(h->d_model, kmodel, sizeof(KModel), cudaMemcpyHostToDevice));
@@ -970,9 +1022,11 @@ int cemk_create(const void* kmodel, int kmodel_bytes, int device, cemk_handle** 
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_BIG, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                           (int)rollout_smem<KM_NC_BIG, 1>()));
   h->d_mc = nullptr;
-  CK(cudaMalloc(&h->d_mc, sizeof(float) * mc_blocks(MC_BLOCKED_MAXK) * mc_stride(MAXVAR)));
+  { const int rc = mc_alloc(h); if (rc) return rc; }
   CK(cudaFuncSetAttribute(k_rank_select, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(unsigned long long) * RANK_MAXN)));
   CK(cudaFuncSetAttribute(k_sample, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem(MAXVAR)));
+  CK(cudaFuncSetAttribute(k_chol_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)chol_wide_smem()));
+  CK(cudaFuncSetAttribute(k_mc_partial_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mc_wide_smem()));
   CK(cudaFuncSetAttribute(k_merge_lists<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(unsigned) * MERGE_MAXKEYS)));
   *out = h;
   return CEMK_OK;
@@ -991,14 +1045,23 @@ int cemk_set_model(cemk_handle* h, const void* kmodel, int kmodel_bytes) {
   CK(cudaMemcpy(h->d_model, kmodel, sizeof(KModel), cudaMemcpyHostToDevice));
   return CEMK_OK;
 }
+int cemk_set_dof(cemk_handle* h, int ndof) {
+  if (!h) return set_err(CEMK_ERR_ARG, "cemk_set_dof: null handle");
+  if (ndof < 1 || ndof > MAXDOF) return set_err(CEMK_ERR_ARG, "cemk_set_dof: DOF count out of range [1, 12]");
+  DevGuard guard(h->device);
+  if (h->d_G) { CK(cudaFree(h->d_G)); h->d_G = nullptr; }     // the horizon tables belong to the old width
+  h->T = 0;
+  h->ndof = ndof; h->nvar = ndof * h->ncoef;
+  return mc_alloc(h);
+}
 int cemk_set_order(cemk_handle* h, int ncoef) {
   if (!h) return set_err(CEMK_ERR_ARG, "cemk_set_order: null handle");
   if (ncoef < MINCOEF || ncoef > MAXCOEF) return set_err(CEMK_ERR_ARG, "cemk_set_order: coefficients per DOF out of range [4, 16]");
   DevGuard guard(h->device);
   if (h->d_G) { CK(cudaFree(h->d_G)); h->d_G = nullptr; }     // the horizon tables belong to the old order
   h->T = 0;
-  h->ncoef = ncoef; h->nvar = KM_NL * ncoef;
-  return CEMK_OK;
+  h->ncoef = ncoef; h->nvar = h->ndof * ncoef;
+  return mc_alloc(h);
 }
 int cemk_set_horizon(cemk_handle* h, int T, const float* G, const float* Kpp, const float* Kpe, const float* bounds3) {
   if (!h || !G || !Kpp || !Kpe || !bounds3) return set_err(CEMK_ERR_ARG, "cemk_set_horizon: null argument");
@@ -1016,8 +1079,10 @@ int cemk_set_horizon(cemk_handle* h, int T, const float* G, const float* Kpp, co
   CEMK_FOR_NCOEF(nc, { smem = project_smem<NC>(T, 32 * PROJ_WARPS); });
   if (smem > 227 * 1024) return set_err(CEMK_ERR_ARG, "cemk_set_horizon: horizon too long for the projection kernel's shared memory");
   const int carve = 100 * PROJ_MINB * smem / (228 * 1024) + 8;                       // room for PROJ_MINB CTAs per SM, in percent
-  CEMK_FOR_NCOEF(nc, { CK(cudaFuncSetAttribute(k_project<NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-                       CK(cudaFuncSetAttribute(k_project<NC>, cudaFuncAttributePreferredSharedMemoryCarveout, carve > 100 ? 100 : carve)); });
+  CEMK_FOR_NCOEF(nc, { CK(cudaFuncSetAttribute(k_project<NC, KM_NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+                       CK(cudaFuncSetAttribute(k_project<NC, KM_NL>, cudaFuncAttributePreferredSharedMemoryCarveout, carve > 100 ? 100 : carve));
+                       CK(cudaFuncSetAttribute(k_project<NC, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+                       CK(cudaFuncSetAttribute(k_project<NC, 0>, cudaFuncAttributePreferredSharedMemoryCarveout, carve > 100 ? 100 : carve)); });
   return CEMK_OK;
 }
 
@@ -1025,7 +1090,8 @@ int cemk_sample(cemk_handle* h, int B, const float* z, const float* mean, const 
   if (!h || !z || !mean || !cov || !chol_ws || !xi || B <= 0) return set_err(CEMK_ERR_ARG, "cemk_sample: bad argument");
   DevGuard guard(h->device);
   cudaStream_t st = (cudaStream_t)stream;
-  k_chol66<<<1, 256, 0, st>>>(h->nvar, cov, chol_ws);
+  if (h->nvar <= CHOL_SMALL_N) k_chol66<<<1, 256, 0, st>>>(h->nvar, cov, chol_ws);
+  else k_chol_wide<<<1, 256, chol_wide_smem(), st>>>(h->nvar, cov, chol_ws);
   k_sample<<<(B + SAMPLE_TILE - 1) / SAMPLE_TILE, SAMPLE_THREADS, sample_smem(h->nvar), st>>>(B, h->nvar, z, mean, chol_ws, xi);
   h->launches += 2;
   CK(cudaPeekAtLastError());
@@ -1047,9 +1113,14 @@ int cemk_project(cemk_handle* h, int B, int iters, const float* xi, const float*
   DevGuard guard(h->device);
   if (!h->d_G) return set_err(CEMK_ERR_ARG, "cemk_project: cemk_set_horizon has not been called");
   const int T = h->T;
-  const int wpc = project_warps(B), warps = (B * 6 + PROJ_PPW - 1) / PROJ_PPW;
-  CEMK_FOR_NCOEF(h->ncoef, (k_project<NC><<<(warps + wpc - 1) / wpc, 32 * wpc, project_smem<NC>(T, 32 * wpc), (cudaStream_t)stream>>>(
-                                B, T, iters, h->d_G, h->d_K, xi, state_term, xi_f, thetadot)));
+  const int nprob = B * h->ndof, wpc = project_warps(nprob), warps = (nprob + PROJ_PPW - 1) / PROJ_PPW;
+  const int grid = (warps + wpc - 1) / wpc;
+  if (h->ndof == KM_NL)
+    CEMK_FOR_NCOEF(h->ncoef, (k_project<NC, KM_NL><<<grid, 32 * wpc, project_smem<NC>(T, 32 * wpc), (cudaStream_t)stream>>>(
+                                  B, h->ndof, T, iters, h->d_G, h->d_K, xi, state_term, xi_f, thetadot)))
+  else
+    CEMK_FOR_NCOEF(h->ncoef, (k_project<NC, 0><<<grid, 32 * wpc, project_smem<NC>(T, 32 * wpc), (cudaStream_t)stream>>>(
+                                  B, h->ndof, T, iters, h->d_G, h->d_K, xi, state_term, xi_f, thetadot)))
   h->launches += 1;
   CK(cudaPeekAtLastError());
   return CEMK_OK;
@@ -1060,6 +1131,7 @@ int cemk_rollout_cost(cemk_handle* h, int B, int T, const float* thetadot, const
                       float* eef_rot, float* collision, float* qacc, int* flags, void* stream) {
   if (!h || !thetadot || !q0 || !v0 || !target_pos || !target_rot || !theta || !cost4 || B <= 0 || T <= 0)
     return set_err(CEMK_ERR_ARG, "cemk_rollout_cost: bad argument");
+  { const int rc = rollout_dof_check(h, "cemk_rollout_cost"); if (rc) return rc; }
   DevGuard guard(h->device);
   cudaStream_t st = (cudaStream_t)stream;
   if (!flags) {
@@ -1256,8 +1328,14 @@ int cemk_mean_cov(cemk_handle* h, int k, const float* cost_elite, const float* x
   DevGuard guard(h->device);
   if (k >= MC_BLOCKED_MINK && k <= MC_BLOCKED_MAXK) {
     const int nblk = mc_blocks(k);
-    k_mc_partial<<<nblk, 256, 0, (cudaStream_t)stream>>>(h->nvar, k, cost_elite, xi_elite, mean_prev, lamda, h->d_mc);
-    k_mc_finish<<<h->nvar, 128, 0, (cudaStream_t)stream>>>(h->nvar, nblk, h->d_mc, mean_prev, cov_prev, alpha_mean, alpha_cov, mean_out, cov_out);
+    if (h->nvar < MC_LD_SMALL)
+      k_mc_partial<<<nblk, 256, 0, (cudaStream_t)stream>>>(h->nvar, k, cost_elite, xi_elite, mean_prev, lamda, h->d_mc);
+    else
+      k_mc_partial_wide<<<nblk, 256, mc_wide_smem(), (cudaStream_t)stream>>>(h->nvar, k, cost_elite, xi_elite, mean_prev, lamda, h->d_mc);
+    if (h->nvar < 128)
+      k_mc_finish<128><<<h->nvar, 128, 0, (cudaStream_t)stream>>>(h->nvar, nblk, h->d_mc, mean_prev, cov_prev, alpha_mean, alpha_cov, mean_out, cov_out);
+    else
+      k_mc_finish<256><<<h->nvar, 256, 0, (cudaStream_t)stream>>>(h->nvar, nblk, h->d_mc, mean_prev, cov_prev, alpha_mean, alpha_cov, mean_out, cov_out);
     h->launches += 2;
     CK(cudaPeekAtLastError());
     return CEMK_OK;
@@ -1308,6 +1386,7 @@ int cemk_tick_record(cemk_handle* h, int iter, int n_iter, int last, int B, int 
                      float* best_row, void* stream) {
   if (!h || !cost_elite || !gidx_elite || !flags || !thetadot || !theta || !cost4 || !xi_mean || !out || iter < 0 || iter >= n_iter || B <= 0 || T <= 0)
     return set_err(CEMK_ERR_ARG, "cemk_tick_record: bad argument");
+  { const int rc = rollout_dof_check(h, "cemk_tick_record"); if (rc) return rc; }
   DevGuard guard(h->device);
   k_tick_record<<<1, 256, 0, (cudaStream_t)stream>>>(h->nvar, iter, n_iter, last, B, T, cost_elite, gidx_elite, idx_base, flags, thetadot, theta, cost4,
                                                     xi_mean, out, best_row);

@@ -18,6 +18,11 @@ standard-normal draws are reused every tick; the covariance restarts at 10*I eve
 from the device generator ``cemk_jax_normal`` (same counters, bit -> uniform -> erf_inv mapping as
 jax 0.5.3), so identical seeds give the reference's samples up to float32 rounding of the Cholesky.
 
+Other DOF counts (``num_dof`` 1..12): the per-iteration algebra (sampling, projection filter + Bernstein evaluation,
+elite selection, mean / covariance, the constant matrices) runs on the GPU at that width (nvar = num_dof * (order + 1)
+<= 192).  The model is still scene A's 6-DOF UR5e, so the rollout and everything built on it (``compute_rollout_batch``,
+``cem_iter``, ``compute_cem``) raise ``NotImplementedError`` there.
+
 Multi-GPU (extension, SURVEY.md section 8e): pass ``process_group``; ``num_batch`` is then the global
 batch, each rank rolls out ``num_batch / world`` samples, keeps its local top-k and one NCCL
 all-gather merges the elite lists so every rank computes the identical mean / covariance.
@@ -91,11 +96,12 @@ class cem_planner:
     def __init__(self, num_dof=None, num_batch=None, num_steps=None, timestep=None, maxiter_cem=None, num_elite=None,
                  w_pos=None, w_rot=None, w_col=None, maxiter_projection=None, *, model_path=None, device=None,
                  process_group=None, seed=0, contact_exclude=None, threefry_partitionable=True, bernstein_order=10):
+        if isinstance(num_dof, bool) or not isinstance(num_dof, (int, np.integer)) or not 1 <= num_dof <= 12:
+            raise ValueError(f"num_dof must be an integer in [1, 12], got {num_dof!r}")
+        num_dof = int(num_dof)
         if not torch.cuda.is_available():
             raise RuntimeError("cem_planner needs a CUDA device (B200 / sm_100a); there is no CPU fallback")
         self._lib = _lib.load()
-        if num_dof != 6:
-            raise NotImplementedError("the rollout kernel is built for the 6-DOF UR5e chain (num_dof=6)")
         self.num_dof = num_dof
         self.num_batch = num_batch
         self.t = timestep
@@ -186,10 +192,12 @@ class cem_planner:
         h = _VP()
         _lib.check(self._lib.cemk_create(C.byref(km), C.sizeof(km), dev.index or 0, C.byref(h)), self._lib)
         self._h = h
+        # mjx.forward at qpos0 (:107): its qacc becomes the first warm start of every rollout (the model is 6-DOF whatever
+        # num_dof is, so this runs while the handle still has its default 6 DOF)
+        self.mjx_data = self._initial_forward()
+        _lib.check(self._lib.cemk_set_dof(self._h, self.num_dof), self._lib)
         _lib.check(self._lib.cemk_set_order(self._h, self.nvar_single), self._lib)
         self._set_horizon(Q_inv)
-        # mjx.forward at qpos0 (:107): its qacc becomes the first warm start of every rollout
-        self.mjx_data = self._initial_forward()
 
         # attributes the notebooks touch (mjx_planner.py:98,108): the vmapped outer product and the jitted single step
         self.vec_product = lambda diffs, d: self._t(d).reshape(-1, 1, 1) * torch.einsum("ki,kj->kij", self._t(diffs), self._t(diffs))
@@ -243,7 +251,7 @@ class cem_planner:
         return np.linalg.inv(np.vstack((np.hstack((Q, A_eq.T)), np.hstack((A_eq, np.zeros((ne, ne)))))))
 
     def _set_horizon(self, Q_inv):
-        """Per-DOF blocks of Q_inv (block diagonal: every DOF solves the same 11-variable problem)."""
+        """Per-DOF blocks of Q_inv (block diagonal: every DOF solves the same (order + 1)-variable problem)."""
         n1, nd, nv = self.nvar_single, self.num_dof, self.nvar
         Kpp = Q_inv[:n1, :n1]
         Kpe = Q_inv[:n1, nv:nv + 5]
@@ -255,7 +263,7 @@ class cem_planner:
                     or np.abs(blk[:, nv + 5 * d:nv + 5 * d + 5] - Kpe).max() > 1e-6 * scale):
                 raise RuntimeError("Q_inv is not block diagonal per DOF")
         off = Q_inv[:n1, n1:nv]
-        if np.abs(off).max() > 1e-6 * scale:
+        if off.size and np.abs(off).max() > 1e-6 * scale:
             raise RuntimeError("Q_inv couples different DOFs")
         c32 = lambda a: np.ascontiguousarray(a, dtype=np.float32)
         G, Kpp, Kpe = c32(np.stack((self.Pdot, self.Pddot, self.P))), c32(Kpp), c32(Kpe)
@@ -355,6 +363,12 @@ class cem_planner:
         t = torch.as_tensor(np.asarray(a) if not torch.is_tensor(a) else a, dtype=torch.float32, device=self.device)
         t = t.contiguous()
         return t if shape is None else t.reshape(shape)
+
+    def _require_rollout_dof(self, what):
+        if self.num_dof != 6:
+            raise NotImplementedError(
+                f"{what} needs the rollout, which models scene A's 6-DOF UR5e arm; this planner has num_dof={self.num_dof} "
+                "and the dual-arm model is not built (the planner algebra runs at any num_dof in [1, 12])")
 
     def _stream(self):
         return _VP(torch.cuda.current_stream(self.device).cuda_stream)
@@ -464,6 +478,7 @@ class cem_planner:
 
     def compute_rollout_batch(self, thetadot, init_pos, init_vel):
         """mjx_planner.py:123,266-274 -> theta [B,6T], eef_pos [B,T,3], eef_rot [B,T,4], collision [B,T,187]."""
+        self._require_rollout_dof("compute_rollout_batch")
         tp = torch.zeros(3, device=self.device)
         tr = torch.tensor([1.0, 0, 0, 0], device=self.device)
         theta, _c, eef_pos, eef_rot, collision = self._rollout(thetadot, init_pos, init_vel, tp, tr, True)
@@ -547,6 +562,7 @@ class cem_planner:
 
     # ------------------------------------------------------------------ cem_iter / compute_cem (mjx_planner.py:337-406)
     def cem_iter(self, carry, _):
+        self._require_rollout_dof("cem_iter")
         init_pos, init_vel, target_pos, target_rot, xi_mean, xi_cov, key, state_term = carry
         xi_mean_prev, xi_cov_prev = xi_mean, xi_cov
         xi_samples, key = self.compute_xi_samples(key, xi_mean, xi_cov)
@@ -604,6 +620,7 @@ class cem_planner:
 
     def compute_cem(self, xi_mean, init_pos=np.array([1.5, -1.8, 1.75, -1.25, -1.6, 0]), init_vel=np.zeros(6),
                     init_acc=np.zeros(6), target_pos=np.zeros(3), target_rot=np.zeros(4)):
+        self._require_rollout_dof("compute_cem")
         dev = self.device
         Bl, T, nd, nv = self.num_batch_local, self.num, self.num_dof, self.nvar
         # one packed host->device copy for the per-tick inputs
