@@ -103,22 +103,14 @@ int cemk_cost_batch(cemk_handle* h, int B, int T, int nslot, const float* eef_po
 int cemk_argsort_topk(cemk_handle* h, int n, const float* cost, int cost_stride, int idx_base, unsigned long long* keys_ws,
                       int* idx_sorted, int k, const float* xi, float* xi_elite, float* cost_elite, void* stream);
 
-/* Merge of per-GPU elite lists after the NCCL all-gather: n candidates (cost[n], gidx[n] global
- * sample indices, xi[n][66]); selects the k best by (cost, global index).  keys_ws as above. */
-int cemk_merge_elites(cemk_handle* h, int n, const float* cost, const int* gidx, const float* xi, unsigned long long* keys_ws,
-                      int k, float* xi_elite, float* cost_elite, int* gidx_elite, void* stream);
-
 /* The two halves of the multi-GPU form of compute_ellite_samples without intermediate tensors.
- * cemk_topk_pack: this rank's k best samples as exchange records pack[k][68] = xi[66], cost, global index
- * (idx_base + local row, stored as float: exact below 2^24) -- the send buffer of the NCCL all-gather.
- * cemk_merge_packed: n gathered records (rank-major) -> the k best by (cost, row) = (cost, global index). */
+ * cemk_topk_pack: this rank's k best samples, sorted as above, as exchange records pack[k][68] = xi[66], cost, global index
+ * (idx_base + local row, stored as float: exact below 2^24) -- the send buffer of the NCCL all-gather, and what
+ * cemk_merge_sorted_lists consumes.  keys_ws as above.
+ * cemk_merge_sorted_lists: the all-gathered `nlist` blocks of `kl` such records (rank-major) -> the k best by (cost, row) =
+ * (cost, global index).  No sort: every record finds its global position by binary searches in the other blocks (one launch). */
 int cemk_topk_pack(cemk_handle* h, int n, const float* cost, int cost_stride, int idx_base, unsigned long long* keys_ws, int k,
                    const float* xi, float* pack, void* stream);
-int cemk_merge_packed(cemk_handle* h, int n, const float* packed, unsigned long long* keys_ws, int k, float* xi_elite,
-                      float* cost_elite, int* gidx_elite, void* stream);
-/* The same merge for what the all-gather actually delivers: `nlist` blocks of `kl` records, each block already sorted by
- * cemk_topk_pack on its rank.  No sort: every record finds its global (cost, row) position by binary searches in the other
- * blocks (one launch). */
 int cemk_merge_sorted_lists(cemk_handle* h, int nlist, int kl, const float* packed, int k, float* xi_elite, float* cost_elite,
                             int* gidx_elite, void* stream);
 

@@ -49,9 +49,7 @@ _SIGS = {
     "cemk_rollout_cost": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
     "cemk_cost_batch": ([_vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp], _i),
     "cemk_argsort_topk": ([_vp, _i, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp], _i),
-    "cemk_merge_elites": ([_vp, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp], _i),
     "cemk_topk_pack": ([_vp, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp], _i),
-    "cemk_merge_packed": ([_vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp], _i),
     "cemk_merge_sorted_lists": ([_vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp], _i),
     "cemk_mean_cov": ([_vp, _i, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp, _vp], _i),
     "cemk_set_option": ([_vp, C.c_char_p, _i], _i),

@@ -5,7 +5,7 @@
 //   k_project                compute_projection_filter + A_thetadot @ xi   (:181-249, :348)
 //   k_rollout                vmap(scan(mjx.step)) + compute_cost_batch     (:251-303)   <- hot kernel
 //   k_cost_batch             compute_cost_batch on materialised trajectories (:277-303)
-//   k_rank_select (n <= 8192) | k_make_keys / k_bitonic* / k_finish_sort / k_pack_sorted     compute_ellite_samples   (:306-310)
+//   k_rank_select (n <= 8192) | k_make_keys / k_bitonic* / k_gather_sorted    compute_ellite_samples   (:306-310)
 //   k_merge_lists            the same selection over the per-rank sorted lists of several GPUs
 //   k_mean_cov | k_mc_partial[_wide] + k_mc_finish (k >= 1024)             compute_mean_cov (:326-335)
 //   k_tick_record            what compute_cem keeps of an iteration        (:390-404)
@@ -562,31 +562,11 @@ __global__ void k_make_keys(int n, int npow2, const float* __restrict__ cost, in
   keys[i] = i < n ? (((unsigned long long)float_order(cost[(size_t)i * stride]) << 32) | (unsigned int)i) : ~0ull;
 }
 #define SORT_BLK 4096    // keys per CTA held in shared memory (32 KB)
-// all stages with partner distance < SORT_BLK for merge size k; kfirst: run the full local sort (k = 2..SORT_BLK)
-__global__ void __launch_bounds__(1024) k_bitonic_local(unsigned long long* __restrict__ keys, int npow2, int k_outer, int full) {
-  __shared__ unsigned long long s[SORT_BLK];
-  const int base = blockIdx.x * SORT_BLK;
-  const int cnt = npow2 < SORT_BLK ? npow2 : SORT_BLK;
-  for (int e = threadIdx.x; e < cnt; e += blockDim.x) s[e] = keys[base + e];
-  __syncthreads();
-  for (int k = full ? 2 : k_outer; k <= (full ? cnt : k_outer); k <<= 1) {
-    for (int j = (k >> 1) < cnt ? (k >> 1) : (cnt >> 1); j > 0; j >>= 1) {
-      for (int e = threadIdx.x; e < cnt / 2; e += blockDim.x) {
-        const int i = 2 * e - (e & (j - 1));            // index with bit j clear
-        const int p = i + j;
-        const bool up = (((base + i) & k) == 0);
-        unsigned long long a = s[i], b = s[p];
-        if ((a > b) == up) { s[i] = b; s[p] = a; }
-      }
-      __syncthreads();
-    }
-  }
-  for (int e = threadIdx.x; e < cnt; e += blockDim.x) keys[base + e] = s[e];
-}
-// The same stages for a full block of SORT_BLK keys with four consecutive keys per thread in registers: partner distances
-// 1, 2 stay inside a thread, 4 .. 64 inside a warp (shuffles), only distances >= 128 go through shared memory -- 15 of the 78
-// stages of a full 4096-key sort need a barrier pair instead of all of them (39 -> about 20 us).  Keys are unique (the low
-// word is the index), so any correct sorting network gives the identical result.
+// All stages with partner distance < SORT_BLK for merge size k_outer (full: the whole local sort, k = 2..SORT_BLK) on a block of
+// SORT_BLK keys, four consecutive keys per thread in registers: partner distances 1, 2 stay inside a thread, 4 .. 64 inside a
+// warp (shuffles), only distances >= 128 go through shared memory -- 15 of the 78 stages of a full 4096-key sort need a barrier
+// pair instead of all of them (39 -> about 20 us).  Keys are unique (the low word is the index), so any correct sorting
+// network gives the identical result.
 __device__ __forceinline__ void bitonic_cas(unsigned long long& a, unsigned long long b, bool keep_min) {
   a = keep_min ? (a < b ? a : b) : (a > b ? a : b);
 }
@@ -691,48 +671,23 @@ __global__ void __launch_bounds__(RANK_THREADS) k_rank_select(int NVAR, int n, c
     }
   }
 }
-static void rank_select(cemk_handle* h, int n, const float* cost, int stride, int idx_base, unsigned long long* keys, int* idx_sorted, int k,
-                        const float* xi, float* xi_elite, float* cost_elite, float* pack, cudaStream_t st) {
-  k_rank_select<<<(n + RANK_CAND - 1) / RANK_CAND, RANK_THREADS, sizeof(unsigned long long) * n, st>>>(h->nvar, n, cost, stride, idx_base, keys, idx_sorted,
-                                                                                                     k, xi, xi_elite, cost_elite, pack);
-  h->launches += 1;
-}
-__global__ void k_finish_sort(int NVAR, int n, const unsigned long long* __restrict__ keys, int idx_base, int* __restrict__ idx_sorted, int k,
-                              const float* __restrict__ cost, int stride, const float* __restrict__ xi, float* __restrict__ xi_elite,
-                              float* __restrict__ cost_elite, const int* __restrict__ aux_in, int* __restrict__ aux_out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+static_assert(RANK_MAXN >= SORT_BLK, "the bitonic path (n > RANK_MAXN) assumes full SORT_BLK blocks");
+// The gather after the bitonic sort, with k_rank_select's outputs: idx_sorted[n] when given, then the k best rows either as
+// xi_elite / cost_elite or as the elite exchange records pack[k][nvar + 2] = xi[nvar], cost, global index (as float, exact
+// below 2^24) that one rank contributes to the NCCL all-gather.
+__global__ void k_gather_sorted(int NVAR, int n, const unsigned long long* __restrict__ keys, int idx_base, int* __restrict__ idx_sorted, int k,
+                                const float* __restrict__ cost, int stride, const float* __restrict__ xi, float* __restrict__ xi_elite,
+                                float* __restrict__ cost_elite, float* __restrict__ pack) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x, W = pack ? NVAR + 2 : NVAR;
   if (idx_sorted && i < n) idx_sorted[i] = (int)(unsigned int)(keys[i] & 0xffffffffull) + idx_base;
-  if (i < k * NVAR) {
-    const int e = i / NVAR, c = i % NVAR;
-    const int src = (int)(unsigned int)(keys[e] & 0xffffffffull);
+  if (i >= k * W) return;
+  const int e = i / W, c = i % W;
+  const int src = (int)(unsigned int)(keys[e] & 0xffffffffull);
+  if (pack) pack[i] = c < NVAR ? xi[(size_t)src * NVAR + c] : (c == NVAR ? cost[(size_t)src * stride] : (float)(src + idx_base));
+  else {
     xi_elite[i] = xi[(size_t)src * NVAR + c];
-    if (c == 0) {
-      cost_elite[e] = cost[(size_t)src * stride];
-      if (aux_out) aux_out[e] = aux_in[src];
-    }
+    if (c == 0) cost_elite[e] = cost[(size_t)src * stride];
   }
-}
-
-// Elite exchange records [..][nvar + 2] = xi[nvar], cost, global index (as float, exact below 2^24):
-// what one rank contributes to the NCCL all-gather, written / read without intermediate tensors.
-__global__ void k_pack_sorted(int NVAR, const unsigned long long* __restrict__ keys, int idx_base, int k, const float* __restrict__ cost, int stride,
-                              const float* __restrict__ xi, float* __restrict__ pack) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x, PACKW = NVAR + 2;
-  if (i >= k * PACKW) return;
-  const int e = i / PACKW, c = i % PACKW;
-  const int src = (int)(unsigned int)(keys[e] & 0xffffffffull);
-  pack[i] = c < NVAR ? xi[(size_t)src * NVAR + c] : (c == NVAR ? cost[(size_t)src * stride] : (float)(src + idx_base));
-}
-__global__ void k_unpack_sorted(int NVAR, const unsigned long long* __restrict__ keys, int k, const float* __restrict__ packed,
-                                float* __restrict__ xi_elite, float* __restrict__ cost_elite, int* __restrict__ gidx_elite) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x, PACKW = NVAR + 2;
-  if (i >= k * PACKW) return;
-  const int e = i / PACKW, c = i % PACKW;
-  const int src = (int)(unsigned int)(keys[e] & 0xffffffffull);
-  const float v = packed[(size_t)src * PACKW + c];
-  if (c < NVAR) xi_elite[e * NVAR + c] = v;
-  else if (c == NVAR) cost_elite[e] = v;
-  else gidx_elite[e] = (int)v;
 }
 
 // Merge of the gathered elite lists without sorting: the candidates arrive as `nlist` blocks of `kl` records, each block
@@ -998,7 +953,7 @@ static int rollout_dof_check(const cemk_handle* h, const char* fn) {
 
 extern "C" {
 
-int cemk_version(void) { return 2; }
+int cemk_version(void) { return 3; }
 const char* cemk_last_error(void) { return g_err; }
 int cemk_sizeof_kmodel(void) { return (int)sizeof(KModel); }
 
@@ -1209,11 +1164,10 @@ int cemk_cost_batch(cemk_handle* h, int B, int T, int nslot, const float* eef_po
   return CEMK_OK;
 }
 
-static int sort_keys(cemk_handle* h, int npow2, unsigned long long* keys, cudaStream_t st) {
-  const int nblk = npow2 > SORT_BLK ? npow2 / SORT_BLK : 1;
-  const bool blk4 = npow2 >= SORT_BLK;                     // full blocks: the register / shuffle variant
-  if (blk4) k_bitonic_local4<<<nblk, SORT_BLK / 4, 0, st>>>(keys, 0, 1);
-  else k_bitonic_local<<<nblk, 1024, 0, st>>>(keys, npow2, 0, 1);
+// npow2 >= SORT_BLK: only called above RANK_MAXN
+static void sort_keys(cemk_handle* h, int npow2, unsigned long long* keys, cudaStream_t st) {
+  const int nblk = npow2 / SORT_BLK;
+  k_bitonic_local4<<<nblk, SORT_BLK / 4, 0, st>>>(keys, 0, 1);
   h->launches += 1;
   for (int k = 2 * SORT_BLK; k <= npow2; k <<= 1) {
     for (int j = k >> 1; j >= SORT_BLK; j >>= 1) {
@@ -1223,48 +1177,37 @@ static int sort_keys(cemk_handle* h, int npow2, unsigned long long* keys, cudaSt
     k_bitonic_local4<<<nblk, SORT_BLK / 4, 0, st>>>(keys, k, 0);
     h->launches += 1;
   }
-  return CEMK_OK;
 }
 static int next_pow2(int n) { int p = 1; while (p < n) p <<= 1; return p; }
+
+// The stable top-k of cost behind cemk_argsort_topk (pack null) and cemk_topk_pack (pack given, xi_elite / cost_elite /
+// idx_sorted null): one counting-rank launch up to RANK_MAXN keys, else key generation + the bitonic sort + the gather.
+static int select_topk(cemk_handle* h, int n, const float* cost, int stride, int idx_base, unsigned long long* keys, int* idx_sorted, int k,
+                       const float* xi, float* xi_elite, float* cost_elite, float* pack, cudaStream_t st) {
+  const int NVAR = h->nvar;
+  if (n <= RANK_MAXN) {
+    k_rank_select<<<(n + RANK_CAND - 1) / RANK_CAND, RANK_THREADS, sizeof(unsigned long long) * n, st>>>(NVAR, n, cost, stride, idx_base, keys, idx_sorted,
+                                                                                                       k, xi, xi_elite, cost_elite, pack);
+    h->launches += 1;
+  } else {
+    const int np2 = next_pow2(n);
+    k_make_keys<<<(np2 + 255) / 256, 256, 0, st>>>(n, np2, cost, stride, keys);
+    h->launches += 1;
+    sort_keys(h, np2, keys, st);
+    const int work = pack ? k * (NVAR + 2) : (n > k * NVAR ? n : k * NVAR);
+    k_gather_sorted<<<(work + 255) / 256, 256, 0, st>>>(NVAR, n, keys, idx_base, idx_sorted, k, cost, stride, xi, xi_elite, cost_elite, pack);
+    h->launches += 1;
+  }
+  CK(cudaPeekAtLastError());
+  return CEMK_OK;
+}
 
 int cemk_argsort_topk(cemk_handle* h, int n, const float* cost, int cost_stride, int idx_base, unsigned long long* keys_ws,
                       int* idx_sorted, int k, const float* xi, float* xi_elite, float* cost_elite, void* stream) {
   if (!h || !cost || !keys_ws || n <= 0 || k < 0 || k > n || cost_stride < 1) return set_err(CEMK_ERR_ARG, "cemk_argsort_topk: bad argument");
   DevGuard guard(h->device);
   if (k > 0 && (!xi || !xi_elite || !cost_elite)) return set_err(CEMK_ERR_ARG, "cemk_argsort_topk: elite buffers missing");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (n <= RANK_MAXN) {
-    rank_select(h, n, cost, cost_stride, idx_base, keys_ws, idx_sorted, k, xi, xi_elite, cost_elite, nullptr, st);
-    CK(cudaPeekAtLastError());
-    return CEMK_OK;
-  }
-  const int np2 = next_pow2(n);
-  k_make_keys<<<(np2 + 255) / 256, 256, 0, st>>>(n, np2, cost, cost_stride, keys_ws);
-  h->launches += 1;
-  sort_keys(h, np2, keys_ws, st);
-  const int NVAR = h->nvar, work = n > k * NVAR ? n : k * NVAR;
-  k_finish_sort<<<(work + 255) / 256, 256, 0, st>>>(NVAR, n, keys_ws, idx_base, idx_sorted, k, cost, cost_stride, xi, xi_elite, cost_elite, nullptr, nullptr);
-  h->launches += 1;
-  CK(cudaPeekAtLastError());
-  return CEMK_OK;
-}
-
-int cemk_merge_elites(cemk_handle* h, int n, const float* cost, const int* gidx, const float* xi, unsigned long long* keys_ws, int k,
-                      float* xi_elite, float* cost_elite, int* gidx_elite, void* stream) {
-  if (!h || !cost || !gidx || !xi || !keys_ws || !xi_elite || !cost_elite || !gidx_elite || n <= 0 || k <= 0 || k > n)
-    return set_err(CEMK_ERR_ARG, "cemk_merge_elites: bad argument");
-  DevGuard guard(h->device);
-  cudaStream_t st = (cudaStream_t)stream;
-  const int np2 = next_pow2(n);
-  // candidate rows arrive rank-major and (cost, index)-sorted within a rank, so the row number breaks
-  // cost ties exactly like the global sample index does
-  k_make_keys<<<(np2 + 255) / 256, 256, 0, st>>>(n, np2, cost, 1, keys_ws);
-  h->launches += 1;
-  sort_keys(h, np2, keys_ws, st);
-  k_finish_sort<<<(k * h->nvar + 255) / 256, 256, 0, st>>>(h->nvar, 0, keys_ws, 0, nullptr, k, cost, 1, xi, xi_elite, cost_elite, gidx, gidx_elite);
-  h->launches += 1;
-  CK(cudaPeekAtLastError());
-  return CEMK_OK;
+  return select_topk(h, n, cost, cost_stride, idx_base, keys_ws, idx_sorted, k, xi, xi_elite, cost_elite, nullptr, (cudaStream_t)stream);
 }
 
 int cemk_topk_pack(cemk_handle* h, int n, const float* cost, int cost_stride, int idx_base, unsigned long long* keys_ws, int k,
@@ -1272,38 +1215,7 @@ int cemk_topk_pack(cemk_handle* h, int n, const float* cost, int cost_stride, in
   if (!h || !cost || !keys_ws || !xi || !pack || n <= 0 || k <= 0 || k > n || cost_stride < 1)
     return set_err(CEMK_ERR_ARG, "cemk_topk_pack: bad argument");
   DevGuard guard(h->device);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (n <= RANK_MAXN) {
-    rank_select(h, n, cost, cost_stride, idx_base, keys_ws, nullptr, k, xi, nullptr, nullptr, pack, st);
-    CK(cudaPeekAtLastError());
-    return CEMK_OK;
-  }
-  const int np2 = next_pow2(n);
-  k_make_keys<<<(np2 + 255) / 256, 256, 0, st>>>(n, np2, cost, cost_stride, keys_ws);
-  h->launches += 1;
-  sort_keys(h, np2, keys_ws, st);
-  k_pack_sorted<<<(k * (h->nvar + 2) + 255) / 256, 256, 0, st>>>(h->nvar, keys_ws, idx_base, k, cost, cost_stride, xi, pack);
-  h->launches += 1;
-  CK(cudaPeekAtLastError());
-  return CEMK_OK;
-}
-
-int cemk_merge_packed(cemk_handle* h, int n, const float* packed, unsigned long long* keys_ws, int k, float* xi_elite,
-                      float* cost_elite, int* gidx_elite, void* stream) {
-  if (!h || !packed || !keys_ws || !xi_elite || !cost_elite || !gidx_elite || n <= 0 || k <= 0 || k > n)
-    return set_err(CEMK_ERR_ARG, "cemk_merge_packed: bad argument");
-  DevGuard guard(h->device);
-  cudaStream_t st = (cudaStream_t)stream;
-  const int np2 = next_pow2(n);
-  // candidate rows arrive rank-major and (cost, index)-sorted within a rank, so the row number breaks
-  // cost ties exactly like the global sample index does
-  k_make_keys<<<(np2 + 255) / 256, 256, 0, st>>>(n, np2, packed + h->nvar, h->nvar + 2, keys_ws);
-  h->launches += 1;
-  sort_keys(h, np2, keys_ws, st);
-  k_unpack_sorted<<<(k * (h->nvar + 2) + 255) / 256, 256, 0, st>>>(h->nvar, keys_ws, k, packed, xi_elite, cost_elite, gidx_elite);
-  h->launches += 1;
-  CK(cudaPeekAtLastError());
-  return CEMK_OK;
+  return select_topk(h, n, cost, cost_stride, idx_base, keys_ws, nullptr, k, xi, nullptr, nullptr, pack, (cudaStream_t)stream);
 }
 
 int cemk_merge_sorted_lists(cemk_handle* h, int nlist, int kl, const float* packed, int k, float* xi_elite, float* cost_elite,

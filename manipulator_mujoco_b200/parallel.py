@@ -10,7 +10,7 @@ does -- i.e. like the reference's stable ``jnp.argsort`` over the whole batch (m
 Every rank therefore holds the identical elite list and computes the identical mean / covariance;
 no broadcast is needed.
 
-Exchange record (what ``cemk_topk_pack`` writes and ``cemk_merge_packed`` reads): ``[k'][nvar + 2]`` float32 =
+Exchange record (what ``cemk_topk_pack`` writes and ``cemk_merge_sorted_lists`` reads): ``[k'][nvar + 2]`` float32 =
 xi[nvar], cost, global sample index (exact in float32 below 2^24, checked once at construction).
 """
 from __future__ import annotations

@@ -498,10 +498,10 @@ class cem_planner:
                                              self._stream()), self._lib)
         return cost4[:, 0], cost4[:, 1], cost4[:, 2], cost4[:, 3]
 
-    def _argsort_topk(self, cost, stride, n, k, xi, idx_base=0, want_idx=True):
+    def _argsort_topk(self, cost, stride, n, k, xi, idx_base=0):
         np2 = 1 << max(0, (n - 1).bit_length())
         keys = self._buf("keys", (np2,), torch.int64)
-        idx = torch.empty(n, dtype=torch.int32, device=self.device) if want_idx else None
+        idx = torch.empty(n, dtype=torch.int32, device=self.device)
         xi_e = torch.empty(k, self.nvar, device=self.device)
         cost_e = torch.empty(k, device=self.device)
         _lib.check(self._lib.cemk_argsort_topk(self._h, n, _ptr(cost), stride, idx_base, _ptr(keys), _ptr(idx), k, _ptr(xi),

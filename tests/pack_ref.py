@@ -1,9 +1,7 @@
-"""numpy restatement of the elite-exchange kernels (test infrastructure; csrc/cemk.cu k_make_keys / k_pack_sorted /
-k_unpack_sorted behind cemk_topk_pack and cemk_merge_packed).  Used by the gloo tests on the CPU and compared bit for bit
-with the CUDA kernels in tests/test_gpu_kernels.py."""
+"""numpy restatement of the elite exchange (test infrastructure; csrc/cemk.cu behind cemk_topk_pack and
+cemk_merge_sorted_lists), at any width nvar.  Used by the gloo tests on the CPU and compared bit for bit with the CUDA
+kernels in tests/test_gpu_kernels.py and tests/test_gpu_dof.py."""
 import numpy as np
-
-NVAR = 66
 
 
 def stable_order(cost):
@@ -14,16 +12,36 @@ def stable_order(cost):
 
 
 def topk_pack_ref(cost, idx_base, k, xi):
-    """cemk_topk_pack: records [k][NVAR + 2] = xi, cost, global index (as float32) of the k best local samples."""
+    """cemk_topk_pack: records [k][nvar + 2] = xi, cost, global index (as float32) of the k best local samples."""
+    nv = xi.shape[1]
     loc = stable_order(cost)[:k]
-    out = np.empty((k, NVAR + 2), np.float32)
-    out[:, :NVAR] = xi[loc]
-    out[:, NVAR] = np.asarray(cost, np.float32)[loc]
-    out[:, NVAR + 1] = (loc + idx_base).astype(np.float32)
+    out = np.empty((k, nv + 2), np.float32)
+    out[:, :nv] = xi[loc]
+    out[:, nv] = np.asarray(cost, np.float32)[loc]
+    out[:, nv + 1] = (loc + idx_base).astype(np.float32)
     return out
 
 
-def merge_packed_ref(packed, k):
-    """cemk_merge_packed: the k best candidate rows by (cost, row) -> xi_elite, cost_elite, gidx_elite."""
-    sel = stable_order(packed[:, NVAR])[:k]
-    return packed[sel, :NVAR].copy(), packed[sel, NVAR].copy(), packed[sel, NVAR + 1].astype(np.int32)
+def _order_key(cost):
+    """float_order in csrc/cemk.cu: float32 bits mapped to an ascending unsigned key, every NaN last."""
+    u = np.asarray(cost, np.float32).view(np.uint32)
+    key = np.where(u & 0x80000000, ~u, u | 0x80000000)
+    return np.where(np.isnan(cost), np.uint32(0xffffffff), key).astype(np.uint32)
+
+
+def merge_sorted_lists_ref(packed, nlist, kl, k):
+    """cemk_merge_sorted_lists: `nlist` blocks of `kl` (cost, index)-sorted records -> the k best by (cost, row) as xi_elite,
+    cost_elite, gidx_elite.  k_merge_lists' rule: a record's position is its position in its own block plus, for every other
+    block, the number of records with a smaller key; blocks before its own also count equal keys."""
+    nv = packed.shape[1] - 2
+    key = _order_key(packed[:, nv]).reshape(nlist, kl)
+    pos = np.tile(np.arange(kl), (nlist, 1))
+    for a in range(nlist):
+        for b in range(nlist):
+            if b != a:
+                pos[a] += np.searchsorted(key[b], key[a], side="right" if b < a else "left")
+    pos = pos.ravel()
+    win = np.flatnonzero(pos < k)
+    sel = np.empty(k, np.int64)
+    sel[pos[win]] = win
+    return packed[sel, :nv].copy(), packed[sel, nv].copy(), packed[sel, nv + 1].astype(np.int32)

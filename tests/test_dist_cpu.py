@@ -1,8 +1,8 @@
 """world_size-2 (and 4) gloo tests of the sample-sharded CEM plumbing (manipulator_mujoco_b200/parallel.py), on the exchange
-record layout the kernels use (cemk_topk_pack -> all-gather -> cemk_merge_packed; tests/pack_ref.py restates the two
-kernels in numpy and tests/test_gpu_kernels.py checks the kernels against that restatement bit for bit):
-local top-k' + all-gather + (cost, row) merge == the reference's global stable argsort top-k, including cost ties across
-ranks and NaN costs; the best-sample exchange survives NaN rows on non-owning ranks."""
+record layout the kernels use (cemk_topk_pack -> all-gather -> cemk_merge_sorted_lists; tests/pack_ref.py restates the
+two in numpy and tests/test_gpu_kernels.py checks the kernels against that restatement bit for bit):
+local top-k' + all-gather + merge of the per-rank sorted blocks == the reference's global stable argsort top-k, including
+cost ties across ranks and NaN costs; the best-sample exchange survives NaN rows on non-owning ranks."""
 import os
 import socket
 
@@ -13,7 +13,7 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 from manipulator_mujoco_b200 import parallel
-from pack_ref import merge_packed_ref, stable_order, topk_pack_ref
+from pack_ref import merge_sorted_lists_ref, stable_order, topk_pack_ref
 
 NVAR = 66
 
@@ -44,7 +44,7 @@ def _worker(rank, world, port, B, k, seed, ret):
     pack = torch.from_numpy(topk_pack_ref(cost4[:, 0], lo, kl, xi[lo:hi]))           # cemk_topk_pack
     gathered = parallel.gather_elites(pack, world, out=torch.empty(world * kl, NVAR + 2))     # the planner's call (persistent buffer)
     assert torch.equal(gathered[rank * kl:(rank + 1) * kl].view(torch.int32), pack.view(torch.int32))
-    xi_e, cost_e, gidx_e = merge_packed_ref(gathered.numpy(), k)                     # cemk_merge_packed
+    xi_e, cost_e, gidx_e = merge_sorted_lists_ref(gathered.numpy(), world, kl, k)     # cemk_merge_sorted_lists
     # best-sample exchange (planner._cem_device): the owner of the global best contributes its row, every other
     # rank's candidate row is an arbitrary local sample -- here NaN / Inf on purpose
     gbest = int(gidx_e[0])

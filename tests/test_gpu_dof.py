@@ -9,6 +9,8 @@ import numpy as np
 import pytest
 import torch
 
+from pack_ref import stable_order, topk_pack_ref
+
 pytestmark = pytest.mark.gpu
 
 DOFS = [12, 7, 1]
@@ -32,22 +34,6 @@ def _pair(nd, order):
 
 def _p(t):
     return C.c_void_p(t.data_ptr()) if t is not None else None
-
-
-def _stable_order(cost):
-    key = np.where(np.isnan(cost), np.inf, cost)
-    return np.lexsort((np.arange(len(cost)), np.isnan(cost), key))
-
-
-def topk_pack_ref(cost, idx_base, k, xi):
-    """cemk_topk_pack at any width: records [k][nvar + 2] = xi, cost, global index (as float32) of the k best local samples."""
-    nv = xi.shape[1]
-    loc = _stable_order(cost)[:k]
-    out = np.empty((k, nv + 2), np.float32)
-    out[:, :nv] = xi[loc]
-    out[:, nv] = np.asarray(cost, np.float32)[loc]
-    out[:, nv + 1] = (loc + idx_base).astype(np.float32)
-    return out
 
 
 @pytest.mark.parametrize("nd,order", GRID)
@@ -136,7 +122,7 @@ def test_elite_selection_is_stable_with_nan_last(nd, order, n):
     cost[7], cost[11] = -5.0, np.inf
     xi = rng.normal(size=(n, nv)).astype(np.float32)
     xe, idx, ce = pl.compute_ellite_samples(cost, xi)
-    ref = _stable_order(cost)
+    ref = stable_order(cost)
     k = pl.ellite_num
     np.testing.assert_array_equal(idx.cpu().numpy(), ref)
     np.testing.assert_array_equal(xe.cpu().numpy(), xi[ref[:k]])
@@ -171,7 +157,7 @@ def test_topk_pack_and_merge_of_sorted_lists(nd, order):
     ge = torch.empty(k, dtype=torch.int32, device="cuda")
     _lib.check(lib.cemk_merge_sorted_lists(h, len(sizes), k, _p(gathered), k, _p(xe), _p(ce), _p(ge), None), lib)
     torch.cuda.synchronize()
-    ref = _stable_order(cost)[:k]
+    ref = stable_order(cost)[:k]
     np.testing.assert_array_equal(ge.cpu().numpy(), ref)
     np.testing.assert_array_equal(xe.cpu().numpy(), xi[ref])
     np.testing.assert_array_equal(ce.cpu().numpy().view(np.int32), cost[ref].view(np.int32))

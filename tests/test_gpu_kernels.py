@@ -180,46 +180,41 @@ def test_compute_cem_end_to_end_against_oracle_pipeline(oracle64):
         np.testing.assert_allclose(xi_mean, m_ref, atol=5e-3)
 
 
-def test_packed_topk_and_merge_equal_global_stable_topk(planner):
-    """cemk_topk_pack on two shards + cemk_merge_packed (the multi-GPU elite exchange without NCCL in between)
-    must give the global stable top-k, ties and NaNs included."""
+def test_topk_pack_and_merge_of_sorted_lists_equal_global_stable_topk(planner):
+    """cemk_topk_pack on three shards (two rank-select, one bitonic) + cemk_merge_sorted_lists (the multi-GPU elite exchange
+    without NCCL in between) must give the global stable top-k, ties and NaNs included."""
     import ctypes as C
     from manipulator_mujoco_b200 import _lib
-    from pack_ref import merge_packed_ref, topk_pack_ref
+    from pack_ref import merge_sorted_lists_ref, topk_pack_ref
     lib, h = planner._lib, planner._h
     rng = np.random.default_rng(4)
-    n, k, nv = 3000, 150, 66
+    sizes, k, nv = (1500, 1500, 9000), 150, 66
+    n = sum(sizes)
     cost = rng.uniform(0, 100, n).astype(np.float32)
-    cost[rng.integers(0, n, 600)] = 5.0                                # ties across both shards
-    cost[[7, 2000]] = np.nan
+    cost[rng.integers(0, n, n // 5)] = 1.0                             # ties across all shards, the k-th best among them
+    cost[[7, 2000, 9000]] = np.nan
     xi = rng.normal(size=(n, nv)).astype(np.float32)
     p = lambda t: C.c_void_p(t.data_ptr())
-    packs = []
-    for r in range(2):
-        lo, hi = r * n // 2, (r + 1) * n // 2
-        c = torch.tensor(cost[lo:hi], device="cuda"); x = torch.tensor(xi[lo:hi], device="cuda")
-        keys = torch.empty(2048, dtype=torch.int64, device="cuda")
+    packs, lo = [], 0
+    for m in sizes:
+        c = torch.tensor(cost[lo:lo + m], device="cuda"); x = torch.tensor(xi[lo:lo + m], device="cuda")
+        keys = torch.empty(1 << (m - 1).bit_length(), dtype=torch.int64, device="cuda")
         pack = torch.empty(k, nv + 2, device="cuda")
-        _lib.check(lib.cemk_topk_pack(h, hi - lo, p(c), 1, lo, p(keys), k, p(x), p(pack), None), lib)
+        _lib.check(lib.cemk_topk_pack(h, m, p(c), 1, lo, p(keys), k, p(x), p(pack), None), lib)
         packs.append(pack)
         # the numpy restatement the gloo tests run on (tests/pack_ref.py) is the kernel's record, bit for bit
-        np.testing.assert_array_equal(pack.cpu().numpy().view(np.int32), topk_pack_ref(cost[lo:hi], lo, k, xi[lo:hi]).view(np.int32))
+        np.testing.assert_array_equal(pack.cpu().numpy().view(np.int32), topk_pack_ref(cost[lo:lo + m], lo, k, xi[lo:lo + m]).view(np.int32))
+        lo += m
     gathered = torch.cat(packs).contiguous()
-    keys = torch.empty(512, dtype=torch.int64, device="cuda")
     xe = torch.empty(k, nv, device="cuda"); ce = torch.empty(k, device="cuda"); ge = torch.empty(k, dtype=torch.int32, device="cuda")
-    _lib.check(lib.cemk_merge_packed(h, 2 * k, p(gathered), p(keys), k, p(xe), p(ce), p(ge), None), lib)
+    _lib.check(lib.cemk_merge_sorted_lists(h, len(sizes), k, p(gathered), k, p(xe), p(ce), p(ge), None), lib)
     torch.cuda.synchronize()
     key = np.where(np.isnan(cost), np.inf, cost)
     ref = np.lexsort((np.arange(n), np.isnan(cost), key))[:k]
     np.testing.assert_array_equal(ge.cpu().numpy(), ref)
     np.testing.assert_array_equal(xe.cpu().numpy(), xi[ref])
     np.testing.assert_array_equal(ce.cpu().numpy().view(np.int32), cost[ref].view(np.int32))
-    # the sort-free merge of per-rank sorted blocks (what the planner calls after the all-gather) gives the same answer
-    xe2 = torch.empty(k, nv, device="cuda"); ce2 = torch.empty(k, device="cuda"); ge2 = torch.empty(k, dtype=torch.int32, device="cuda")
-    _lib.check(lib.cemk_merge_sorted_lists(h, 2, k, p(gathered), k, p(xe2), p(ce2), p(ge2), None), lib)
-    torch.cuda.synchronize()
-    assert torch.equal(ge2, ge) and torch.equal(xe2, xe) and torch.equal(ce2.view(torch.int32), ce.view(torch.int32))
-    rx, rc, rg = merge_packed_ref(gathered.cpu().numpy(), k)
+    rx, rc, rg = merge_sorted_lists_ref(gathered.cpu().numpy(), len(sizes), k, k)
     np.testing.assert_array_equal(ge.cpu().numpy(), rg)
     np.testing.assert_array_equal(xe.cpu().numpy(), rx)
     np.testing.assert_array_equal(ce.cpu().numpy().view(np.int32), rc.view(np.int32))
