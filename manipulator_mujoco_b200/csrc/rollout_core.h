@@ -90,7 +90,10 @@ struct WarpSmemT {
       float bstage[KM_MAXBPAIR][4][4], bnrm[KM_MAXBPAIR][4];
       union {
         struct { float bbR[12], bbc[4], bbsz[2][4], bbrf[4][4], bben[4][4], bbpoly[2][8][4], bbpref[8][4]; };
-        struct { float estage[KW][16], eres[KW][8]; };      // near pass: box-frame geometry of the pairs in their edge stage, and its result
+        struct {                                            // near pass: box-frame geometry of the pairs in their edge stage (by list slot),
+          float estage[KW][16], eres[KW][8];                // the result of the edge item each lane evaluated in this round,
+          unsigned short eidx[KW * 12];                     // and the edge items of the group: list slot << 4 | edge
+        };
       };
     };
   };
@@ -417,8 +420,8 @@ KNOINLINE CapBoxEdge capbox_edges(float ax, float ay, float az, float bx, float 
 // Near path, in box coordinates; the caller has established has_support (= !capbox_far).  Face part in registers
 // (no dynamic indexing); FULL also produces contact positions / normals.
 // Returns the number of box axes on which the segment's bounding interval sticks out of the box (the edge stage can only
-// matter when that is >= 2).  EDGES = false leaves the edge stage to the caller (the near pass spreads the 12 edges of a pair
-// over lanes, see capbox_edge_lane) and also returns the outward normal of the best face in `nface`.
+// matter when that is >= 2).  EDGES = false leaves the edge stage to the caller (the near pass deals the candidate edges of its
+// pairs over lanes, see capbox_edge_mask) and also returns the outward normal of the best face in `nface`.
 template <bool FULL, bool EDGES = true>
 KFN int capsule_box_near(const float* a, const float* b, float r, const float* bsize, CapBoxOut& o, float* nface = nullptr) {
   // best face: first argmax over (+x,-x,+y,-y,+z,-z) of min over end points of the signed face distance
@@ -486,12 +489,14 @@ KFN int capsule_box_near(const float* a, const float* b, float r, const float* b
 // One of the 12 box edges against the capsule segment: the body of capbox_edges' loop for edge e = 4 k + 2 iu + iw, written in
 // the edge's own (k, u, w) coordinates with component selects instead of indices (e is a lane number here, and a dynamic index
 // would put the vectors in local memory).  epen = r - distance if the edge qualifies, -1 otherwise; pa / pb = closest points
-// on the edge / on the segment, dir = normalised pa - pb, all in box coordinates.
+// on the edge / on the segment, dir = normalised pa - pb, all in box coordinates.  TEST = false: the caller knows the edge passes the
+// interval test (capbox_edge_mask), which is then not evaluated again.
 struct EdgeEval { float epen, deg, dir[3], pa[3], pb[3]; };
 KFN float pick3(const float* v, int k) { return k == 0 ? v[0] : (k == 1 ? v[1] : v[2]); }
 KFN void unpick3(float* out, int k, int u, float vk, float vu, float vw) {
   out[0] = k == 0 ? vk : (u == 0 ? vu : vw); out[1] = k == 1 ? vk : (u == 1 ? vu : vw); out[2] = k == 2 ? vk : (u == 2 ? vu : vw);
 }
+template <bool TEST = true>
 KFN EdgeEval capbox_edge_lane(int e, const float* a, const float* b, float r, const float* bsize) {
   EdgeEval out;
   out.epen = -1.f; out.deg = 0.f;
@@ -504,7 +509,7 @@ KFN EdgeEval capbox_edge_lane(int e, const float* a, const float* b, float r, co
   const float cu = eu * su, cw = ew * sw;
   const float fu = eu > 0.f ? hiu - cu : cu - lou, fw = ew > 0.f ? hiw - cw : cw - low;
   const float gu = eu > 0.f ? lou - cu : cu - hiu, gw = ew > 0.f ? low - cw : cw - hiw;
-  if (!(fu > 0.f && fw > 0.f && gu < r && gw < r && lok < sk + r && hik > -sk - r)) return out;
+  if (TEST && !(fu > 0.f && fw > 0.f && gu < r && gw < r && lok < sk + r && hik > -sk - r)) return out;
   // closest points of the edge and the segment (same formulas as capbox_edges), vectors as (k, u, w) triples
   const float abk = bk - ak, abu = bu - au, abw = bw - aw;
   const float den = abk * abk + abu * abu + abw * abw + 1e-6f;
@@ -541,6 +546,26 @@ KFN EdgeEval capbox_edge_lane(int e, const float* a, const float* b, float r, co
   unpick3(out.pa, k, u, pa[0], pa[1], pa[2]);
   unpick3(out.pb, k, u, pb[0], pb[1], pb[2]);
   return out;
+}
+// The edges that pass capbox_edge_lane's interval test: bit e set iff edge e does (the others return epen = -1, which never
+// becomes the contact).  The same comparisons, evaluated once per face: bit 2 j + (s > 0) of `face` says the segment reaches past
+// face (j, s) and comes within r of its plane, bit j of `along` that it overlaps the r-inflated extent of axis j.
+KFN int capbox_edge_mask(const float* a, const float* b, float r, const float* bsize) {
+  int face = 0, along = 0;
+#pragma unroll
+  for (int j = 0; j < 3; ++j) {
+    const float lo = fminf(a[j], b[j]), hi = fmaxf(a[j], b[j]), s = bsize[j], cn = -1.f * s;
+    if (hi - s > 0.f && lo - s < r) face |= 2 << (2 * j);
+    if (cn - lo > 0.f && cn - hi < r) face |= 1 << (2 * j);
+    if (lo < s + r && hi > -s - r) along |= 1 << j;
+  }
+  int mask = 0;
+#pragma unroll
+  for (int e = 0; e < 12; ++e) {
+    const int k = e >> 2, u = k == 2 ? 0 : k + 1, w = k == 0 ? 2 : k - 1;
+    if (((along >> k) & 1) && ((face >> (2 * u + ((e >> 1) & 1))) & 1) && ((face >> (2 * w + (e & 1))) & 1)) mask |= 1 << e;
+  }
+  return mask;
 }
 template <bool FULL>
 KFN void capsule_box(const float* A, const float* B, float r, const float* bpos, const float* bmat, const float* bsize, Contact2& c) {
@@ -1822,10 +1847,11 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
       for (int i0 = 0; warp_any_groups(W, i0 < ntot); i0 += KW) {
         const long long tk0 = TICK(); (void)tk0;
         // (1) one near pair per lane: the face part of the collider (both slots, in box coordinates; parked in R.h); the
-        //     pairs that need the edge stage leave their box-frame geometry in S.estage
+        //     pairs that need the edge stage leave their box-frame geometry in S.estage and their candidate edges in R.off
         LANES(W, R)
           const int i = i0 + lane;
-          R.nact = 0;
+          R.off = 0;
+          R.f2 = -1.f;                           // best edge penetration so far (only a positive one can become the contact)
           if (i < ntot) {
             const int e = S.nlist[i] & 0x3fff, x = m.rp[e], a = KP_A(x), b = KP_B(x);
             const bool st = b < m.nsbox;
@@ -1839,65 +1865,82 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
             for (int k = 0; k < 3; ++k) { R.h[k] = c.pos[0][k]; R.h[3 + k] = c.nrm[0][k]; R.h[6 + k] = c.pos[1][k]; R.h[9 + k] = c.nrm[1][k]; }
             R.f0 = c.dist[0]; R.f1 = c.dist[1];
             if (nout >= 2) {
-              R.nact = 1;
+              R.off = capbox_edge_mask(la, lb, m.cap_r[a], bsz);
               float* g = S.estage[lane];
               g[0] = la[0]; g[1] = la[1]; g[2] = la[2]; g[3] = lb[0]; g[4] = lb[1]; g[5] = lb[2];
               g[6] = bsz[0]; g[7] = bsz[1]; g[8] = bsz[2]; g[9] = m.cap_r[a]; g[10] = nf[0]; g[11] = nf[1]; g[12] = nf[2];
             }
           }
         END_LANES
-        // (2) the shallow edge contact of those pairs (MJX: closest box edge in front of two faces, see capbox_edges):
-        //     the 12 edges of a pair on 12 lanes, first maximum of the penetration by a lane reduction
-        const unsigned emine = warp_ballot(W, [](int, LaneRegs& R) { return R.nact != 0; });
+        // (2) the shallow edge contact of those pairs (MJX: closest box edge in front of two faces, see capbox_edges).  The
+        //     candidate edges of all pairs of the group are items in (list slot, edge) order, dealt KW per round over the lanes,
+        //     so a round serves every pair at once.  A pair's items are consecutive, in ascending edge order, and its owner folds
+        //     them in that order keeping strictly greater penetrations: the first maximum, as capbox_edges and a lane argmax.
+        const int nitem = warp_excl_scan(W, [](int, LaneRegs& R) { return KPOPC(R.off); }, [](int, LaneRegs& R, int o) { R.actmask = o; });
+        if (warp_any_groups(W, nitem > 0)) {
+          LANES(W, R)
+            int it = R.actmask;
 #pragma unroll 1
-        for (unsigned rem = warp_or_groups(W, emine); rem != 0u; rem &= rem - 1u) {
-          const int q = KFFS(rem) - 1;
-          const bool mine = (emine >> q) & 1u;
-          LANES(W, R)
-            R.f2 = -INFINITY;
-            if (mine && lane < 12) {
-              const float* g = S.estage[q];
-              const EdgeEval e1 = capbox_edge_lane(lane, g, g + 3, g[9], g + 6);
-              R.f2 = e1.epen;
-              if (e1.epen > 0.f) {                 // (only a positive penetration can become the contact: park the candidate)
-                R.acc[0] = e1.dir[0]; R.acc[1] = e1.dir[1]; R.acc[2] = e1.dir[2];
-                R.acc[3] = 0.5f * (e1.pa[0] + e1.pb[0] + e1.dir[0] * g[9]); R.acc[4] = 0.5f * (e1.pa[1] + e1.pb[1] + e1.dir[1] * g[9]);
-                R.acc[5] = 0.5f * (e1.pa[2] + e1.pb[2] + e1.dir[2] * g[9]);
+            for (int rem = R.off; rem; rem &= rem - 1, ++it) S.eidx[it] = (unsigned short)((lane << 4) | (KFFS(rem) - 1));
+          END_LANES
+#pragma unroll 1
+          for (int base = 0; warp_any_groups(W, base < nitem); base += KW) {
+            LANES(W, R)
+              const int it = base + lane;
+              if (it < nitem) {
+                const int q = S.eidx[it] >> 4;
+                const float* g = S.estage[q];
+                const EdgeEval e1 = capbox_edge_lane<false>(S.eidx[it] & 15, g, g + 3, g[9], g + 6);
+                float* o = S.eres[lane];
+                o[0] = e1.epen;
+                if (e1.epen > 0.f) {
+                  o[1] = e1.dir[0]; o[2] = e1.dir[1]; o[3] = e1.dir[2];
+                  o[4] = 0.5f * (e1.pa[0] + e1.pb[0] + e1.dir[0] * g[9]); o[5] = 0.5f * (e1.pa[1] + e1.pb[1] + e1.dir[1] * g[9]);
+                  o[6] = 0.5f * (e1.pa[2] + e1.pb[2] + e1.dir[2] * g[9]);
+                }
               }
-            }
-          END_LANES
-          const int bl = warp_argmax_first(W, [](int, LaneRegs& R) { return R.f2; });
-          LANES(W, R)
-            if (mine && lane == bl) {
-              float* g = S.eres[q];
-              g[0] = R.f2;
-              if (R.f2 > 0.f) { g[1] = R.acc[0]; g[2] = R.acc[1]; g[3] = R.acc[2]; g[4] = R.acc[3]; g[5] = R.acc[4]; g[6] = R.acc[5]; }
-            }
-          END_LANES
+            END_LANES
+            // the owner folds its items of this round (parked in R.f2 / R.acc[0..5]); after its last one, edge contact or not
+            LANES(W, R)
+              const int lo = R.actmask > base ? R.actmask : base, end = R.actmask + KPOPC(R.off);
+#pragma unroll 1
+              for (int it = lo; it < end && it < base + KW; ++it) {
+                const float* o = S.eres[it - base];
+                if (o[0] > R.f2) {
+                  R.f2 = o[0];
+                  if (o[0] > 0.f) { R.acc[0] = o[1]; R.acc[1] = o[2]; R.acc[2] = o[3]; R.acc[3] = o[4]; R.acc[4] = o[5]; R.acc[5] = o[6]; }
+                }
+              }
+              if (end > base && end <= base + KW && R.f2 > 0.f) {
+                const float* nf = S.estage[lane] + 10;
+                const float bpen = R.f2, minface = fminf(-R.f0, -R.f1);
+                const bool parallel = fabsf(R.acc[0] * nf[0] + R.acc[1] * nf[1] + R.acc[2] * nf[2]) > 0.99f;
+                if ((minface > 0.f ? bpen < minface : true) && !parallel) {
+                  R.f0 = -bpen;
+                  R.h[0] = R.acc[3]; R.h[1] = R.acc[4]; R.h[2] = R.acc[5]; R.h[3] = R.acc[0]; R.h[4] = R.acc[1]; R.h[5] = R.acc[2];
+                }
+              }
+            END_LANES
+          }
         }
-        // (3) back on the pair's lane: edge contact or not, the pair's share of the collision cost, its previous-distance
-        //     record, world position and normal of the penetrating slots
+        RLANES(W, R)
+          R.nact = i0 + lane < ntot ? (R.f0 < 0.f ? 1 : 0) + (R.f1 < 0.f ? 2 : 0) : 0;
+#ifdef CEMK_X_NEARNOCON
+          R.nact = 0;   // timing experiment only (wrong results): near pass without the contacts it finds
+#endif
+        END_RLANES
+        const long long tk1 = TICK(); (void)tk1;
+        EVENT(W, 14, (int)(tk1 - tk0));
+        // (3) back on the pair's lane, its contacts' list positions known: the pair's share of the collision cost, its
+        //     previous-distance record, world position and normal of the penetrating slots and their contact records
+        const int nnew = warp_excl_scan(W, [](int, LaneRegs& R) { return (R.nact & 1) + (R.nact >> 1); }, [](int, LaneRegs& R, int o) { R.actmask = o; });
         LANES(W, R)
           const int i = i0 + lane;
-          const bool edges = R.nact != 0;
-          R.nact = 0;
           if (i < ntot) {
             const int e = S.nlist[i] & 0x3fff, x = m.rp[e], a = KP_A(x), b = KP_B(x);
             const bool wasfar = (S.nlist[i] >> 15) != 0, pref = ((S.nlist[i] >> 14) & 1) != 0, st = b < m.nsbox;
             const float* bpos = st ? m.sb_pos[b] : S.qpos + KM_NL;
             const float* bmat = st ? m.sb_mat[b] : S.bmat;
-            if (edges) {
-              const float* g = S.eres[lane];
-              const float* nf = S.estage[lane] + 10;
-              const float bpen = g[0], minface = fminf(-R.f0, -R.f1);
-              if (bpen > 0.f) {
-                const bool parallel = fabsf(g[1] * nf[0] + g[2] * nf[1] + g[3] * nf[2]) > 0.99f;
-                if ((minface > 0.f ? bpen < minface : true) && !parallel) {
-                  R.f0 = -bpen;
-                  R.h[0] = g[4]; R.h[1] = g[5]; R.h[2] = g[6]; R.h[3] = g[1]; R.h[4] = g[2]; R.h[5] = g[3];
-                }
-              }
-            }
             const float d0 = R.f0, d1 = R.f1;
             float cc = (d0 < 0.f ? 1.f : 0.f) + (d1 < 0.f ? 1.f : 0.f);
             float* pd = io.prevd + (2 * (e / KW)) * KW + (e & (KW - 1));       // the owner's slots: pass e / KW, capsule lane e % KW
@@ -1908,10 +1951,6 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
             pd[0] = d0; pd[KW] = d1;
             if (io.collision_row) { io.collision_row[KP_SLOT(x)] = d0; io.collision_row[KP_SLOT(x) + 1] = d1; }
             R.cost_c += cc;                        // (cost_c is summed over the lanes at the end of the rollout: any lane may book a pair)
-            R.nact = (d0 < 0.f ? 1 : 0) + (d1 < 0.f ? 2 : 0);
-#ifdef CEMK_X_NEARNOCON
-            R.nact = 0;   // timing experiment only (wrong results): near pass without the contacts it finds
-#endif
             if (R.nact) {
               // world position and normal of both slots: box frame -> world
 #pragma unroll
@@ -1924,24 +1963,14 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
                 R.h[6 * j] = w[0]; R.h[6 * j + 1] = w[1]; R.h[6 * j + 2] = w[2];
                 R.h[6 * j + 3] = nw[0]; R.h[6 * j + 4] = nw[1]; R.h[6 * j + 5] = nw[2];
               }
-              R.f2 = m.cap_invw[a] + (st ? 0.f : m.fb_invw);
-              R.tri = (R.tri & 0xffff) | (m.cap_link[a] << 16) | ((st ? 15 : KM_NL) << 20);     // links of the pair, parked above the triangle entries
+              const float invw = m.cap_invw[a] + (st ? 0.f : m.fb_invw);
+              const int l1 = m.cap_link[a], l2 = st ? -1 : KM_NL;
+              int o = ncbcon + R.actmask;
+              if (R.nact & 1) { put_contact<NC>(S, o, R.h, R.h + 3, nullptr, d0, invw, l1, l2); ++o; }
+              if (R.nact & 2) put_contact<NC>(S, o, R.h + 6, R.h + 9, nullptr, d1, invw, l1, l2);
             }
           }
         END_LANES
-        const long long tk1 = TICK(); (void)tk1;
-        EVENT(W, 14, (int)(tk1 - tk0));
-        const int nnew = warp_excl_scan(W, [](int, LaneRegs& R) { return (R.nact & 1) + (R.nact >> 1); }, [](int, LaneRegs& R, int o) { R.actmask = o; });
-        if (warp_any_groups(W, nnew > 0)) {
-          LANES(W, R)
-            if (R.nact) {
-              const int l1 = (R.tri >> 16) & 15, l2raw = (R.tri >> 20) & 15, l2 = l2raw == 15 ? -1 : l2raw;
-              int o = ncbcon + R.actmask;
-              if (R.nact & 1) { put_contact<NC>(S, o, R.h, R.h + 3, nullptr, R.f0, R.f2, l1, l2); ++o; }
-              if (R.nact & 2) put_contact<NC>(S, o, R.h + 6, R.h + 9, nullptr, R.f1, R.f2, l1, l2);
-            }
-          END_LANES
-        }
         ncbcon += nnew;
         EVENT(W, 15, (int)(TICK() - tk1));
       }
