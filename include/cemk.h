@@ -15,7 +15,7 @@
  *     nc = Bernstein coefficients per DOF (cemk_set_order, default 11), NV = nvar = nd * nc decision variables.
  *     "66", "30" and "6T" in the shapes below are NV, 5 nd and nd T at the defaults.
  *   - The planner algebra (sampling, projection, elite selection, mean / covariance) runs at any
- *     1 <= nd <= 12 and 4 <= nc <= 16 (NV <= 192).  The rollout (cemk_rollout_cost, cemk_tick_record)
+ *     1 <= nd <= 12 and 4 <= nc <= 16 (NV <= 192).  The rollout (cemk_rollout_cost, cemk_step_states, cemk_tick_record)
  *     models the 6-DOF arm of the KModel only and returns CEMK_ERR_ARG on a handle with nd != 6.
  */
 #ifndef CEMK_H
@@ -88,6 +88,18 @@ int cemk_rollout_cost(cemk_handle* h, int B, int T, const float* thetadot, const
                       const float* target_pos, const float* target_rot, float w_pos, float w_rot, float w_col,
                       float* theta, float* cost4, float* eef_pos, float* eef_rot, float* collision, float* qacc,
                       int* flags, void* stream);
+
+/* vmap(mjx.step) over N environments, each from its own state, chained over T steps (the rollout body of
+ * cemk_rollout_cost without the cost and without the handle's KModel snapshot, which is neither read nor changed):
+ *   qpos[N][13], qvel[N][12], warm[N][12] (qacc_warmstart) -> qpos_out, qvel_out, warm_out (same shapes) after T steps.
+ *   thetadot[N][6T] (dof-major as in cemk_rollout_cost) overwrites qvel[:6] before each step (mjx_planner.py:254); NULL is
+ *   allowed with T = 1 only, each environment then keeps its own qvel[:6] (a plain mjx.step).  Outputs may be the inputs
+ *   (in-place stepping).  warm_out is the last step's qacc.  Optional (NULL to skip): theta[N][6T] and the dumps and flags
+ *   of cemk_rollout_cost.  A run split into chunks, each fed the previous chunk's outputs, gives the same bits as one call.
+ *   CEMK_ERR_ARG for N <= 0, T <= 0, a missing state pointer, NULL thetadot with T > 1, or a handle with nd != 6. */
+int cemk_step_states(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm,
+                     const float* thetadot, float* qpos_out, float* qvel_out, float* warm_out, float* theta,
+                     float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags, void* stream);
 
 /* compute_cost_batch alone (mjx_planner.py:277-303), per-sample targets as in the reference method:
  *   eef_pos[B][T][3], eef_rot[B][T][4], collision[B][T][nslot], target_pos[B][3], target_rot[B][4] -> cost4[B][4]. */

@@ -47,6 +47,7 @@ _SIGS = {
     "cemk_jax_normal": ([_vp, C.c_uint, C.c_uint, _i, C.c_uint, C.c_uint, C.c_uint, _vp, _vp], _i),
     "cemk_project": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp], _i),
     "cemk_rollout_cost": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
+    "cemk_step_states": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
     "cemk_cost_batch": ([_vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp], _i),
     "cemk_argsort_topk": ([_vp, _i, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp], _i),
     "cemk_topk_pack": ([_vp, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp], _i),

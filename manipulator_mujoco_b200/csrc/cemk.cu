@@ -4,6 +4,7 @@
 //   k_jax_normal / k_chol66 | k_chol_wide / k_sample   compute_xi_samples  (:313-316)
 //   k_project                compute_projection_filter + A_thetadot @ xi   (:181-249, :348)
 //   k_rollout                vmap(scan(mjx.step)) + compute_cost_batch     (:251-303)   <- hot kernel
+//   k_rollout<.., STATES>    vmap(mjx.step) over per-environment states, chained T steps (cemk_step_states)
 //   k_cost_batch             compute_cost_batch on materialised trajectories (:277-303)
 //   k_rank_select (n <= 8192) | k_make_keys / k_bitonic* / k_gather_sorted    compute_ellite_samples   (:306-310)
 //   k_merge_lists            the same selection over the per-rank sorted lists of several GPUs
@@ -86,14 +87,18 @@ struct RolloutBatch {
   // CTA -> samples: the first n_hi CTAs run w_hi samples each, the others w_lo (both <= the launch width);
   // warps beyond a CTA's share exit at once
   int n_hi, w_hi, w_lo;
+  // cemk_step_states (STATES): q0 / v0 are then qpos [B][13] / qvel [B][12], and warm [B][12] is the third state input
+  const float* warm;
+  float* qpos_out; float* qvel_out; float* warm_out;
 };
 
 // NC = contacts of a sample kept in shared memory (the rest, up to KM_NC_TOT, in the global spill area),
 // WARPS = warps per CTA; a warp carries 32 / KW samples (one per lane group, warp_dsl.h).  The fast
 // instantiation (NC = KM_NC_FAST) is the product path.  ONLY_FLAGGED is the debug instantiation behind
 // cemk_set_option("force_rerun"): NC = 48 (no spill area), one warp per CTA, samples whose flag bit 0 is set.
+// STATES: every sample steps from its own state rows and writes its final state (cemk_step_states, rollout_sample).
 #define GPW (32 / KW)                                     // lane groups (samples) per warp
-template <int NC, int WARPS, bool ONLY_FLAGGED>
+template <int NC, int WARPS, bool ONLY_FLAGGED, bool STATES = false>
 __global__ void __launch_bounds__(WARPS * 32, ROLLOUT_MINB) k_rollout(const KModel* __restrict__ gm, RolloutBatch a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   KModel* sm = reinterpret_cast<KModel*>(smem_raw);
@@ -138,11 +143,17 @@ __global__ void __launch_bounds__(WARPS * 32, ROLLOUT_MINB) k_rollout(const KMod
   const size_t row = (size_t)s * KM_NL * a.T;
   A.T = a.T;
   A.live = true;
-  A.thetadot = a.thetadot + row;
-  A.q0 = a.q0; A.v0 = a.v0; A.target_pos = a.target_pos; A.target_rot = a.target_rot;
+  A.thetadot = (STATES && !a.thetadot) ? nullptr : a.thetadot + row;
+  if (STATES) {
+    A.q0 = a.q0 + (size_t)s * KM_NQ; A.v0 = a.v0 + (size_t)s * KM_NV; A.warm0 = a.warm + (size_t)s * KM_NV;
+    A.qpos_out = a.qpos_out + (size_t)s * KM_NQ; A.qvel_out = a.qvel_out + (size_t)s * KM_NV; A.warm_out = a.warm_out + (size_t)s * KM_NV;
+  } else {
+    A.q0 = a.q0; A.v0 = a.v0;
+  }
+  A.target_pos = a.target_pos; A.target_rot = a.target_rot;
   A.w_pos = a.w_pos; A.w_rot = a.w_rot; A.w_col = a.w_col;
-  A.theta = a.theta + row;
-  A.cost4 = a.cost4 + (size_t)s * 4;
+  A.theta = (STATES && !a.theta) ? nullptr : a.theta + row;
+  A.cost4 = STATES ? nullptr : a.cost4 + (size_t)s * 4;
   A.eef_pos = a.eef_pos ? a.eef_pos + (size_t)s * a.T * 3 : nullptr;
   A.eef_rot = a.eef_rot ? a.eef_rot + (size_t)s * a.T * 4 : nullptr;
   A.collision = a.collision ? a.collision + (size_t)s * a.T * sm->nslot_robot : nullptr;
@@ -150,7 +161,7 @@ __global__ void __launch_bounds__(WARPS * 32, ROLLOUT_MINB) k_rollout(const KMod
   A.flags = a.flags + s;
   A.prevd = a.prevd + (size_t)s * (2 * KM_NPASS * KW);
   A.ovf = a.ovf + (size_t)s * ((KM_NC_TOT - KM_NC_FAST) * KM_OVF_STRIDE);
-  rollout_sample<NC>(W, *sm, ws[group], A);
+  rollout_sample<NC, STATES>(W, *sm, ws[group], A);
 #ifdef CEMK_PHASE_TIMING
   PHASE(W, 15);
   if (W.lane == 0 && !ONLY_FLAGGED) for (int i = 0; i < 24; ++i) atomicAdd(&g_phase[i], (unsigned long long)W.ph[i]);
@@ -951,9 +962,67 @@ static int rollout_dof_check(const cemk_handle* h, const char* fn) {
   return CEMK_ERR_ARG;
 }
 
+// One launch of the product rollout over a.B samples (cemk_rollout_cost, and cemk_step_states with STATES): grows the
+// library scratch to a.B samples (the flags when a.flags is null, the previous distances, the spill area), points `a` at it
+// and chooses the CTA shares.
+template <bool STATES>
+static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
+  const int B = a.B;
+  if (!a.flags) {
+    if (h->flags_cap < B) {
+      if (h->d_flags) CK(cudaFree(h->d_flags));
+      CK(cudaMalloc(&h->d_flags, sizeof(int) * B));
+      h->flags_cap = B;
+    }
+    a.flags = h->d_flags;
+  }
+  if (h->prevd_cap < B) {
+    if (h->d_prevd) CK(cudaFree(h->d_prevd));
+    CK(cudaMalloc(&h->d_prevd, sizeof(float) * (size_t)B * 2 * KM_NPASS * KW));
+    if (h->d_ovf) CK(cudaFree(h->d_ovf));
+    CK(cudaMalloc(&h->d_ovf, sizeof(float) * (size_t)B * (KM_NC_TOT - KM_NC_FAST) * KM_OVF_STRIDE));
+    h->prevd_cap = B;
+  }
+  a.prevd = h->d_prevd;
+  a.ovf = h->d_ovf;
+  // Samples per CTA (a warp carries GPW = 32 / KW of them).  One CTA is resident per SM and its warps step
+  // in lockstep, so the time of a wave grows with the warps per SM sub-partition (4 schedulers):
+  //  * up to 4 / 8 warps-worth of samples per SM: the 4- / 8-warp instantiations (more registers per
+  //    thread, latency-bound regime, e.g. the closed-loop config B = 1000);
+  //  * one wave: every SM gets ceil(B / SMs) samples;
+  //  * several waves: the ceil(B / SMs) samples an SM has to run are split into `waves` shares counted in
+  //    units of 4 warps where that fits the CTA capacity, otherwise evenly.
+  const int nsm = h->num_sms > 0 ? h->num_sms : 148;
+  const int cap = ROLLOUT_WARPS * GPW, unit = 4 * GPW;
+  int grid;
+#define CEMK_LAUNCH_ROLLOUT(W_) k_rollout<KM_NC_FAST, W_, false, STATES><<<grid, (W_) * 32, rollout_smem<KM_NC_FAST, W_>(), st>>>(h->d_model, a)
+  const int need = (B + nsm - 1) / nsm;                            // samples per SM
+  if (h->cta_samples > 0) {
+    const int w = h->cta_samples < cap ? h->cta_samples : cap;
+    a.n_hi = 0; a.w_hi = a.w_lo = w; grid = (B + w - 1) / w;
+    CEMK_LAUNCH_ROLLOUT(ROLLOUT_WARPS);
+  } else if (need <= cap) {
+    a.n_hi = 0; a.w_hi = a.w_lo = need; grid = (B + need - 1) / need;
+    if (need <= 4 * GPW) CEMK_LAUNCH_ROLLOUT(4);
+    else if (need <= 8 * GPW) CEMK_LAUNCH_ROLLOUT(8);
+    else CEMK_LAUNCH_ROLLOUT(ROLLOUT_WARPS);
+  } else {
+    const int waves = (need + cap - 1) / cap;
+    const int units = (need + unit - 1) / unit, u_lo = units / waves, r = units % waves;
+    a.w_lo = unit * u_lo; a.w_hi = unit * (u_lo + (r ? 1 : 0)); a.n_hi = r * nsm;
+    if (a.w_hi > cap || a.w_lo == 0) { a.n_hi = 0; a.w_hi = a.w_lo = (need + waves - 1) / waves; }
+    const int rest = B - a.n_hi * a.w_hi;
+    grid = a.n_hi + (rest > 0 ? (rest + a.w_lo - 1) / a.w_lo : 0);
+    CEMK_LAUNCH_ROLLOUT(ROLLOUT_WARPS);
+  }
+#undef CEMK_LAUNCH_ROLLOUT
+  h->launches += 1;
+  return CEMK_OK;
+}
+
 extern "C" {
 
-int cemk_version(void) { return 3; }
+int cemk_version(void) { return 4; }
 const char* cemk_last_error(void) { return g_err; }
 int cemk_sizeof_kmodel(void) { return (int)sizeof(KModel); }
 
@@ -974,6 +1043,10 @@ int cemk_create(const void* kmodel, int kmodel_bytes, int device, cemk_handle** 
                           (int)rollout_smem<KM_NC_FAST, ROLLOUT_WARPS>()));
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 8>()));
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 4>()));
+  CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, ROLLOUT_WARPS, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)rollout_smem<KM_NC_FAST, ROLLOUT_WARPS>()));
+  CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 8, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 8>()));
+  CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 4, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 4>()));
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_BIG, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                           (int)rollout_smem<KM_NC_BIG, 1>()));
   h->d_mc = nullptr;
@@ -1089,66 +1162,37 @@ int cemk_rollout_cost(cemk_handle* h, int B, int T, const float* thetadot, const
   { const int rc = rollout_dof_check(h, "cemk_rollout_cost"); if (rc) return rc; }
   DevGuard guard(h->device);
   cudaStream_t st = (cudaStream_t)stream;
-  if (!flags) {
-    if (h->flags_cap < B) {
-      if (h->d_flags) CK(cudaFree(h->d_flags));
-      CK(cudaMalloc(&h->d_flags, sizeof(int) * B));
-      h->flags_cap = B;
-    }
-    flags = h->d_flags;
-  }
-  RolloutBatch a;
+  RolloutBatch a = {};
   a.B = B; a.T = T; a.thetadot = thetadot; a.q0 = q0; a.v0 = v0; a.target_pos = target_pos; a.target_rot = target_rot;
   a.w_pos = w_pos; a.w_rot = w_rot; a.w_col = w_col;
   a.theta = theta; a.cost4 = cost4; a.eef_pos = eef_pos; a.eef_rot = eef_rot; a.collision = collision; a.qacc = qacc; a.flags = flags;
-  if (h->prevd_cap < B) {
-    if (h->d_prevd) CK(cudaFree(h->d_prevd));
-    CK(cudaMalloc(&h->d_prevd, sizeof(float) * (size_t)B * 2 * KM_NPASS * KW));
-    if (h->d_ovf) CK(cudaFree(h->d_ovf));
-    CK(cudaMalloc(&h->d_ovf, sizeof(float) * (size_t)B * (KM_NC_TOT - KM_NC_FAST) * KM_OVF_STRIDE));
-    h->prevd_cap = B;
-  }
-  a.prevd = h->d_prevd;
-  a.ovf = h->d_ovf;
-  // Samples per CTA (a warp carries GPW = 32 / KW of them).  One CTA is resident per SM and its warps step
-  // in lockstep, so the time of a wave grows with the warps per SM sub-partition (4 schedulers):
-  //  * up to 4 / 8 warps-worth of samples per SM: the 4- / 8-warp instantiations (more registers per
-  //    thread, latency-bound regime, e.g. the closed-loop config B = 1000);
-  //  * one wave: every SM gets ceil(B / SMs) samples;
-  //  * several waves: the ceil(B / SMs) samples an SM has to run are split into `waves` shares counted in
-  //    units of 4 warps where that fits the CTA capacity, otherwise evenly.
-  const int nsm = h->num_sms > 0 ? h->num_sms : 148;
-  const int cap = ROLLOUT_WARPS * GPW, unit = 4 * GPW;
-  int grid;
-#define CEMK_LAUNCH_ROLLOUT(W_) k_rollout<KM_NC_FAST, W_, false><<<grid, (W_) * 32, rollout_smem<KM_NC_FAST, W_>(), st>>>(h->d_model, a)
-  const int need = (B + nsm - 1) / nsm;                            // samples per SM
-  if (h->cta_samples > 0) {
-    const int w = h->cta_samples < cap ? h->cta_samples : cap;
-    a.n_hi = 0; a.w_hi = a.w_lo = w; grid = (B + w - 1) / w;
-    CEMK_LAUNCH_ROLLOUT(ROLLOUT_WARPS);
-  } else if (need <= cap) {
-    a.n_hi = 0; a.w_hi = a.w_lo = need; grid = (B + need - 1) / need;
-    if (need <= 4 * GPW) CEMK_LAUNCH_ROLLOUT(4);
-    else if (need <= 8 * GPW) CEMK_LAUNCH_ROLLOUT(8);
-    else CEMK_LAUNCH_ROLLOUT(ROLLOUT_WARPS);
-  } else {
-    const int waves = (need + cap - 1) / cap;
-    const int units = (need + unit - 1) / unit, u_lo = units / waves, r = units % waves;
-    a.w_lo = unit * u_lo; a.w_hi = unit * (u_lo + (r ? 1 : 0)); a.n_hi = r * nsm;
-    if (a.w_hi > cap || a.w_lo == 0) { a.n_hi = 0; a.w_hi = a.w_lo = (need + waves - 1) / waves; }
-    const int rest = B - a.n_hi * a.w_hi;
-    grid = a.n_hi + (rest > 0 ? (rest + a.w_lo - 1) / a.w_lo : 0);
-    CEMK_LAUNCH_ROLLOUT(ROLLOUT_WARPS);
-  }
-#undef CEMK_LAUNCH_ROLLOUT
-  h->launches += 1;
+  { const int rc = launch_rollout<false>(h, a, st); if (rc) return rc; }
   // debug option: recompute every sample with the all-in-shared-memory instantiation (no spill area)
   if (h->force_rerun) {
-    CK(cudaMemsetAsync(flags, 1, sizeof(int) * B, st));                        // 0x01010101: bit 0 set
+    CK(cudaMemsetAsync(a.flags, 1, sizeof(int) * B, st));                      // 0x01010101: bit 0 set
     a.n_hi = 0; a.w_hi = a.w_lo = GPW;
     k_rollout<KM_NC_BIG, 1, true><<<(B + GPW - 1) / GPW, 32, rollout_smem<KM_NC_BIG, 1>(), st>>>(h->d_model, a);
     h->launches += 1;
   }
+  CK(cudaPeekAtLastError());
+  return CEMK_OK;
+}
+
+// force_rerun does not apply here: it re-reads the samples' inputs after the product launch, and with in-place outputs
+// those rows already hold the stepped states.
+int cemk_step_states(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm, const float* thetadot,
+                     float* qpos_out, float* qvel_out, float* warm_out, float* theta, float* eef_pos, float* eef_rot, float* collision,
+                     float* qacc, int* flags, void* stream) {
+  if (!h || !qpos || !qvel || !warm || !qpos_out || !qvel_out || !warm_out || N <= 0 || T <= 0)
+    return set_err(CEMK_ERR_ARG, "cemk_step_states: bad argument");
+  if (!thetadot && T > 1) return set_err(CEMK_ERR_ARG, "cemk_step_states: thetadot may only be NULL with T = 1");
+  { const int rc = rollout_dof_check(h, "cemk_step_states"); if (rc) return rc; }
+  DevGuard guard(h->device);
+  RolloutBatch a = {};
+  a.B = N; a.T = T; a.thetadot = thetadot; a.q0 = qpos; a.v0 = qvel; a.warm = warm;
+  a.qpos_out = qpos_out; a.qvel_out = qvel_out; a.warm_out = warm_out;
+  a.theta = theta; a.eef_pos = eef_pos; a.eef_rot = eef_rot; a.collision = collision; a.qacc = qacc; a.flags = flags;
+  { const int rc = launch_rollout<true>(h, a, (cudaStream_t)stream); if (rc) return rc; }
   CK(cudaPeekAtLastError());
   return CEMK_OK;
 }

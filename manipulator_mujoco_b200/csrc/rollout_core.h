@@ -2131,21 +2131,33 @@ struct RolloutArgs {
   int* flags;
   float* prevd;               // scratch [2 * KM_NPASS][KW] of this sample (StepIO::prevd)
   float* ovf;                 // spill area [KM_NC_TOT - NC][KM_OVF_STRIDE] of this sample (WarpSmemT::ovf)
+  // STATES only: q0 / v0 are this sample's qpos [13] / qvel [12] rows, warm0 its qacc_warmstart [12]; the state after the
+  // last step goes to the *_out rows (they may be the input rows: a sample reads its rows before it writes them)
+  const float* warm0;
+  float* qpos_out; float* qvel_out; float* warm_out;
 };
 
-template <int NC>
+// STATES = false: a planner rollout from the KModel snapshot (arm state q0 / v0, shared by all samples) with its cost.
+// STATES = true: the same steps from the sample's own state rows, which it writes back after the last step; thetadot
+// may be null with T = 1 (the sample keeps its own qvel[:6], a plain mjx.step), theta is optional, no cost, no target.
+template <int NC, bool STATES = false>
 KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const RolloutArgs& A) {
   LANES(W, R)
-    if (lane < KM_NQ) S.qpos[lane] = lane < KM_NL ? A.q0[lane] : m.qpos0[lane];
-    if (lane < KM_NV) { S.qvel[lane] = lane < KM_NL ? A.v0[lane] : m.qvel0[lane]; S.warm[lane] = m.warm0[lane]; }
+    if (STATES) {
+      if (lane < KM_NQ) S.qpos[lane] = A.q0[lane];
+      if (lane < KM_NV) { S.qvel[lane] = A.v0[lane]; S.warm[lane] = A.warm0[lane]; }
+    } else {
+      if (lane < KM_NQ) S.qpos[lane] = lane < KM_NL ? A.q0[lane] : m.qpos0[lane];
+      if (lane < KM_NV) { S.qvel[lane] = lane < KM_NL ? A.v0[lane] : m.qvel0[lane]; S.warm[lane] = m.warm0[lane]; }
+    }
     R.tri = tri_entries(lane);
     if (lane == 0) { S.flags = 0; S.ovf = A.ovf; }
     R.cost_c = 0.f;
     R.farprev = 0;
-    R.td = lane < KM_NL ? A.thetadot[lane * A.T] : 0.f;
+    R.td = lane < KM_NL ? ((!STATES || A.thetadot) ? A.thetadot[lane * A.T] : A.v0[lane]) : 0.f;
   END_LANES
-  const float tp[3] = {A.target_pos[0], A.target_pos[1], A.target_pos[2]};       // read once: the step loop only touches registers for the goal terms
-  float tq[4] = {A.target_rot[0], A.target_rot[1], A.target_rot[2], A.target_rot[3]};
+  const float tp[3] = {STATES ? 0.f : A.target_pos[0], STATES ? 0.f : A.target_pos[1], STATES ? 0.f : A.target_pos[2]};   // read once: the step loop only touches registers for the goal terms
+  float tq[4] = {STATES ? 1.f : A.target_rot[0], STATES ? 0.f : A.target_rot[1], STATES ? 0.f : A.target_rot[2], STATES ? 0.f : A.target_rot[3]};
   {
     float inv = 1.f / sqrtf(tq[0] * tq[0] + tq[1] * tq[1] + tq[2] * tq[2] + tq[3] * tq[3]);
     tq[0] *= inv; tq[1] *= inv; tq[2] *= inv; tq[3] *= inv;
@@ -2190,10 +2202,20 @@ KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const Rollou
     }
     step_euler<NC>(W, m, S);
     LANES(W, R)
-      if (A.live && lane < KM_NL) A.theta[lane * A.T + t] = S.qpos[lane];
+      if (A.live && lane < KM_NL && (!STATES || A.theta)) A.theta[lane * A.T + t] = S.qpos[lane];
     END_LANES
     PHASE(W, 12);
     STEPEND(W);
+  }
+  if (STATES) {
+    LANES(W, R)
+      if (A.live) {
+        if (lane < KM_NQ) A.qpos_out[lane] = S.qpos[lane];
+        if (lane < KM_NV) { A.qvel_out[lane] = S.qvel[lane]; A.warm_out[lane] = S.warm[lane]; }
+        if (lane == 0 && A.flags) *A.flags = S.flags;
+      }
+    END_LANES
+    return;
   }
   const float cost_c = warp_sum(W, [](int, LaneRegs& R) { return R.cost_c; });
   LANES(W, R)

@@ -484,6 +484,42 @@ class cem_planner:
         theta, _c, eef_pos, eef_rot, collision = self._rollout(thetadot, init_pos, init_vel, tp, tr, True)
         return theta, eef_pos, eef_rot, collision
 
+    def step_batch(self, qpos, qvel, qacc_warmstart, thetadot=None):
+        """``jax.vmap(jit_step, in_axes=(None, 0))``: N environments, each stepped from its own state in one launch
+        (``cemk_step_states``); the planner's model snapshot is not used or changed.  qpos [N, 13], qvel [N, 12],
+        qacc_warmstart [N, 12] (numpy or torch).  ``thetadot`` [N, 6T] (dof-major, the rollout's layout) chains T steps with
+        qvel[:6] set to thetadot[:, t] before step t (mjx_planner.py:254); without it each environment takes one plain step
+        with its own qvel.  Returns CUDA tensors: qpos, qvel, qacc (last step), qacc_warmstart (= that qacc), overflow [N]
+        (bool: more simultaneous contacts than the kernel keeps, extra ones dropped) and, with thetadot, theta [N, 6T]."""
+        self._require_rollout_dof("step_batch")
+        qp, qv, wm = self._t(qpos), self._t(qvel), self._t(qacc_warmstart)
+        if qp.dim() != 2 or qp.shape[1] != 13 or qp.shape[0] == 0:
+            raise ValueError(f"qpos must be [N, 13] with N >= 1, got {tuple(qp.shape)}")
+        N = qp.shape[0]
+        if tuple(qv.shape) != (N, 12) or tuple(wm.shape) != (N, 12):
+            raise ValueError(f"qvel and qacc_warmstart must be [{N}, 12], got {tuple(qv.shape)} and {tuple(wm.shape)}")
+        td, T, theta = None, 1, None
+        if thetadot is not None:
+            td = self._t(thetadot)
+            if td.dim() != 2 or td.shape[0] != N or td.shape[1] == 0 or td.shape[1] % 6:
+                raise ValueError(f"thetadot must be [{N}, 6T] with T >= 1, got {tuple(td.shape)}")
+            T = td.shape[1] // 6
+            theta = torch.empty(N, 6 * T, device=self.device)
+        dev = self.device
+        if self._graph is not None and N > self.num_batch_local:
+            # the library grows its rollout scratch to N samples and frees the old one, which the captured tick points at
+            torch.cuda.current_stream(dev).synchronize()
+            self._graph, self._graph_out, self._eager_ticks = None, None, 0
+        qpos_out, qvel_out, warm_out = torch.empty(N, 13, device=dev), torch.empty(N, 12, device=dev), torch.empty(N, 12, device=dev)
+        flags = torch.empty(N, dtype=torch.int32, device=dev)
+        _lib.check(self._lib.cemk_step_states(self._h, N, T, _ptr(qp), _ptr(qv), _ptr(wm), _ptr(td), _ptr(qpos_out), _ptr(qvel_out),
+                                              _ptr(warm_out), _ptr(theta), None, None, None, None, _ptr(flags), self._stream()), self._lib)
+        self._keep_sb = (qp, qv, wm, td)
+        out = dict(qpos=qpos_out, qvel=qvel_out, qacc=warm_out.clone(), qacc_warmstart=warm_out, overflow=(flags & 1).bool())
+        if theta is not None:
+            out["theta"] = theta
+        return out
+
     def compute_cost_batch(self, thetadot, eef_pos, eef_rot, collision, target_pos, target_rot):
         """mjx_planner.py:124,277-303 (thetadot is unused there too) -> cost, cost_g, cost_r, cost_c [B]."""
         ep, er, col = self._t(eef_pos), self._t(eef_rot), self._t(collision)
