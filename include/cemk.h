@@ -57,7 +57,9 @@ int cemk_set_order(cemk_handle* h, int ncoef);
 /* Per-horizon constants, host pointers, float32:
  *   G [3][T][nc] = Pdot, Pddot, P (bernstein_coeff_ordern_new, mjx_planner.py:40);
  *   Kpp [nc][nc], Kpe [nc][5] = per-DOF blocks of Q_inv (mjx_planner.py:166-172, block diagonal per DOF);
- *   bounds = v_max, a_max, p_max (mjx_planner.py:84-86). */
+ *   bounds = v_max, a_max, p_max (mjx_planner.py:84-86).
+ * 2 <= T <= 1024, and the projection kernel's shared memory (3 T pc + nc pc + 4 ceil((5 nc + 3) / 4) + 672 nc floats,
+ * pc = 4 ceil(nc / 4)) must fit 227 KB: T <= 979 at nc = 16.  CEMK_ERR_ARG otherwise, with the handle unchanged. */
 int cemk_set_horizon(cemk_handle* h, int T, const float* G, const float* Kpp, const float* Kpe, const float* bounds3);
 
 /* compute_xi_samples (mjx_planner.py:313-316) with the standard-normal draws injected:
@@ -107,8 +109,8 @@ int cemk_cost_batch(cemk_handle* h, int B, int T, int nslot, const float* eef_po
                     const float* collision, const float* target_pos, const float* target_rot, float w_pos, float w_rot,
                     float w_col, float* cost4, void* stream);
 
-/* compute_ellite_samples (mjx_planner.py:306-310): stable ascending argsort of cost (NaN last, ties
- * by lower index).  cost is read with stride `cost_stride` floats.  keys_ws: [n_pow2] uint64 scratch
+/* compute_ellite_samples (mjx_planner.py:306-310): stable ascending argsort of cost (NaN last, -0.0 ties with
+ * +0.0, ties by lower index).  cost is read with stride `cost_stride` floats.  keys_ws: [n_pow2] uint64 scratch
  * (n_pow2 = next power of two >= n).  idx_base is added to every index (global sample index of this
  * shard).  Outputs: idx_sorted[n] (int32, global indices), and when k > 0 the k best rows gathered:
  * xi_elite[k][66] from xi[n][66] (local rows), cost_elite[k]. */

@@ -562,9 +562,13 @@ __global__ void __launch_bounds__(128) k_cost_batch(int B, int T, int nslot, con
 }
 
 // ---------------------------------------------------------------------------------------------- argsort / top-k
+// Ascending unsigned key of a cost in jnp.argsort's order: NaN last, -0.0 ties with +0.0 (lax's sort canonicalises the
+// zero's sign), every other value -- subnormals included -- in IEEE order.  The zero test looks at the bits: a float
+// comparison would be flushed to zero by -use_fast_math and tie the subnormals with zero as well.
 __device__ __forceinline__ unsigned int float_order(float f) {
   if (f != f) return 0xffffffffu;                       // NaN sorts last (jnp.argsort)
   unsigned int u = __float_as_uint(f);
+  if ((u << 1) == 0u) u = 0u;                           // -0.0 -> +0.0
   return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 __global__ void k_make_keys(int n, int npow2, const float* __restrict__ cost, int stride, unsigned long long* __restrict__ keys) {
@@ -1094,8 +1098,12 @@ int cemk_set_order(cemk_handle* h, int ncoef) {
 int cemk_set_horizon(cemk_handle* h, int T, const float* G, const float* Kpp, const float* Kpe, const float* bounds3) {
   if (!h || !G || !Kpp || !Kpe || !bounds3) return set_err(CEMK_ERR_ARG, "cemk_set_horizon: null argument");
   if (T < 2 || T > 1024) return set_err(CEMK_ERR_ARG, "cemk_set_horizon: T out of range [2, 1024]");
-  DevGuard guard(h->device);
   const int nc = h->ncoef;
+  // every check before the first change: a refused horizon leaves the handle's tables and T as they were
+  int smem = 0;
+  CEMK_FOR_NCOEF(nc, { smem = project_smem<NC>(T, 32 * PROJ_WARPS); });
+  if (smem > 227 * 1024) return set_err(CEMK_ERR_ARG, "cemk_set_horizon: horizon too long for the projection kernel's shared memory");
+  DevGuard guard(h->device);
   if (h->d_G) { CK(cudaFree(h->d_G)); h->d_G = nullptr; }
   CK(cudaMalloc(&h->d_G, sizeof(float) * 3 * T * nc));
   CK(cudaMemcpy(h->d_G, G, sizeof(float) * 3 * T * nc, cudaMemcpyHostToDevice));
@@ -1103,9 +1111,6 @@ int cemk_set_horizon(cemk_handle* h, int T, const float* G, const float* Kpp, co
   memcpy(kc, Kpp, nc * nc * 4); memcpy(kc + nc * nc, Kpe, nc * 5 * 4); memcpy(kc + nc * nc + nc * 5, bounds3, 12);
   CK(cudaMemcpy(h->d_K, kc, (nc * nc + nc * 5 + 3) * sizeof(float), cudaMemcpyHostToDevice));
   h->T = T;
-  int smem = 0;
-  CEMK_FOR_NCOEF(nc, { smem = project_smem<NC>(T, 32 * PROJ_WARPS); });
-  if (smem > 227 * 1024) return set_err(CEMK_ERR_ARG, "cemk_set_horizon: horizon too long for the projection kernel's shared memory");
   const int carve = 100 * PROJ_MINB * smem / (228 * 1024) + 8;                       // room for PROJ_MINB CTAs per SM, in percent
   CEMK_FOR_NCOEF(nc, { CK(cudaFuncSetAttribute(k_project<NC, KM_NL>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
                        CK(cudaFuncSetAttribute(k_project<NC, KM_NL>, cudaFuncAttributePreferredSharedMemoryCarveout, carve > 100 ? 100 : carve));

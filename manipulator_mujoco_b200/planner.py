@@ -132,8 +132,10 @@ class cem_planner:
         self.tot_time = tot_time
         tc = tot_time.reshape(self.num, 1)
         # the reference hard-codes order 10 (mjx_planner.py:40); `bernstein_order` is the order-n extension of SURVEY 8 f.4
-        if not 3 <= int(bernstein_order) <= 15:
-            raise ValueError("bernstein_order must be in [3, 15]")
+        # order 3 has four coefficients per DOF for the five boundary conditions of mjx_planner.py:163-164: its KKT matrix is
+        # singular (np.linalg.inv fails or returns per-DOF blocks of rounding noise)
+        if not 4 <= int(bernstein_order) <= 15:
+            raise ValueError("bernstein_order must be in [4, 15]")
         self.bernstein_order = int(bernstein_order)
         self.P, self.Pdot, self.Pddot = bernstein_coeff_ordern_new(self.bernstein_order, tc[0], tc[-1], tc)
         f32 = lambda a: torch.as_tensor(np.asarray(a), dtype=torch.float32, device=dev)

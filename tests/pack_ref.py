@@ -23,8 +23,10 @@ def topk_pack_ref(cost, idx_base, k, xi):
 
 
 def _order_key(cost):
-    """float_order in csrc/cemk.cu: float32 bits mapped to an ascending unsigned key, every NaN last."""
+    """float_order in csrc/cemk.cu: float32 bits mapped to an ascending unsigned key, every NaN last, -0.0 tied with +0.0
+    (jnp.argsort's order; subnormals stay apart from zero)."""
     u = np.asarray(cost, np.float32).view(np.uint32)
+    u = np.where(u << np.uint32(1) == 0, np.uint32(0), u).astype(np.uint32)
     key = np.where(u & 0x80000000, ~u, u | 0x80000000)
     return np.where(np.isnan(cost), np.uint32(0xffffffff), key).astype(np.uint32)
 

@@ -29,6 +29,7 @@ def _make(B, seed):
     cost = rng.uniform(100, 200, B).astype(np.float32)
     cost[rng.integers(0, B, B // 4)] = 123.0          # many exact ties, spread over all ranks
     cost[[5, B - 3]] = np.nan                         # NaN sorts last in jnp.argsort
+    cost[1], cost[B - 10] = 0.0, -0.0                 # the two best, on the first and the last rank: -0.0 ties with +0.0
     xi = rng.normal(size=(B, NVAR)).astype(np.float32)
     return cost, xi
 

@@ -201,3 +201,7 @@ def test_constructor_range_and_rollout_refusal():
         with pytest.raises(ValueError):
             cem_planner(num_dof=bad, num_batch=8, num_steps=8, timestep=0.05, maxiter_cem=1, num_elite=0.5,
                         w_pos=1.0, w_rot=1.0, w_col=1.0, maxiter_projection=1)
+    for bad in (3, 16):                         # order 3: four coefficients for five boundary conditions (singular KKT matrix)
+        with pytest.raises(ValueError, match="bernstein_order"):
+            cem_planner(num_dof=6, num_batch=8, num_steps=8, timestep=0.05, maxiter_cem=1, num_elite=0.5,
+                        w_pos=1.0, w_rot=1.0, w_col=1.0, maxiter_projection=1, bernstein_order=bad)

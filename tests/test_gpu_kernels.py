@@ -68,13 +68,31 @@ def test_projection_filter_across_horizons_and_ragged_batches(T, B):
 
 @pytest.mark.parametrize("n", [1, 5, 100, 1000, 4096, 5000, 8192, 8193, 20000])   # <= 8192: counting-rank kernel, above: bitonic network
 def test_argsort_topk_is_stable_with_nan_last(planner, n):
+    """jnp.argsort's order (mjx_planner.py:307): NaNs of any sign and payload last, -0.0 tied with +0.0 (lax's sort maps -0.0 to
+    +0.0), subnormals apart from zero, ties by index; signed zeros straddle the top-k cut."""
     rng = np.random.default_rng(n)
     cost = rng.uniform(0, 1000, n).astype(np.float32)
-    if n >= 100:
+    bits = lambda *u: np.array(u, np.uint32).view(np.float32)
+    k = max(1, n // 20)
+    if n == 1:
+        cost[0] = -0.0
+    elif n == 5:
+        cost[:] = [0.0, -0.0, 1.0, -0.0, 0.0]                        # k = 1: the +0.0 at index 0 wins
+    else:
         cost[rng.integers(0, n, n // 5)] = 77.0           # ties
         cost[[3, n // 2]] = np.nan
         cost[[7]] = -5.0
         cost[[11]] = np.inf
+        cost[[13, 17, 19, 23]] = bits(0xffc00000, 0x7f800001, 0xffffffff, 0x7fc12345)   # -NaN, signalling and payload NaNs
+        cost[[29, 31]] = -np.inf
+        cost[[37, 41, 43, 47]] = bits(0x80000001, 0x00000001, 0x807fffff, 0x007fffff)   # -+ smallest and largest subnormals
+        zeros = rng.choice(np.arange(50, n), 8, replace=False)
+        cost[zeros] = np.where(np.arange(8) % 3 == 0, 0.0, -0.0).astype(np.float32)
+        # negative costs in front, so that positions k - 4 .. k + 3 of the order are the eight signed zeros
+        free = np.setdiff1d(np.arange(50, n), zeros)
+        nneg = k - 4 - int((cost < 0).sum())
+        if nneg > 0:
+            cost[rng.choice(free, nneg, replace=False)] = -rng.uniform(1, 100, nneg).astype(np.float32)
     xi = rng.normal(size=(n, 66)).astype(np.float32)
     old = planner.ellite_num
     planner.ellite_num = max(1, n // 20)
@@ -85,9 +103,8 @@ def test_argsort_topk_is_stable_with_nan_last(planner, n):
     key = np.where(np.isnan(cost), np.inf, cost)
     ref = np.lexsort((np.arange(n), np.isnan(cost), key))
     np.testing.assert_array_equal(idx.cpu().numpy(), ref)
-    k = max(1, n // 20)
     np.testing.assert_array_equal(xe.cpu().numpy(), xi[ref[:k]])
-    np.testing.assert_array_equal(ce.cpu().numpy(), cost[ref[:k]])
+    np.testing.assert_array_equal(ce.cpu().numpy().view(np.int32), cost[ref[:k]].view(np.int32))
 
 
 def test_mean_cov(planner):
@@ -193,6 +210,7 @@ def test_topk_pack_and_merge_of_sorted_lists_equal_global_stable_topk(planner):
     cost = rng.uniform(0, 100, n).astype(np.float32)
     cost[rng.integers(0, n, n // 5)] = 1.0                             # ties across all shards, the k-th best among them
     cost[[7, 2000, 9000]] = np.nan
+    cost[[40, 1700, 1701, 5000]] = (0.0, -0.0, 0.0, -0.0)              # -0.0 ties with +0.0, within and across shards
     xi = rng.normal(size=(n, nv)).astype(np.float32)
     p = lambda t: C.c_void_p(t.data_ptr())
     packs, lo = [], 0
@@ -235,6 +253,8 @@ def test_merge_of_many_sorted_lists_with_ties_across_lists(planner, nlist, kl):
         c = np.round(rng.uniform(0, 30, kl), 1).astype(np.float32)          # one decimal: many ties
         if a % 3 == 0:
             c[rng.integers(0, kl, 3)] = np.nan
+        if a < 3:                                   # zeros of both signs: +0.0 in list 0, -0.0 in list 1, both in list 2 (a tie)
+            c[:4] = (0.0, 0.0, -0.0, -0.0) if a == 2 else (0.0 if a == 0 else -0.0)
         gi = a * Bl + np.sort(rng.choice(Bl, kl, replace=False))
         o = np.lexsort((gi, np.isnan(c), np.where(np.isnan(c), np.inf, c)))
         c, gi = c[o], gi[o]
