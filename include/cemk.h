@@ -146,9 +146,7 @@ int cemk_tick_record(cemk_handle* h, int iter, int n_iter, int last, int B, int 
 
 /* Options.  "force_rerun" (0/1): recompute every sample with the rollout instantiation that keeps all 48
  * contacts in shared memory, used by the tests to check that it agrees bit for bit with the fast kernel
- * and its spill area.  "cta_samples" (0..28): fixed
- * number of samples per CTA of the rollout kernel for A/B timing (0 = the library's own choice); never
- * changes a result. */
+ * and its spill area.  Any other name returns CEMK_ERR_ARG. */
 int cemk_set_option(cemk_handle* h, const char* name, int value);
 
 /* Calibration: measured FP32 FMA throughput (TFLOP/s, register operands) of the handle's device; synchronous.

@@ -6,10 +6,10 @@ import os
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# CEMK_LIB_PATH: A/B tools point this at a prebuilt variant under build_variants/ (never set by the product path)
+# CEMK_LIB_PATH: load a prebuilt library from another path, e.g. to time two builds side by side (never set by the product path)
 LIB_PATH = os.environ.get("CEMK_LIB_PATH") or os.path.join(_HERE, "libcemk.so")
 SRC = [os.path.join(_HERE, "csrc", n) for n in ("cemk.cu", "rollout_core.h", "warp_dsl.h", "kmodel.h")]
-NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-DCEMK_STEP_SYNC", "-DCEMK_PHASE_SYNC=18",
+NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-use_fast_math", "-shared", "-Xcompiler", "-fPIC"]
 
 

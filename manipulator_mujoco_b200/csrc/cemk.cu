@@ -26,16 +26,8 @@
 #define MAXCOEF 16
 #define MAXDOF 12
 #define MAXVAR (MAXDOF * MAXCOEF)      // 192
-#ifndef ROLLOUT_WARPS
 #define ROLLOUT_WARPS 14      // warps per CTA (28 samples with two samples per warp: all the shared memory of an SM); they
                               // step in lockstep (STEP_ALIGN) to share the instruction cache
-#endif
-#ifndef ROLLOUT_SETS
-#define ROLLOUT_SETS 1        // independent lockstep sets per CTA (named barriers 1 .. ROLLOUT_SETS)
-#endif
-#ifndef ROLLOUT_MINB
-#define ROLLOUT_MINB 1
-#endif
 
 static thread_local char g_err[256] = "";
 static int set_err(int code, const char* msg) { snprintf(g_err, sizeof g_err, "%s", msg); return code; }
@@ -67,7 +59,6 @@ struct cemk_handle {
   float* d_prevd; int prevd_cap;   // previous-step slot distances of every sample (rollout scratch, stays in L2)
   float* d_ovf;                    // contact spill area of every sample (same capacity as d_prevd)
   int force_rerun;               // debug option: recompute every sample with the all-in-shared-memory instantiation
-  int cta_samples;                 // debug option "cta_samples": fixed number of samples per CTA (0 = see cemk_rollout_cost)
   float* d_mc;                     // block sums of the blocked mean / covariance update (k_mc_partial -> k_mc_finish)
 };
 
@@ -99,7 +90,7 @@ struct RolloutBatch {
 // STATES: every sample steps from its own state rows and writes its final state (cemk_step_states, rollout_sample).
 #define GPW (32 / KW)                                     // lane groups (samples) per warp
 template <int NC, int WARPS, bool ONLY_FLAGGED, bool STATES = false>
-__global__ void __launch_bounds__(WARPS * 32, ROLLOUT_MINB) k_rollout(const KModel* __restrict__ gm, RolloutBatch a) {
+__global__ void __launch_bounds__(WARPS * 32, 1) k_rollout(const KModel* __restrict__ gm, RolloutBatch a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   KModel* sm = reinterpret_cast<KModel*>(smem_raw);
   WarpSmemT<NC>* ws = reinterpret_cast<WarpSmemT<NC>*>(smem_raw + ((sizeof(KModel) + 15) & ~size_t(15)));
@@ -126,13 +117,9 @@ __global__ void __launch_bounds__(WARPS * 32, ROLLOUT_MINB) k_rollout(const KMod
   W.lane = threadIdx.x & (KW - 1);
   W.shift = (threadIdx.x & 31) & ~(KW - 1);
   W.mask = KW_FULL << W.shift;
-  {
-    // alignment sets: the live warps of the CTA step in lockstep within ROLLOUT_SETS sets (warp w -> set w % SETS)
-    const int nw = ONLY_FLAGGED ? 1 : (nlive + GPW - 1) / GPW, w = threadIdx.x >> 5;
-    const int sets = nw < ROLLOUT_SETS ? 1 : ROLLOUT_SETS, set = w % sets;
-    W.bar = 1 + set;
-    W.nthr = ((nw - set + sets - 1) / sets) * 32;
-  }
+  // the live warps of the CTA step in lockstep (CTA_ALIGN on named barrier 1)
+  W.bar = 1;
+  W.nthr = (ONLY_FLAGGED ? 1 : (nlive + GPW - 1) / GPW) * 32;
 #ifdef CEMK_PHASE_TIMING
   W.phase = 14; W.t0 = clock64();
   for (int i = 0; i < 24; ++i) { W.ph[i] = 0; W.phs[i] = 0; W.phc[i] = 0; }
@@ -384,18 +371,12 @@ __global__ void __launch_bounds__(256) k_jax_normal(uint32_t k0, uint32_t k1, in
 // and a CTA size of 7 (or 3 or 1) warps so that 21 per SM is reachable.  The per-problem vectors that are touched once per
 // iteration (xs, cst, the multiplier sum) sit in per-thread shared-memory columns, which brings the kernel to 80 registers:
 // 3 CTAs of 7 warps per SM = 3108 warp slots, one wave.
-#ifndef PROJ_UNROLL
 #define PROJ_UNROLL 2
-#endif
 constexpr int kProjUnroll = PROJ_UNROLL;
 #define PROJ_SLICES 4
 #define PROJ_PPW (32 / PROJ_SLICES)      // problems per warp
-#ifndef PROJ_WARPS
 #define PROJ_WARPS 7
-#endif
-#ifndef PROJ_MINB
 #define PROJ_MINB 3
-#endif
 // NC = Bernstein coefficients per DOF (order + 1), a template parameter so that the iterates stay in registers; a basis
 // row is padded to PC = 4 ceil(NC / 4) floats.  nd = DOF per sample: B nd problems, xi / xi_f rows of nd NC, state_term rows of
 // 5 nd, thetadot rows of nd T.  ND = KM_NL fixes it at compile time (the product path, the code the 6-DOF build always had);
@@ -416,17 +397,9 @@ __global__ void __launch_bounds__(32 * PROJ_WARPS, NC <= 11 ? PROJ_MINB : 1) k_p
   for (int e = threadIdx.x; e < NC * PC; e += blockDim.x) { const int r = e / PC, k = e % PC; sKpp[e] = k < NC ? Kc[r * NC + k] : 0.f; }
   for (int e = threadIdx.x; e < 5 * NC + 3; e += blockDim.x) sK[e] = Kc[NC * NC + e];
   __syncthreads();
-#ifndef PROJ_LANEMAP
-#define PROJ_LANEMAP 1
-#endif
-#if PROJ_LANEMAP
   // lane = 8 slice + problem: the eight lanes of a quarter warp (one phase of a 128-bit shared-memory load) read the same row
   const int lane = threadIdx.x & 31, slice = lane >> 3, pl = lane & (PROJ_PPW - 1);
 #define PROJ_SRC(q) ((q) * PROJ_PPW + pl)
-#else
-  const int lane = threadIdx.x & 31, slice = lane & (PROJ_SLICES - 1), pl = lane >> 2;
-#define PROJ_SRC(q) ((lane & ~(PROJ_SLICES - 1)) | (q))
-#endif
   int prob = (blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * PROJ_PPW + pl;
   const bool act = prob < B * nd;        // idle lanes still take part in the shuffles
   if (!act) prob = B * nd - 1;
@@ -1001,11 +974,7 @@ static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
   int grid;
 #define CEMK_LAUNCH_ROLLOUT(W_) k_rollout<KM_NC_FAST, W_, false, STATES><<<grid, (W_) * 32, rollout_smem<KM_NC_FAST, W_>(), st>>>(h->d_model, a)
   const int need = (B + nsm - 1) / nsm;                            // samples per SM
-  if (h->cta_samples > 0) {
-    const int w = h->cta_samples < cap ? h->cta_samples : cap;
-    a.n_hi = 0; a.w_hi = a.w_lo = w; grid = (B + w - 1) / w;
-    CEMK_LAUNCH_ROLLOUT(ROLLOUT_WARPS);
-  } else if (need <= cap) {
+  if (need <= cap) {
     a.n_hi = 0; a.w_hi = a.w_lo = need; grid = (B + need - 1) / need;
     if (need <= 4 * GPW) CEMK_LAUNCH_ROLLOUT(4);
     else if (need <= 8 * GPW) CEMK_LAUNCH_ROLLOUT(8);
@@ -1026,7 +995,7 @@ static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
 
 extern "C" {
 
-int cemk_version(void) { return 4; }
+int cemk_version(void) { return 5; }
 const char* cemk_last_error(void) { return g_err; }
 int cemk_sizeof_kmodel(void) { return (int)sizeof(KModel); }
 
@@ -1038,7 +1007,7 @@ int cemk_create(const void* kmodel, int kmodel_bytes, int device, cemk_handle** 
     return set_err(CEMK_ERR_MODEL, "cemk_create: unsupported topology");
   DevGuard guard(device);
   cemk_handle* h = new cemk_handle();
-  h->device = device; h->ndof = KM_NL; h->ncoef = 11; h->nvar = KM_NL * 11; h->T = 0; h->d_G = nullptr; h->d_K = nullptr; h->launches = 0; h->d_flags = nullptr; h->flags_cap = 0; h->force_rerun = 0; h->cta_samples = 0; h->d_prevd = nullptr; h->prevd_cap = 0; h->d_ovf = nullptr;
+  h->device = device; h->ndof = KM_NL; h->ncoef = 11; h->nvar = KM_NL * 11; h->T = 0; h->d_G = nullptr; h->d_K = nullptr; h->launches = 0; h->d_flags = nullptr; h->flags_cap = 0; h->force_rerun = 0; h->d_prevd = nullptr; h->prevd_cap = 0; h->d_ovf = nullptr;
   { cudaDeviceProp prop; CK(cudaGetDeviceProperties(&prop, device)); h->num_sms = prop.multiProcessorCount; }
   CK(cudaMalloc(&h->d_model, sizeof(KModel)));
   CK(cudaMemcpy(h->d_model, kmodel, sizeof(KModel), cudaMemcpyHostToDevice));
@@ -1361,7 +1330,6 @@ long long cemk_launch_count(cemk_handle* h) { return h ? h->launches : 0; }
 int cemk_set_option(cemk_handle* h, const char* name, int value) {
   if (!h || !name) return set_err(CEMK_ERR_ARG, "cemk_set_option: null argument");
   if (!strcmp(name, "force_rerun")) { h->force_rerun = value != 0; return CEMK_OK; }
-  if (!strcmp(name, "cta_samples")) { h->cta_samples = value > 0 ? value : 0; return CEMK_OK; }
   return set_err(CEMK_ERR_ARG, "cemk_set_option: unknown option");
 }
 

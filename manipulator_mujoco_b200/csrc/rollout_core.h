@@ -25,19 +25,12 @@
 #include "kmodel.h"
 #include "warp_dsl.h"
 
-#ifndef CEMK_SYNC_EVERY
-#define CEMK_SYNC_EVERY 1                   // env-steps between two CTA-wide re-alignments (STEP_ALIGN)
-#endif
-#define KM_NC_FAST (KW == 16 ? 20 : 24)   // active-contact capacity of the fast kernel (shared-memory budget per sample)
+#define KM_NC_FAST 20                     // active-contact capacity of the fast kernel (shared-memory budget per sample)
 #define KM_NPASS (KM_MAXRPAIR / KW)         // collider passes over the robot pair table
 #define KM_NC_TOT 48                      // contacts a sample can have in total: the ones beyond the shared-memory capacity
                                           // spill to a per-sample global (L2) area
 #define KM_OVF_STRIDE 80                  // floats per spilled contact: geo 16, J 36, dots 2x3, rows 4x4
 #define KM_NC_BIG 48                      // shared-memory capacity of the debug instantiation (everything in shared memory)
-#ifndef CEMK_ROW_UNROLL
-#define CEMK_ROW_UNROLL 1            // unroll factor of the per-row / per-item loops of the constraint solve
-#endif
-constexpr int kRowUnroll = CEMK_ROW_UNROLL;
 #define MJ_MINVAL 1e-15f
 #define MJ_MINIMP 0.0001f
 #define MJ_MAXIMP 0.9999f
@@ -1011,7 +1004,7 @@ KFN int contact_blocks(const float* g) {
 template <int NC, bool SP>
 KFN void contact_dots(Warp& W, WarpSmemT<NC>& S, int ncon, const float* v0, const float* v1) {
   LANES(W, R)
-#pragma unroll(kRowUnroll)
+#pragma unroll 1
     for (int e = lane; e < 3 * ncon; e += KW) {
       const int c = e / 3, k = e - 3 * c;
       const int blk = contact_blocks(S.template geo<SP>(c));
@@ -1228,7 +1221,7 @@ KFN void solve_rows(Warp& W, const KModel& m, WarpSmemT<NC>& S, const int ncon, 
   LANES(W, R)
     // one (contact, dof of a block the contact touches) item per lane: six items per contact, twelve for a contact
     // between a robot link and the free box
-#pragma unroll(kRowUnroll)
+#pragma unroll 1
     for (int e = lane; e < KM_NL * ncon; e += KW) {
       const int c = e / KM_NL, k = e - KM_NL * c;
       const float* g = S.template geo<SP>(c);
@@ -1251,7 +1244,7 @@ KFN void solve_rows(Warp& W, const KModel& m, WarpSmemT<NC>& S, const int ncon, 
   // ---- C3: contact row parameters (the 4 pyramid edges share pos and D) ----
   contact_dots<NC, SP>(W, S, ncon, S.qvel, nullptr);
   LANES(W, R)
-#pragma unroll(kRowUnroll)
+#pragma unroll 1
     for (int r = nlim + lane; r < nrow; r += KW) {
       const float* g = S.template geo<SP>((r - nlim) >> 2);
       float w = g[13];
@@ -1269,13 +1262,12 @@ KFN void solve_rows(Warp& W, const KModel& m, WarpSmemT<NC>& S, const int ncon, 
     }
   END_LANES
   const bool coupled = warp_sum(W, [](int, LaneRegs& R) { return R.f2; }) > 0.f;
-  PHASE_ALIGN(8);
   PHASE(W, 8);
   // ---- S1: warm start vs smooth start (B.6) ----
   contact_dots<NC, SP>(W, S, ncon, S.warm, S.as);
   LANES(W, R)
     float cw = 0.f, cs = 0.f;
-#pragma unroll(kRowUnroll)
+#pragma unroll 1
     for (int r = lane; r < nrow; r += KW) {
       const float ar = S.template Aref<SP>(r, nlim), Dr = S.template D<SP>(r, nlim);
       float jw = row_val<NC, SP>(S, 0, r, S.warm) - ar, js = row_val<NC, SP>(S, 1, r, S.as) - ar;
@@ -1312,7 +1304,7 @@ KFN void solve_rows(Warp& W, const KModel& m, WarpSmemT<NC>& S, const int ncon, 
   // per contact: the pyramid-edge weights w_q = D [Jaref_q < 0] and the force sums that multiply
   // Jn, mu*Jt1, mu*Jt2; the contact position / frame slots of cgeo are dead after C2 and are reused.
   LANES(W, R)
-#pragma unroll(kRowUnroll)
+#pragma unroll 1
     for (int c = lane; c < ncon; c += KW) {
       const int r0 = nlim + 4 * c;
       float w[4], f[4];
@@ -1408,7 +1400,7 @@ KFN void solve_rows(Warp& W, const KModel& m, WarpSmemT<NC>& S, const int ncon, 
   EVENT(W, 7, coupled);
   if (coupled) coupled_solve<NC>(S);            // rare: full 12x12 system (replaces the block solution above); out of line
   REGROUP();
-  PHASE_ALIGN(16);
+  PHASE_ALIGN();
   PHASE(W, 11);
   // ---- S5: line search (BD.10) ----
   // J.search per row, the Gauss-term sums and the constraint sums of the starting point alpha = 0
@@ -1423,7 +1415,7 @@ KFN void solve_rows(Warp& W, const KModel& m, WarpSmemT<NC>& S, const int ncon, 
     // the lane's first row stays in registers for the line-search trips (R.h is free after the solve):
     // ja, jv and the three quadratic coefficients; an idle lane gets a row that is never active
     R.h[0] = 1.f; R.h[1] = 0.f; R.h[2] = 0.f; R.h[3] = 0.f; R.h[4] = 0.f;
-#pragma unroll(kRowUnroll)
+#pragma unroll 1
     for (int r = lane; r < nrow; r += KW) {
       const float jv = row_val<NC, SP>(S, 0, r, S.search), ja = S.template Jaref<SP>(r, nlim), D = S.template D<SP>(r, nlim);
       S.template Jv<SP>(r, nlim) = jv;
@@ -1458,9 +1450,7 @@ KFN void solve_rows(Warp& W, const KModel& m, WarpSmemT<NC>& S, const int ncon, 
       done = done || !swapped;
       done = done || ((lo.d0 < 0.f) && (lo.d0 > -gtol));
       done = done || ((hi.d0 > 0.f) && (hi.d0 < gtol));
-#ifndef CEMK_X_ALLTRIPS
       if (warp_all_groups(W, done)) break;
-#endif
       EVENT(W, 6, 1); EVENT(W, 5, !done);
       al0 = lo.alpha - lo.d0 / lo.d1; al1 = hi.alpha - hi.d0 / hi.d1; al2 = 0.5f * (lo.alpha + hi.alpha);
     }
@@ -1473,7 +1463,7 @@ KFN void solve_rows(Warp& W, const KModel& m, WarpSmemT<NC>& S, const int ncon, 
         if (ja + al1 * jv < 0.f) { b0 = q0; b1 = q1; b2 = q2; }
         if (ja + al2 * jv < 0.f) { c0 = q0; c1 = q1; c2 = q2; }
       }
-#pragma unroll(kRowUnroll)
+#pragma unroll 1
       for (int r = lane + KW; r < nrow; r += KW) {             // more than KW rows: the rest from shared memory
         const float ja = S.template Jaref<SP>(r, nlim), jv = S.template Jv<SP>(r, nlim), D = S.template D<SP>(r, nlim);
         const float q0 = 0.5f * D * ja * ja, q1 = D * jv * ja, q2 = 0.5f * D * jv * jv;
@@ -1716,7 +1706,6 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
       for (int k = 0; k < 3; ++k) { S.as[KM_NL + k] = S.fs[KM_NL + k] / m.fb_mass; S.as[KM_NL + 3 + k] = S.fs[KM_NL + 3 + k] / m.fb_inertia[k]; }
     } END_UNIFORM_WRITE
   }
-  PHASE_ALIGN(1);
   PHASE(W, 4);
   // ---- N1: narrow phase + collision cost of this step (mjx_planner.py:287-296:
   //      cost_c = sum max(0, (1-y) c_t - c_{t+1}) + #(c < 0), y = 0.005) ----
@@ -1827,9 +1816,6 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
     // List position of a near pair: lane-major (capsule), pass-minor (box).
     int ntot = warp_excl_scan(W, [](int, LaneRegs& R) { return KPOPC(R.off & 0xffff); }, [](int, LaneRegs& R, int o) { R.actmask = o; });
     EVENT(W, 0, 1); EVENT(W, 1, ntot > 0); EVENT(W, 2, ntot); EVENT(W, 11, warp_any_groups(W, ntot > 0));
-#ifdef CEMK_X_NONEAR
-    ntot = 0;      // timing experiment only (wrong results): what the near pass costs, lockstep wait included
-#endif
     // (Letting every warp walk this pass with a dummy pair, so that it runs in lockstep like the rest of the step, was
     //  measured: +1.4 %.)
     if (warp_any_groups(W, ntot > 0)) {
@@ -1925,9 +1911,6 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
         }
         RLANES(W, R)
           R.nact = i0 + lane < ntot ? (R.f0 < 0.f ? 1 : 0) + (R.f1 < 0.f ? 2 : 0) : 0;
-#ifdef CEMK_X_NEARNOCON
-          R.nact = 0;   // timing experiment only (wrong results): near pass without the contacts it finds
-#endif
         END_RLANES
         const long long tk1 = TICK(); (void)tk1;
         EVENT(W, 14, (int)(tk1 - tk0));
@@ -1978,7 +1961,6 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
     }
   }
   PHASE(W, 23);
-  PHASE_ALIGN(4);
   PHASE(W, 5);
   // free-box pairs: broad phase for all pairs at once (one lane per pair), then the cooperative
   // narrow phase only for the pairs that pass
@@ -2039,9 +2021,7 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
   PHASE(W, 6);
   // ---- N2: full contact records for the active slots (divergent, rare for robot slots) ----
   LANES(W, R)
-#ifndef CEMK_X_NOEMIT
     if (R.nact > 0) emit_robot_contacts<NC>(m, S, lane, R.actmask, R.off);
-#endif
     for (int sl = lane; sl < 32; sl += KW) {
       if (!(bmask & (1u << sl))) continue;
       const int o = nrob + KPOPC(bmask & ((1u << sl) - 1u)), q = sl >> 2;
@@ -2058,7 +2038,7 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
     }
   END_LANES
   PHASE(W, 18);
-  PHASE_ALIGN(2);
+  PHASE_ALIGN();
   PHASE(W, 7);
   // ---- C1: joint-limit rows ----
   LANES(W, R)
@@ -2166,7 +2146,7 @@ KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const Rollou
 #pragma unroll 1
   for (int t = 0; t < A.T; ++t) {
     PHASE(W, 13);
-    if ((t % CEMK_SYNC_EVERY) == 0) { STEP_ALIGN(); }
+    STEP_ALIGN();
     PHASE(W, 0);
     LANES(W, R)
       if (lane < KM_NL) {

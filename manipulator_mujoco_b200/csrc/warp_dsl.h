@@ -1,12 +1,11 @@
 // warp_dsl.h -- a tiny "one lane group = one sample" programming layer.
 //
-// A sample is owned by a group of KW lanes: KW = 16 (default, two samples per warp) or 32 (one sample
-// per warp, -DCEMK_KW=32).  The rollout core (rollout_core.h) is written once against these macros and
-// compiled twice:
+// A sample is owned by a group of KW = 16 lanes, two samples per warp.  The rollout core (rollout_core.h)
+// is written once against these macros and compiled twice:
 //   * by nvcc for sm_100a, where a LANES block is the body executed by each of the KW lanes of the
 //     group, per-lane state lives in registers, collectives are shuffles / ballots restricted to the
 //     group (member mask = the group's lanes, width = KW) and every block is fenced by
-//     __syncwarp(group mask).  With KW = 16 the two halves of a warp run the same instruction stream on
+//     __syncwarp(group mask).  The two halves of a warp run the same instruction stream on
 //     two samples: "uniform" scalar code (small dense solves, the serial joint chain, line-search control)
 //     is issued once for both, and phases that only have 6..16 work items fill the warp twice as well.
 //     Two flavours of every fence / collective exist.  The plain ones (LANES, UNIFORM_WRITE, warp_sum ...)
@@ -29,12 +28,8 @@
 #pragma once
 #include <math.h>
 
-#ifndef CEMK_KW
-#define CEMK_KW 16
-#endif
-#define KW CEMK_KW
-static_assert(KW == 16 || KW == 32, "CEMK_KW must be 16 or 32");
-#define KW_FULL (KW == 32 ? 0xffffffffu : 0xffffu)
+#define KW 16
+#define KW_FULL 0xffffu
 
 #ifdef CEMK_EMU
 #include <cstring>
@@ -42,7 +37,7 @@ static_assert(KW == 16 || KW == 32, "CEMK_KW must be 16 or 32");
 #define KMEM inline
 #define KNOINLINE static
 #define STEP_ALIGN()
-#define PHASE_ALIGN(bit)
+#define PHASE_ALIGN()
 #ifdef CEMK_EMU_RACE
 // Race-checking emulation (tests/test_emu_race.py): every lane of a LANES block runs against the scratch as it was when
 // the block started (plus its own writes); the lanes' writes are merged when the block ends.  That is exactly what rule 1
@@ -123,18 +118,10 @@ static inline int __float_as_int(float f) { int i; std::memcpy(&i, &f, 4); retur
 // live thread count of this CTA (a CTA may run fewer samples than its launch width, see
 // cemk_rollout_cost).  The two groups of a warp re-converge first (bar.sync is a per-warp instruction).
 #define CTA_ALIGN(W) do { __syncwarp(); asm volatile("bar.sync %0, %1;" :: "r"((W).bar), "r"((W).nthr) : "memory"); } while (0)
-#ifdef CEMK_STEP_SYNC
+// STEP_ALIGN: once per env-step.  PHASE_ALIGN: inside a step, only at points every group reaches (before the
+// constraint rows and before the line search)
 #define STEP_ALIGN() CTA_ALIGN(W)
-#else
-#define STEP_ALIGN()
-#endif
-// optional extra CTA-wide re-alignments inside a step, selected by the bits of CEMK_PHASE_SYNC
-// (only at points every group reaches)
-#if defined(CEMK_STEP_SYNC) && defined(CEMK_PHASE_SYNC)
-#define PHASE_ALIGN(bit) do { if ((CEMK_PHASE_SYNC) & (bit)) CTA_ALIGN(W); } while (0)
-#else
-#define PHASE_ALIGN(bit)
-#endif
+#define PHASE_ALIGN() CTA_ALIGN(W)
 #define LANES(W, R) { __syncwarp(); const int lane = (W).lane; auto& R = (W).regs; (void)R;
 #define END_LANES } __syncwarp();
 #define DLANES(W, R) { __syncwarp((W).mask); const int lane = (W).lane; auto& R = (W).regs; (void)R;
@@ -172,8 +159,8 @@ struct WarpCtx {
   int lane;          // lane within the group, 0..KW-1
   int shift;         // first lane of the group within the warp (0 or 16)
   unsigned mask;     // member mask of the group
-  int nthr;          // threads of this warp's alignment set (barrier width)
-  int bar;           // named barrier of the alignment set (1 ..)
+  int nthr;          // threads of the CTA's live warps (barrier width of CTA_ALIGN)
+  int bar;           // named barrier of CTA_ALIGN (1)
 #ifdef CEMK_PHASE_TIMING
   long long t0; int phase; long long ph[24];
   long long phs[24], phc[24]; int stepflag, nflag;   // this step's clocks; clocks of the steps with stepflag set (conditional profile)
@@ -349,11 +336,6 @@ KFN void warp_sum9(W& w, float* out) {
   float v[9], u[5], t[3], s2[2], r[1];
 #pragma unroll
   for (int k = 0; k < 9; ++k) v[k] = w.regs.acc[k];
-  if (KW == 32) {
-    // lanes 16..31 carry no extra values: plain add first, then the same four folding rounds
-#pragma unroll
-    for (int k = 0; k < 9; ++k) v[k] += __shfl_xor_sync(KMASK(w), v[k], 16, KW);
-  }
   fold_round<9, DIV>(w, v, u, lane & 8, 8);
   fold_round<5, DIV>(w, u, t, lane & 4, 4);
   fold_round<3, DIV>(w, t, s2, lane & 2, 2);

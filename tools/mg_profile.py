@@ -3,7 +3,7 @@ synchronisation inside an iteration), averaged over 20 iterations, per rank.  Ru
     timeout 300 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29544 tools/mg_profile.py
 The all-gather stage of a rank includes its wait for the slowest rank's rollout.
 DUMP=<file.npz> (one GPU): also save every stage's outputs of one iteration, for bitwise A/B of library variants
-(CEMK_LIB_PATH=build_variants/<name>.so; compare with tools/mg_profile.py --compare a.npz b.npz)."""
+(CEMK_LIB_PATH=<another build>/libcemk.so; compare with tools/mg_profile.py --compare a.npz b.npz)."""
 import contextlib
 import io
 import os

@@ -1,8 +1,7 @@
-"""Time the fused rollout+cost kernel alone for several CTA shares (A/B tool, GPU box only).
+"""Time the fused rollout+cost kernel alone (GPU box only).
 
-usage: python tools/time_rollout.py [--batch 4096] [--horizon 100] [--cta 0,12,14,16] [--reps 5]
-`--cta 0` is the library's own choice (balanced waves).  Also checks that every setting returns
-bit-identical costs (the CTA share must not change any result).
+usage: python tools/time_rollout.py [--batch 4096] [--horizon 100] [--reps 5]
+Also checks that every timed run returns costs bit-identical to the warm-up run's.
 """
 import argparse
 import contextlib
@@ -14,14 +13,13 @@ import numpy as np
 import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
-from manipulator_mujoco_b200 import _lib, cem_planner  # noqa: E402
+from manipulator_mujoco_b200 import cem_planner  # noqa: E402
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batch", default="4096")
     ap.add_argument("--horizon", type=int, default=100)
-    ap.add_argument("--cta", default="0")
     ap.add_argument("--reps", type=int, default=5)
     args = ap.parse_args()
     dev = torch.device("cuda:0")
@@ -37,26 +35,21 @@ def main():
         state_term = torch.cat([q0, z6, z6, z6, z6]).unsqueeze(0).expand(B, 30).contiguous()
         xi, _ = pl.compute_xi_samples(pl.key, torch.zeros(pl.nvar, device=dev), 10 * torch.eye(pl.nvar, device=dev))
         _, thetadot = pl._project(xi, state_term, True)
-        ref = None
-        for w in [int(x) for x in args.cta.split(",")]:
-            _lib.check(pl._lib.cemk_set_option(pl._h, b"cta_samples", w), pl._lib)
-            for _ in range(2):
-                out = pl._rollout(thetadot, q0, z6, tp, tr, False)
-            ms = []
-            for _ in range(args.reps):
-                flush.fill_(1.0)
-                a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                a.record()
-                out = pl._rollout(thetadot, q0, z6, tp, tr, False)
-                b.record()
-                torch.cuda.synchronize()
-                ms.append(a.elapsed_time(b))
-            cost = out[1].detach().cpu().numpy().view(np.int32).copy()
-            same = "" if ref is None else ("  bit-identical" if np.array_equal(ref, cost) else "  RESULTS DIFFER")
-            if ref is None:
-                ref = cost
-            print(f"B={B} T={args.horizon} cta_samples={w:2d}: {np.mean(ms):7.3f} ms (min {np.min(ms):.3f})  {B * args.horizon / np.mean(ms) * 1e3:.3e} env-steps/s{same}",
-                  flush=True)
+        for _ in range(2):
+            out = pl._rollout(thetadot, q0, z6, tp, tr, False)
+        ref = out[1].detach().cpu().numpy().view(np.int32).copy()
+        ms, same = [], True
+        for _ in range(args.reps):
+            flush.fill_(1.0)
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record()
+            out = pl._rollout(thetadot, q0, z6, tp, tr, False)
+            b.record()
+            torch.cuda.synchronize()
+            ms.append(a.elapsed_time(b))
+            same = same and np.array_equal(ref, out[1].detach().cpu().numpy().view(np.int32))
+        print(f"B={B} T={args.horizon}: {np.mean(ms):7.3f} ms (min {np.min(ms):.3f})  {B * args.horizon / np.mean(ms) * 1e3:.3e} env-steps/s"
+              f"  {'bit-identical' if same else 'RESULTS DIFFER'}", flush=True)
         del pl
 
 

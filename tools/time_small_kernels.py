@@ -1,5 +1,5 @@
 """Event-timed launches of the small kernels around k_rollout (one GPU), for A/B of library variants:
-    [CEMK_LIB_PATH=build_variants/<name>.so] python tools/time_small_kernels.py
+    [CEMK_LIB_PATH=<another build>/libcemk.so] python tools/time_small_kernels.py
 sample (k_chol66 + k_sample), k_project, local top-k (argsort / pack), the merge of 8 gathered elite lists, mean / cov."""
 import contextlib
 import io
