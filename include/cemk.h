@@ -15,7 +15,7 @@
  *     nc = Bernstein coefficients per DOF (cemk_set_order, default 11), NV = nvar = nd * nc decision variables.
  *     "66", "30" and "6T" in the shapes below are NV, 5 nd and nd T at the defaults.
  *   - The planner algebra (sampling, projection, elite selection, mean / covariance) runs at any
- *     1 <= nd <= 12 and 4 <= nc <= 16 (NV <= 192).  The rollout (cemk_rollout_cost, cemk_step_states, cemk_tick_record)
+ *     1 <= nd <= 12 and 4 <= nc <= 16 (NV <= 192).  The rollout (cemk_rollout_cost, cemk_step_states[_contacts], cemk_tick_record)
  *     models the 6-DOF arm of the KModel only and returns CEMK_ERR_ARG on a handle with nd != 6.
  */
 #ifndef CEMK_H
@@ -102,6 +102,27 @@ int cemk_rollout_cost(cemk_handle* h, int B, int T, const float* thetadot, const
 int cemk_step_states(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm,
                      const float* thetadot, float* qpos_out, float* qvel_out, float* warm_out, float* theta,
                      float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags, void* stream);
+
+/* Contacts a step keeps per environment, and floats per contact record of cemk_step_states_contacts. */
+#define CEMK_MAX_CONTACTS 48
+#define CEMK_CONTACT_REC 12
+
+/* cemk_step_states, plus what mjx.step's Data holds about the constraints of the last step (at the accepted qacc, MJX's
+ * solver finish: f_r = -D_r (J_r qacc - aref_r) where that is negative, else 0):
+ *   qfrc_constraint[N][12] = sum_r J_r^T f_r over the joint-limit and contact rows;
+ *   ncon[N] = contacts kept (<= 48; flags bit 0 reports dropped ones);
+ *   con_slot[N][48] = the model's contact-slot index of each contact, ascending, padded with -1;
+ *   con_rec[N][48][CEMK_CONTACT_REC] = dist, pos[3], normal[3] (first row of the contact frame), force[3] (contact frame:
+ *   normal, tangent 1, tangent 2, decoded from the four pyramid rows as mju_decodePyramid does), 2 unused; zeros as padding.
+ * slot_map (device, int): the model's contact slot of each contact key of the KModel, [nslot_robot + 4 nbpair]; key k <
+ * nslot_robot is robot slot k (the cost slots of cemk_rollout_cost, in model order), key nslot_robot + 4 q + j is slot j of
+ * free-box pair q (bp_type order).  The KModel numbers its pairs but not the model's slots, hence the map.
+ * slot_map and the four outputs are all given or all NULL (then this is cemk_step_states); CEMK_ERR_ARG for some but not
+ * all, and for everything cemk_step_states refuses. */
+int cemk_step_states_contacts(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm,
+                              const float* thetadot, float* qpos_out, float* qvel_out, float* warm_out, float* theta,
+                              float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags, const int* slot_map,
+                              float* qfrc_constraint, int* ncon, int* con_slot, float* con_rec, void* stream);
 
 /* compute_cost_batch alone (mjx_planner.py:277-303), per-sample targets as in the reference method:
  *   eef_pos[B][T][3], eef_rot[B][T][4], collision[B][T][nslot], target_pos[B][3], target_rot[B][4] -> cost4[B][4]. */

@@ -48,6 +48,7 @@ _SIGS = {
     "cemk_project": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp], _i),
     "cemk_rollout_cost": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
     "cemk_step_states": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
+    "cemk_step_states_contacts": ([_vp, _i, _i] + [_vp] * 19, _i),
     "cemk_cost_batch": ([_vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp], _i),
     "cemk_argsort_topk": ([_vp, _i, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp], _i),
     "cemk_topk_pack": ([_vp, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp], _i),

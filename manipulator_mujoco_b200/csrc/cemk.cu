@@ -5,6 +5,7 @@
 //   k_project                compute_projection_filter + A_thetadot @ xi   (:181-249, :348)
 //   k_rollout                vmap(scan(mjx.step)) + compute_cost_batch     (:251-303)   <- hot kernel
 //   k_rollout<.., STATES>    vmap(mjx.step) over per-environment states, chained T steps (cemk_step_states)
+//   k_rollout<.., STATES, CONTACTS>   the same, plus the last step's contacts and constraint forces (cemk_step_states_contacts)
 //   k_cost_batch             compute_cost_batch on materialised trajectories (:277-303)
 //   k_rank_select (n <= 8192) | k_make_keys / k_bitonic* / k_gather_sorted    compute_ellite_samples   (:306-310)
 //   k_merge_lists            the same selection over the per-rank sorted lists of several GPUs
@@ -18,6 +19,7 @@
 
 #include "../../include/cemk.h"
 #include "rollout_core.h"
+static_assert(CEMK_MAX_CONTACTS == KM_NC_TOT && CEMK_CONTACT_REC == KM_CON_REC, "contact output layout of cemk.h");
 
 // Bernstein order n (mjx_planner.py:40 hard-codes 10; SURVEY 8 f.4 asks for order n): ncoef = n + 1 coefficients per DOF,
 // nvar = ndof ncoef decision variables, chosen per handle by cemk_set_dof / cemk_set_order (default 6 DOF x 11 = 66).  The
@@ -81,6 +83,9 @@ struct RolloutBatch {
   // cemk_step_states (STATES): q0 / v0 are then qpos [B][13] / qvel [B][12], and warm [B][12] is the third state input
   const float* warm;
   float* qpos_out; float* qvel_out; float* warm_out;
+  // cemk_step_states_contacts (CONTACTS): contact key -> model slot, and the outputs [B][12], [B], [B][48], [B][48][KM_CON_REC]
+  const int* slot_map;
+  float* qfrc; int* ncon; int* con_slot; float* con_rec;
 };
 
 // NC = contacts of a sample kept in shared memory (the rest, up to KM_NC_TOT, in the global spill area),
@@ -88,8 +93,9 @@ struct RolloutBatch {
 // instantiation (NC = KM_NC_FAST) is the product path.  ONLY_FLAGGED is the debug instantiation behind
 // cemk_set_option("force_rerun"): NC = 48 (no spill area), one warp per CTA, samples whose flag bit 0 is set.
 // STATES: every sample steps from its own state rows and writes its final state (cemk_step_states, rollout_sample).
+// CONTACTS (with STATES): and the last step's contacts and constraint forces (cemk_step_states_contacts, contact_outputs).
 #define GPW (32 / KW)                                     // lane groups (samples) per warp
-template <int NC, int WARPS, bool ONLY_FLAGGED, bool STATES = false>
+template <int NC, int WARPS, bool ONLY_FLAGGED, bool STATES = false, bool CONTACTS = false>
 __global__ void __launch_bounds__(WARPS * 32, 1) k_rollout(const KModel* __restrict__ gm, RolloutBatch a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   KModel* sm = reinterpret_cast<KModel*>(smem_raw);
@@ -148,7 +154,12 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_rollout(const KModel* __restr
   A.flags = a.flags + s;
   A.prevd = a.prevd + (size_t)s * (2 * KM_NPASS * KW);
   A.ovf = a.ovf + (size_t)s * ((KM_NC_TOT - KM_NC_FAST) * KM_OVF_STRIDE);
-  rollout_sample<NC, STATES>(W, *sm, ws[group], A);
+  if (CONTACTS) {
+    A.slot_map = a.slot_map;
+    A.qfrc = a.qfrc + (size_t)s * KM_NV; A.ncon = a.ncon + s;
+    A.con_slot = a.con_slot + (size_t)s * KM_NC_TOT; A.con_rec = a.con_rec + (size_t)s * KM_NC_TOT * KM_CON_REC;
+  }
+  rollout_sample<NC, STATES, CONTACTS>(W, *sm, ws[group], A);
 #ifdef CEMK_PHASE_TIMING
   PHASE(W, 15);
   if (W.lane == 0 && !ONLY_FLAGGED) for (int i = 0; i < 24; ++i) atomicAdd(&g_phase[i], (unsigned long long)W.ph[i]);
@@ -939,10 +950,10 @@ static int rollout_dof_check(const cemk_handle* h, const char* fn) {
   return CEMK_ERR_ARG;
 }
 
-// One launch of the product rollout over a.B samples (cemk_rollout_cost, and cemk_step_states with STATES): grows the
-// library scratch to a.B samples (the flags when a.flags is null, the previous distances, the spill area), points `a` at it
-// and chooses the CTA shares.
-template <bool STATES>
+// One launch of the product rollout over a.B samples (cemk_rollout_cost, and cemk_step_states[_contacts] with STATES
+// [and CONTACTS]): grows the library scratch to a.B samples (the flags when a.flags is null, the previous distances, the
+// spill area), points `a` at it and chooses the CTA shares.
+template <bool STATES, bool CONTACTS = false>
 static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
   const int B = a.B;
   if (!a.flags) {
@@ -972,7 +983,7 @@ static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
   const int nsm = h->num_sms > 0 ? h->num_sms : 148;
   const int cap = ROLLOUT_WARPS * GPW, unit = 4 * GPW;
   int grid;
-#define CEMK_LAUNCH_ROLLOUT(W_) k_rollout<KM_NC_FAST, W_, false, STATES><<<grid, (W_) * 32, rollout_smem<KM_NC_FAST, W_>(), st>>>(h->d_model, a)
+#define CEMK_LAUNCH_ROLLOUT(W_) k_rollout<KM_NC_FAST, W_, false, STATES, CONTACTS><<<grid, (W_) * 32, rollout_smem<KM_NC_FAST, W_>(), st>>>(h->d_model, a)
   const int need = (B + nsm - 1) / nsm;                            // samples per SM
   if (need <= cap) {
     a.n_hi = 0; a.w_hi = a.w_lo = need; grid = (B + need - 1) / need;
@@ -995,7 +1006,7 @@ static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
 
 extern "C" {
 
-int cemk_version(void) { return 5; }
+int cemk_version(void) { return 6; }
 const char* cemk_last_error(void) { return g_err; }
 int cemk_sizeof_kmodel(void) { return (int)sizeof(KModel); }
 
@@ -1020,6 +1031,10 @@ int cemk_create(const void* kmodel, int kmodel_bytes, int device, cemk_handle** 
                           (int)rollout_smem<KM_NC_FAST, ROLLOUT_WARPS>()));
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 8, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 8>()));
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 4, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 4>()));
+  CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, ROLLOUT_WARPS, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)rollout_smem<KM_NC_FAST, ROLLOUT_WARPS>()));
+  CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 8, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 8>()));
+  CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 4, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 4>()));
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_BIG, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                           (int)rollout_smem<KM_NC_BIG, 1>()));
   h->d_mc = nullptr;
@@ -1154,21 +1169,47 @@ int cemk_rollout_cost(cemk_handle* h, int B, int T, const float* thetadot, const
 
 // force_rerun does not apply here: it re-reads the samples' inputs after the product launch, and with in-place outputs
 // those rows already hold the stepped states.
+// cemk_step_states and cemk_step_states_contacts: the checks and the launch; fn names the entry in error messages, and
+// with a.slot_map set the contact outputs are written too
+static int step_states(cemk_handle* h, RolloutBatch& a, void* stream, const char* fn) {
+  if (!h || !a.q0 || !a.v0 || !a.warm || !a.qpos_out || !a.qvel_out || !a.warm_out || a.B <= 0 || a.T <= 0) {
+    snprintf(g_err, sizeof g_err, "%s: bad argument", fn);
+    return CEMK_ERR_ARG;
+  }
+  if (!a.thetadot && a.T > 1) {
+    snprintf(g_err, sizeof g_err, "%s: thetadot may only be NULL with T = 1", fn);
+    return CEMK_ERR_ARG;
+  }
+  { const int rc = rollout_dof_check(h, fn); if (rc) return rc; }
+  DevGuard guard(h->device);
+  { const int rc = a.slot_map ? launch_rollout<true, true>(h, a, (cudaStream_t)stream) : launch_rollout<true>(h, a, (cudaStream_t)stream); if (rc) return rc; }
+  CK(cudaPeekAtLastError());
+  return CEMK_OK;
+}
+
 int cemk_step_states(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm, const float* thetadot,
                      float* qpos_out, float* qvel_out, float* warm_out, float* theta, float* eef_pos, float* eef_rot, float* collision,
                      float* qacc, int* flags, void* stream) {
-  if (!h || !qpos || !qvel || !warm || !qpos_out || !qvel_out || !warm_out || N <= 0 || T <= 0)
-    return set_err(CEMK_ERR_ARG, "cemk_step_states: bad argument");
-  if (!thetadot && T > 1) return set_err(CEMK_ERR_ARG, "cemk_step_states: thetadot may only be NULL with T = 1");
-  { const int rc = rollout_dof_check(h, "cemk_step_states"); if (rc) return rc; }
-  DevGuard guard(h->device);
   RolloutBatch a = {};
   a.B = N; a.T = T; a.thetadot = thetadot; a.q0 = qpos; a.v0 = qvel; a.warm = warm;
   a.qpos_out = qpos_out; a.qvel_out = qvel_out; a.warm_out = warm_out;
   a.theta = theta; a.eef_pos = eef_pos; a.eef_rot = eef_rot; a.collision = collision; a.qacc = qacc; a.flags = flags;
-  { const int rc = launch_rollout<true>(h, a, (cudaStream_t)stream); if (rc) return rc; }
-  CK(cudaPeekAtLastError());
-  return CEMK_OK;
+  return step_states(h, a, stream, "cemk_step_states");
+}
+
+int cemk_step_states_contacts(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm,
+                              const float* thetadot, float* qpos_out, float* qvel_out, float* warm_out, float* theta,
+                              float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags, const int* slot_map,
+                              float* qfrc_constraint, int* ncon, int* con_slot, float* con_rec, void* stream) {
+  const int given = (slot_map ? 1 : 0) + (qfrc_constraint ? 1 : 0) + (ncon ? 1 : 0) + (con_slot ? 1 : 0) + (con_rec ? 1 : 0);
+  if (given != 0 && given != 5)
+    return set_err(CEMK_ERR_ARG, "cemk_step_states_contacts: slot_map and the contact outputs are all given or all NULL");
+  RolloutBatch a = {};
+  a.B = N; a.T = T; a.thetadot = thetadot; a.q0 = qpos; a.v0 = qvel; a.warm = warm;
+  a.qpos_out = qpos_out; a.qvel_out = qvel_out; a.warm_out = warm_out;
+  a.theta = theta; a.eef_pos = eef_pos; a.eef_rot = eef_rot; a.collision = collision; a.qacc = qacc; a.flags = flags;
+  a.slot_map = slot_map; a.qfrc = qfrc_constraint; a.ncon = ncon; a.con_slot = con_slot; a.con_rec = con_rec;
+  return step_states(h, a, stream, "cemk_step_states_contacts");
 }
 
 int cemk_cost_batch(cemk_handle* h, int B, int T, int nslot, const float* eef_pos, const float* eef_rot, const float* collision,

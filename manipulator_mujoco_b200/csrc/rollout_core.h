@@ -1192,7 +1192,13 @@ struct StepIO {
   bool first;                 // t == 0: no previous distance yet
   float* collision_row;       // optional dump of this step's robot-slot distances [nslot_robot]
   float* prevd;               // this sample's previous-step distances, [2 * KM_NPASS][KW] (global scratch, L2-resident)
+  // step_forward<NC, true> only (null: not this step): per contact in list order, its key (robot slot, or nslot_robot +
+  // 4 box pair + slot; RolloutArgs::slot_map) and a KM_CON_REC record with dist, pos and normal.  The solve overwrites the
+  // position and frame in the contact record, so contact_outputs takes them from here.
+  int* con_key;
+  float* con_rec;
 };
+#define KM_CON_REC 12                     // floats per contact output record: dist, pos[3], normal[3], force[3], 2 unused
 
 // search = -H^-1 grad for the full 12x12 system (a contact couples a robot link and the free box).  Cold: a real
 // function with its own lane-group context; may be entered by one of the two samples of a warp (D-flavoured fences).
@@ -1529,7 +1535,8 @@ KNOINLINE void solve_rows_spilled(const KModel& m, WarpSmemT<NC>& S, int ncon, i
 // ------------------------------------------------------------------------------------------ one forward()
 // Inputs: S.qpos, S.qvel, S.warm.  Outputs: S.qacc (= new warm start), link frames, and the
 // collision-cost contribution of this step added to R.cost_c (mjx_planner.py:287-296).
-template <int NC>
+// CON: also the contact keys and geometry of io.con_key / io.con_rec when they are set.
+template <int NC, bool CON = false>
 KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& io) {
   PHASE(W, 1);
   // ---- P1: joint chain as a parallel prefix of rigid transforms.  Lane 0 holds the static base frame, lane
@@ -1949,6 +1956,11 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
               const float invw = m.cap_invw[a] + (st ? 0.f : m.fb_invw);
               const int l1 = m.cap_link[a], l2 = st ? -1 : KM_NL;
               int o = ncbcon + R.actmask;
+              if (CON && io.con_key) {
+                if ((R.nact & 1) && o < KM_NC_TOT) io.con_key[o] = KP_SLOT(x);
+                const int o1 = o + (R.nact & 1);
+                if ((R.nact & 2) && o1 < KM_NC_TOT) io.con_key[o1] = KP_SLOT(x) + 1;
+              }
               if (R.nact & 1) { put_contact<NC>(S, o, R.h, R.h + 3, nullptr, d0, invw, l1, l2); ++o; }
               if (R.nact & 2) put_contact<NC>(S, o, R.h + 6, R.h + 9, nullptr, d1, invw, l1, l2);
             }
@@ -2022,9 +2034,18 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
   // ---- N2: full contact records for the active slots (divergent, rare for robot slots) ----
   LANES(W, R)
     if (R.nact > 0) emit_robot_contacts<NC>(m, S, lane, R.actmask, R.off);
+    if (CON && io.con_key && R.nact > 0) {         // the keys of those contacts, in emit_robot_contacts' order
+      int o = R.off;
+#pragma unroll 1
+      for (int p = m.ncbpass; p < KM_NPASS; ++p)
+#pragma unroll 1
+        for (int k = 0; k < 2; ++k)
+          if ((R.actmask >> (2 * p + k)) & 1) { if (o < KM_NC_TOT) io.con_key[o] = KP_SLOT(m.rp[p * KW + lane]) + k; ++o; }
+    }
     for (int sl = lane; sl < 32; sl += KW) {
       if (!(bmask & (1u << sl))) continue;
       const int o = nrob + KPOPC(bmask & ((1u << sl) - 1u)), q = sl >> 2;
+      if (CON && io.con_key && o < KM_NC_TOT) io.con_key[o] = m.nslot_robot + sl;
       if (o < KM_NC_TOT) {
         const bool sw = m.bp_type[q] == KB_BOX_BOX_SWAP;
         const float* st = S.bstage[q][sl & 3];
@@ -2037,6 +2058,18 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
       }
     }
   END_LANES
+  if (CON && io.con_rec) {
+    LANES(W, R)
+#pragma unroll 1
+      for (int c = lane; c < ncon; c += KW) {
+        const float* g = S.template geo<true>(c);
+        float* rec = io.con_rec + c * KM_CON_REC;
+        rec[0] = g[12];
+#pragma unroll
+        for (int k = 0; k < 6; ++k) rec[1 + k] = g[k];
+      }
+    END_LANES
+  }
   PHASE(W, 18);
   PHASE_ALIGN();
   PHASE(W, 7);
@@ -2115,12 +2148,109 @@ struct RolloutArgs {
   // last step goes to the *_out rows (they may be the input rows: a sample reads its rows before it writes them)
   const float* warm0;
   float* qpos_out; float* qvel_out; float* warm_out;
+  // CONTACTS only: the last step's contacts and constraint forces (contact_outputs).  slot_map [nslot_robot + 4 nbpair]
+  // maps a contact key to the model's contact slot; qfrc [12], ncon [1], con_slot [KM_NC_TOT], con_rec [KM_NC_TOT][KM_CON_REC]
+  const int* slot_map;
+  float* qfrc; int* ncon; int* con_slot; float* con_rec;
 };
+
+// The contact list and constraint forces of the last forward() (rollout_sample<.., CONTACTS>), after MJX's solver finish:
+// at the accepted qacc, Jaref_r = J_r qacc - aref_r and f_r = -D_r Jaref_r where Jaref_r < 0 (SURVEY BD.10).  Reads the
+// rows the last solve left in the sample's record and the keys and geometry step_forward<NC, true> put in A.con_slot /
+// A.con_rec (list order); writes the contacts sorted by model slot, padded with slot -1 and zero records, and
+// qfrc_constraint = sum_r J_r^T f_r, summed over the limit rows, then the contacts in slot order (the row order of
+// oracle/mjstep.c make_constraint).  Per contact, force = (sum f, mu (f0 - f1), mu (f2 - f3)) of its four pyramid rows
+// Jn + mu Jt1, Jn - mu Jt1, Jn + mu Jt2, Jn - mu Jt2 (mju_decodePyramid).
+template <int NC>
+KFN void contact_outputs(Warp& W, const KModel& m, WarpSmemT<NC>& S, const RolloutArgs& A) {
+  const int ncon = A.live ? S.ncon : 0, nlim = S.nlim;       // (a padding sample wrote no keys)
+  int* inv = reinterpret_cast<int*>(&S.H[0][0]);      // list position of the k-th contact in slot order (H is dead here)
+  // (1) per contact: the force sums of its rows, which replace the contact record's dead fields with the geometry kept in
+  //     A.con_rec (g[0..2] force sums, g[3..5] normal, g[6..8] position, g[13] model slot; g[12] dist and the links stay)
+  LANES(W, R)
+#pragma unroll 1
+    for (int c = lane; c < ncon; c += KW) {
+      float* g = S.template geo<true>(c);
+      const float* J = S.template jac<true>(c);
+      const int blk = contact_blocks(g), o = (blk & 1) ? 0 : KM_NL, nd = blk == 3 ? KM_NV : KM_NL;
+      float dn = 0.f, d1 = 0.f, d2 = 0.f;
+#pragma unroll 1
+      for (int d = o; d < o + nd; ++d) { dn += J[d] * S.qacc[d]; d1 += J[12 + d] * S.qacc[d]; d2 += J[24 + d] * S.qacc[d]; }
+      float f[4];
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const int r = nlim + 4 * c + q;
+        const float dt = q < 2 ? d1 : d2;
+        const float ja = ((q & 1) ? dn - dt : dn + dt) - S.template Aref<true>(r, nlim);
+        f[q] = ja < 0.f ? -S.template D<true>(r, nlim) * ja : 0.f;
+      }
+      const float* rec = A.con_rec + c * KM_CON_REC;
+      const int slot = A.slot_map[A.con_slot[c]];
+      g[0] = f[0] + f[1] + f[2] + f[3]; g[1] = f[0] - f[1]; g[2] = f[2] - f[3];
+#pragma unroll
+      for (int k = 0; k < 3; ++k) { g[3 + k] = rec[4 + k]; g[6 + k] = rec[1 + k]; }
+      g[13] = __int_as_float(slot);
+    }
+  END_LANES
+  // (2) ranks by model slot (the slots of a sample's contacts are distinct)
+  LANES(W, R)
+#pragma unroll 1
+    for (int c = lane; c < ncon; c += KW) {
+      const int s = __float_as_int(S.template geo<true>(c)[13]);
+      int rank = 0;
+#pragma unroll 1
+      for (int c2 = 0; c2 < ncon; ++c2) rank += __float_as_int(S.template geo<true>(c2)[13]) < s ? 1 : 0;
+      inv[rank] = c;
+    }
+  END_LANES
+  // (3) the sorted outputs and qfrc_constraint
+  LANES(W, R)
+    if (A.live) {
+#pragma unroll 1
+      for (int k = lane; k < KM_NC_TOT; k += KW) {
+        float* rec = A.con_rec + k * KM_CON_REC;
+        if (k < ncon) {
+          const float* g = S.template geo<true>(inv[k]);
+          A.con_slot[k] = __float_as_int(g[13]);
+          rec[0] = g[12];
+          rec[1] = g[6]; rec[2] = g[7]; rec[3] = g[8];
+          rec[4] = g[3]; rec[5] = g[4]; rec[6] = g[5];
+          rec[7] = g[0]; rec[8] = m.mu * g[1]; rec[9] = m.mu * g[2];
+          rec[10] = 0.f; rec[11] = 0.f;
+        } else {
+          A.con_slot[k] = -1;
+#pragma unroll
+          for (int i = 0; i < KM_CON_REC; ++i) rec[i] = 0.f;
+        }
+      }
+      if (lane < KM_NV) {
+        float fc = 0.f;
+#pragma unroll 1
+        for (int r = 0; r < nlim; ++r) {
+          if (S.limdof[r] != lane) continue;
+          const float ja = S.limsign[r] * S.qacc[lane] - S.rAref[r];
+          if (ja < 0.f) fc += S.limsign[r] * (-S.rD[r] * ja);
+        }
+        const int need = lane < KM_NL ? 1 : 2;
+#pragma unroll 1
+        for (int k = 0; k < ncon; ++k) {
+          const float* g = S.template geo<true>(inv[k]);
+          if (!(contact_blocks(g) & need)) continue;        // the Jacobian only exists in the blocks the contact touches
+          const float* J = S.template jac<true>(inv[k]);
+          fc += J[lane] * g[0] + J[12 + lane] * g[1] + J[24 + lane] * g[2];
+        }
+        A.qfrc[lane] = fc;
+      }
+      if (lane == 0) *A.ncon = ncon;
+    }
+  END_LANES
+}
 
 // STATES = false: a planner rollout from the KModel snapshot (arm state q0 / v0, shared by all samples) with its cost.
 // STATES = true: the same steps from the sample's own state rows, which it writes back after the last step; thetadot
 // may be null with T = 1 (the sample keeps its own qvel[:6], a plain mjx.step), theta is optional, no cost, no target.
-template <int NC, bool STATES = false>
+// CONTACTS (with STATES): also the contacts and constraint forces of the last step (contact_outputs).
+template <int NC, bool STATES = false, bool CONTACTS = false>
 KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const RolloutArgs& A) {
   LANES(W, R)
     if (STATES) {
@@ -2158,7 +2288,12 @@ KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const Rollou
     io.first = t == 0;
     io.collision_row = (A.collision && A.live) ? A.collision + (size_t)t * m.nslot_robot : nullptr;
     io.prevd = A.prevd;
-    step_forward<NC>(W, m, S, io);
+    if (CONTACTS) {
+      const bool last = A.live && t + 1 == A.T;
+      io.con_key = last ? A.con_slot : nullptr;
+      io.con_rec = last ? A.con_rec : nullptr;
+    }
+    step_forward<NC, CONTACTS>(W, m, S, io);
     PHASE(W, 12);
     // pre-step observations (mjx_planner.py:259-261) and running cost (:277-285)
     {
@@ -2187,6 +2322,7 @@ KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const Rollou
     PHASE(W, 12);
     STEPEND(W);
   }
+  if (CONTACTS) contact_outputs<NC>(W, m, S, A);           // (step_euler changes nothing it reads)
   if (STATES) {
     LANES(W, R)
       if (A.live) {

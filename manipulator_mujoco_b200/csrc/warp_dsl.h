@@ -46,7 +46,7 @@
 // missing fence) gives that lane the stale value here and the results differ.  Two lanes writing different values to
 // the same scratch byte in one block are counted directly (RaceState::waw).
 struct RaceState {
-  struct Region { unsigned char* p; size_t n; } reg[4];
+  struct Region { unsigned char* p; size_t n; } reg[8];
   int nreg = 0, open = -1, line = 0;
   long long waw = 0, blocks = 0;
   int first_line = 0, first_word = 0, first_lanes = 0;      // where the first write-write conflict was seen (source line of the block)

@@ -255,10 +255,12 @@ def build_kmodel(mc: ModelConsts, timestep: float, robot_geom_names=None, tcp_si
     # ---- pairs ----
     robot_ids = {mc.geom_id(n) for n in robot_geom_names if n in mc.geom_names}
     rpairs, bpairs, slot = [], [], 0
-    for (g1, g2), ns in zip(mc.pair_geom, mc.pair_nslot):
+    robot_slots, box_slots = [], []           # the model's contact slot of each robot slot / free-box pair slot
+    for (g1, g2), ns, adr in zip(mc.pair_geom, mc.pair_nslot, mc.pair_slotadr):
         g1, g2 = int(g1), int(g2)
         is_robot = g1 in robot_ids or g2 in robot_ids
         if g1 in caps or g2 in caps:
+            robot_slots.extend(range(int(adr), int(adr) + int(ns)))
             if not is_robot:
                 raise NotImplementedError("every capsule pair must be robot-involving (cost mask)")
             if g1 in planes:
@@ -276,6 +278,7 @@ def build_kmodel(mc: ModelConsts, timestep: float, robot_geom_names=None, tcp_si
             if is_robot:
                 raise NotImplementedError("robot geoms must be capsules")
             other = g1 if g2 == fbox else g2
+            box_slots.extend(int(adr) + k if k < ns else -1 for k in range(4))     # the kernel stages four slots per pair
             if fbox not in (g1, g2):
                 raise NotImplementedError("non-robot pair without the free box")
             if other in planes:
@@ -316,5 +319,8 @@ def build_kmodel(mc: ModelConsts, timestep: float, robot_geom_names=None, tcp_si
     _set(m.qpos0, mc.qpos0)
     if warm0 is not None:
         _set(m.warm0, warm0)
-    info = dict(links=links, nslot_robot=slot, robot_ids=sorted(robot_ids))
+    # contact_key_slot: the model's contact slot of each contact key of the kernel (cemk_step_states_contacts' slot_map):
+    # key k < nslot_robot is robot slot k, key nslot_robot + 4 q + j is slot j of free-box pair q
+    info = dict(links=links, nslot_robot=slot, robot_ids=sorted(robot_ids),
+                contact_key_slot=np.array(robot_slots + box_slots, dtype=np.int32))
     return m, info

@@ -181,6 +181,7 @@ class cem_planner:
         self.data = _DataView(self._mc)
         km, info = build_kmodel(self._mc, self.t)
         self.mjx_model = km
+        self._key_slot, self._key_slot_dev = info["contact_key_slot"], None
         self.geom_ids = np.array([self._mc.geom_id(f'robot_{i}') for i in range(10)])
         mask = np.zeros(self._mc.ncon, dtype=bool)
         for (g1, g2), a, n in zip(self._mc.pair_geom, self._mc.pair_slotadr, self._mc.pair_nslot):
@@ -486,13 +487,31 @@ class cem_planner:
         theta, _c, eef_pos, eef_rot, collision = self._rollout(thetadot, init_pos, init_vel, tp, tr, True)
         return theta, eef_pos, eef_rot, collision
 
-    def step_batch(self, qpos, qvel, qacc_warmstart, thetadot=None):
+    @property
+    def contact_slot_geoms(self):
+        """[ncon, 2] geom ids of each contact slot of the model (``contact_slot`` of ``step_batch(..., contacts=True)``);
+        names through ``model.geom``.  Read-only."""
+        mc = self._mc
+        g = np.zeros((mc.ncon, 2), dtype=np.int64)
+        for (g1, g2), a, n in zip(mc.pair_geom, mc.pair_slotadr, mc.pair_nslot):
+            g[a:a + n] = (g1, g2)
+        g.flags.writeable = False
+        return g
+
+    def step_batch(self, qpos, qvel, qacc_warmstart, thetadot=None, contacts=False):
         """``jax.vmap(jit_step, in_axes=(None, 0))``: N environments, each stepped from its own state in one launch
         (``cemk_step_states``); the planner's model snapshot is not used or changed.  qpos [N, 13], qvel [N, 12],
         qacc_warmstart [N, 12] (numpy or torch).  ``thetadot`` [N, 6T] (dof-major, the rollout's layout) chains T steps with
         qvel[:6] set to thetadot[:, t] before step t (mjx_planner.py:254); without it each environment takes one plain step
         with its own qvel.  Returns CUDA tensors: qpos, qvel, qacc (last step), qacc_warmstart (= that qacc), overflow [N]
-        (bool: more simultaneous contacts than the kernel keeps, extra ones dropped) and, with thetadot, theta [N, 6T]."""
+        (bool: more simultaneous contacts than the kernel keeps, extra ones dropped) and, with thetadot, theta [N, 6T].
+
+        ``contacts=True`` (``cemk_step_states_contacts``) adds what MJX's Data holds about the constraints of the last step,
+        at its final qacc: qfrc_constraint [N, 12], ncon [N] (contacts kept, at most 48) and, per contact sorted by contact
+        slot and padded with slot -1 and zeros: contact_slot [N, 48] (int32; geoms in ``contact_slot_geoms``), contact_dist
+        [N, 48], contact_pos [N, 48, 3], contact_normal [N, 48, 3] (first row of the contact frame) and contact_force
+        [N, 48, 3] (normal, tangent 1, tangent 2 in the contact frame, mju_decodePyramid of the four pyramid rows).  The
+        state outputs are the same bits as with ``contacts=False``."""
         self._require_rollout_dof("step_batch")
         qp, qv, wm = self._t(qpos), self._t(qvel), self._t(qacc_warmstart)
         if qp.dim() != 2 or qp.shape[1] != 13 or qp.shape[0] == 0:
@@ -514,12 +533,25 @@ class cem_planner:
             self._graph, self._graph_out, self._eager_ticks = None, None, 0
         qpos_out, qvel_out, warm_out = torch.empty(N, 13, device=dev), torch.empty(N, 12, device=dev), torch.empty(N, 12, device=dev)
         flags = torch.empty(N, dtype=torch.int32, device=dev)
-        _lib.check(self._lib.cemk_step_states(self._h, N, T, _ptr(qp), _ptr(qv), _ptr(wm), _ptr(td), _ptr(qpos_out), _ptr(qvel_out),
-                                              _ptr(warm_out), _ptr(theta), None, None, None, None, _ptr(flags), self._stream()), self._lib)
+        if not contacts:
+            _lib.check(self._lib.cemk_step_states(self._h, N, T, _ptr(qp), _ptr(qv), _ptr(wm), _ptr(td), _ptr(qpos_out), _ptr(qvel_out),
+                                                  _ptr(warm_out), _ptr(theta), None, None, None, None, _ptr(flags), self._stream()), self._lib)
+        else:
+            if self._key_slot_dev is None:
+                self._key_slot_dev = torch.as_tensor(self._key_slot, dtype=torch.int32, device=dev)
+            qfrc, ncon = torch.empty(N, 12, device=dev), torch.empty(N, dtype=torch.int32, device=dev)
+            slot, rec = torch.empty(N, 48, dtype=torch.int32, device=dev), torch.empty(N, 48, 12, device=dev)
+            _lib.check(self._lib.cemk_step_states_contacts(
+                self._h, N, T, _ptr(qp), _ptr(qv), _ptr(wm), _ptr(td), _ptr(qpos_out), _ptr(qvel_out), _ptr(warm_out), _ptr(theta),
+                None, None, None, None, _ptr(flags), _ptr(self._key_slot_dev), _ptr(qfrc), _ptr(ncon), _ptr(slot), _ptr(rec),
+                self._stream()), self._lib)
         self._keep_sb = (qp, qv, wm, td)
         out = dict(qpos=qpos_out, qvel=qvel_out, qacc=warm_out.clone(), qacc_warmstart=warm_out, overflow=(flags & 1).bool())
         if theta is not None:
             out["theta"] = theta
+        if contacts:
+            out.update(qfrc_constraint=qfrc, ncon=ncon, contact_slot=slot, contact_dist=rec[:, :, 0], contact_pos=rec[:, :, 1:4],
+                       contact_normal=rec[:, :, 4:7], contact_force=rec[:, :, 7:10])
         return out
 
     def compute_cost_batch(self, thetadot, eef_pos, eef_rot, collision, target_pos, target_rot):
