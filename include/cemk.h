@@ -124,6 +124,35 @@ int cemk_step_states_contacts(cemk_handle* h, int N, int T, const float* qpos, c
                               float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags, const int* slot_map,
                               float* qfrc_constraint, int* ncon, int* con_slot, float* con_rec, void* stream);
 
+/* Scenes and start states given per call.  The model's topology, sizes, pairs, floor plane and robot stay the handle's;
+ * only the poses of the static boxes and the free box's start state become inputs (float32, device):
+ *   scene record [CEMK_SCENE_FLOATS] = the KModel's sb_pos[8][4] | sb_mat[8][12] | sb_size[8][4] block: per static box its
+ *     world position, rotation matrix (row-major) with its half sizes along the world axes in [9..11] when the box is
+ *     axis-aligned, half sizes with [3] = 1 for an axis-aligned box; unused rows zero.  Build it with
+ *     manipulator_mujoco_b200.kmodel.scene_records (cem_planner.make_scene): a hand-made record whose flag and world half
+ *     sizes disagree with its rotation gives wrong far-field tests.
+ *   start record [CEMK_START_FLOATS] = the KModel's qpos0[16] | warm0[12] | qvel0[12] block: qpos[13] (3 unused), qacc_warmstart[12],
+ *     qvel[12].  A planner rollout takes the free box (qpos[6:13], qvel[6:12]) and the warm start from it; the arm still
+ *     comes from q0 / v0.
+ * The handle's table holds the default records, so a NULL record and the table's own give the same bits; nothing is stored
+ * in the handle.
+ * cemk_rollout_cost_scene: cemk_rollout_cost with a scene (sample s reads scene + s * scene_stride; scene_stride 0 = one
+ *   scene for all samples, or CEMK_SCENE_FLOATS) and a start record, each NULL for the handle's own.
+ * cemk_step_states_scene: cemk_step_states_contacts with per-environment (scene_stride CEMK_SCENE_FLOATS) or shared (0)
+ *   scenes, NULL for the handle's own.  The environments' state rows hold their start state.
+ * Both refuse what the calls they extend refuse, and a scene_stride other than 0 or CEMK_SCENE_FLOATS (CEMK_ERR_ARG). */
+#define CEMK_SCENE_FLOATS 160
+#define CEMK_START_FLOATS 40
+int cemk_rollout_cost_scene(cemk_handle* h, int B, int T, const float* thetadot, const float* q0, const float* v0,
+                            const float* target_pos, const float* target_rot, float w_pos, float w_rot, float w_col,
+                            float* theta, float* cost4, float* eef_pos, float* eef_rot, float* collision, float* qacc,
+                            int* flags, const float* scene, int scene_stride, const float* start, void* stream);
+int cemk_step_states_scene(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm,
+                           const float* thetadot, float* qpos_out, float* qvel_out, float* warm_out, float* theta,
+                           float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags, const int* slot_map,
+                           float* qfrc_constraint, int* ncon, int* con_slot, float* con_rec, const float* scene, int scene_stride,
+                           void* stream);
+
 /* compute_cost_batch alone (mjx_planner.py:277-303), per-sample targets as in the reference method:
  *   eef_pos[B][T][3], eef_rot[B][T][4], collision[B][T][nslot], target_pos[B][3], target_rot[B][4] -> cost4[B][4]. */
 int cemk_cost_batch(cemk_handle* h, int B, int T, int nslot, const float* eef_pos, const float* eef_rot,

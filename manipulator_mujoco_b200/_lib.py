@@ -49,6 +49,8 @@ _SIGS = {
     "cemk_rollout_cost": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
     "cemk_step_states": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], _i),
     "cemk_step_states_contacts": ([_vp, _i, _i] + [_vp] * 19, _i),
+    "cemk_rollout_cost_scene": ([_vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f] + [_vp] * 7 + [_vp, _i, _vp, _vp], _i),
+    "cemk_step_states_scene": ([_vp, _i, _i] + [_vp] * 18 + [_vp, _i, _vp], _i),
     "cemk_cost_batch": ([_vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _f, _f, _vp, _vp], _i),
     "cemk_argsort_topk": ([_vp, _i, _vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp], _i),
     "cemk_topk_pack": ([_vp, _i, _vp, _i, _i, _vp, _i, _vp, _vp, _vp], _i),

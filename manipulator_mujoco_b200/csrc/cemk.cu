@@ -6,6 +6,7 @@
 //   k_rollout                vmap(scan(mjx.step)) + compute_cost_batch     (:251-303)   <- hot kernel
 //   k_rollout<.., STATES>    vmap(mjx.step) over per-environment states, chained T steps (cemk_step_states)
 //   k_rollout<.., STATES, CONTACTS>   the same, plus the last step's contacts and constraint forces (cemk_step_states_contacts)
+//   k_rollout_scene<..>      any of the above against scene / start records given per call (cemk_*_scene)
 //   k_cost_batch             compute_cost_batch on materialised trajectories (:277-303)
 //   k_rank_select (n <= 8192) | k_make_keys / k_bitonic* / k_gather_sorted    compute_ellite_samples   (:306-310)
 //   k_merge_lists            the same selection over the per-rank sorted lists of several GPUs
@@ -13,6 +14,7 @@
 //   k_tick_record            what compute_cem keeps of an iteration        (:390-404)
 // The rollout core lives in rollout_core.h (shared with the CPU emulation used by the no-GPU tests).
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -20,6 +22,12 @@
 #include "../../include/cemk.h"
 #include "rollout_core.h"
 static_assert(CEMK_MAX_CONTACTS == KM_NC_TOT && CEMK_CONTACT_REC == KM_CON_REC, "contact output layout of cemk.h");
+static_assert(CEMK_SCENE_FLOATS == KM_SCENE_FLOATS && CEMK_START_FLOATS == KM_START_FLOATS, "record sizes of cemk.h");
+static_assert(offsetof(KModel, sb_mat) == offsetof(KModel, sb_pos) + 4 * 4 * KM_MAXSBOX &&
+              offsetof(KModel, sb_size) == offsetof(KModel, sb_pos) + 4 * 16 * KM_MAXSBOX &&
+              offsetof(KModel, fb_size) == offsetof(KModel, sb_pos) + 4 * KM_SCENE_FLOATS, "scene record = sb_pos | sb_mat | sb_size");
+static_assert(offsetof(KModel, warm0) == offsetof(KModel, qpos0) + 4 * 16 && offsetof(KModel, qvel0) == offsetof(KModel, qpos0) + 4 * 28 &&
+              sizeof(KModel) == offsetof(KModel, qpos0) + 4 * KM_START_FLOATS, "start record = qpos0 | warm0 | qvel0");
 
 // Bernstein order n (mjx_planner.py:40 hard-codes 10; SURVEY 8 f.4 asks for order n): ncoef = n + 1 coefficients per DOF,
 // nvar = ndof ncoef decision variables, chosen per handle by cemk_set_dof / cemk_set_order (default 6 DOF x 11 = 66).  The
@@ -87,6 +95,11 @@ struct RolloutBatch {
   const int* slot_map;
   float* qfrc; int* ncon; int* con_slot; float* con_rec;
 };
+// k_rollout_scene: sample s reads the scene record scene + s * stride (stride 0: one record for all) and, without STATES,
+// the start record `start`.
+struct SceneArgs {
+  const float* scene; int stride; const float* start;
+};
 
 // NC = contacts of a sample kept in shared memory (the rest, up to KM_NC_TOT, in the global spill area),
 // WARPS = warps per CTA; a warp carries 32 / KW samples (one per lane group, warp_dsl.h).  The fast
@@ -94,9 +107,11 @@ struct RolloutBatch {
 // cemk_set_option("force_rerun"): NC = 48 (no spill area), one warp per CTA, samples whose flag bit 0 is set.
 // STATES: every sample steps from its own state rows and writes its final state (cemk_step_states, rollout_sample).
 // CONTACTS (with STATES): and the last step's contacts and constraint forces (cemk_step_states_contacts, contact_outputs).
+// SCENE: static boxes (and, without STATES, the snapshot) from the call's records (cemk_rollout_cost_scene, cemk_step_states_scene):
+// the kernels k_rollout_scene, with a parameter of their own; k_rollout keeps its signature.
 #define GPW (32 / KW)                                     // lane groups (samples) per warp
-template <int NC, int WARPS, bool ONLY_FLAGGED, bool STATES = false, bool CONTACTS = false>
-__global__ void __launch_bounds__(WARPS * 32, 1) k_rollout(const KModel* __restrict__ gm, RolloutBatch a) {
+template <int NC, int WARPS, bool ONLY_FLAGGED, bool STATES, bool CONTACTS, bool SCENE>
+__device__ __forceinline__ void rollout_cta(const KModel* __restrict__ gm, RolloutBatch a, SceneArgs sc) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   KModel* sm = reinterpret_cast<KModel*>(smem_raw);
   WarpSmemT<NC>* ws = reinterpret_cast<WarpSmemT<NC>*>(smem_raw + ((sizeof(KModel) + 15) & ~size_t(15)));
@@ -159,13 +174,21 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_rollout(const KModel* __restr
     A.qfrc = a.qfrc + (size_t)s * KM_NV; A.ncon = a.ncon + s;
     A.con_slot = a.con_slot + (size_t)s * KM_NC_TOT; A.con_rec = a.con_rec + (size_t)s * KM_NC_TOT * KM_CON_REC;
   }
-  rollout_sample<NC, STATES, CONTACTS>(W, *sm, ws[group], A);
+  rollout_sample<NC, STATES, CONTACTS, SCENE>(W, *sm, ws[group], A, SCENE ? sc.scene + (size_t)s * sc.stride : nullptr, sc.start);
 #ifdef CEMK_PHASE_TIMING
   PHASE(W, 15);
   if (W.lane == 0 && !ONLY_FLAGGED) for (int i = 0; i < 24; ++i) atomicAdd(&g_phase[i], (unsigned long long)W.ph[i]);
   if (W.lane == 0 && !ONLY_FLAGGED) for (int i = 0; i < 24; ++i) atomicAdd(&g_event[i], (unsigned long long)W.ev[i]);
   if (W.lane == 0 && !ONLY_FLAGGED) { for (int i = 0; i < 24; ++i) atomicAdd(&g_phase_cond[i], (unsigned long long)W.phc[i]); atomicAdd(&g_phase_cond[24], (unsigned long long)W.nflag); }
 #endif
+}
+template <int NC, int WARPS, bool ONLY_FLAGGED, bool STATES = false, bool CONTACTS = false>
+__global__ void __launch_bounds__(WARPS * 32, 1) k_rollout(const KModel* __restrict__ gm, RolloutBatch a) {
+  rollout_cta<NC, WARPS, ONLY_FLAGGED, STATES, CONTACTS, false>(gm, a, SceneArgs{});
+}
+template <int NC, int WARPS, bool ONLY_FLAGGED, bool STATES = false, bool CONTACTS = false>
+__global__ void __launch_bounds__(WARPS * 32, 1) k_rollout_scene(const KModel* __restrict__ gm, RolloutBatch a, SceneArgs sc) {
+  rollout_cta<NC, WARPS, ONLY_FLAGGED, STATES, CONTACTS, true>(gm, a, sc);
 }
 template <int NC, int WARPS>
 static size_t rollout_smem() { return ((sizeof(KModel) + 15) & ~size_t(15)) + WARPS * GPW * sizeof(WarpSmemT<NC>); }
@@ -953,8 +976,8 @@ static int rollout_dof_check(const cemk_handle* h, const char* fn) {
 // One launch of the product rollout over a.B samples (cemk_rollout_cost, and cemk_step_states[_contacts] with STATES
 // [and CONTACTS]): grows the library scratch to a.B samples (the flags when a.flags is null, the previous distances, the
 // spill area), points `a` at it and chooses the CTA shares.
-template <bool STATES, bool CONTACTS = false>
-static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
+template <bool STATES, bool CONTACTS = false, bool SCENE = false>
+static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st, const SceneArgs& sc = SceneArgs{}) {
   const int B = a.B;
   if (!a.flags) {
     if (h->flags_cap < B) {
@@ -983,7 +1006,10 @@ static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
   const int nsm = h->num_sms > 0 ? h->num_sms : 148;
   const int cap = ROLLOUT_WARPS * GPW, unit = 4 * GPW;
   int grid;
-#define CEMK_LAUNCH_ROLLOUT(W_) k_rollout<KM_NC_FAST, W_, false, STATES, CONTACTS><<<grid, (W_) * 32, rollout_smem<KM_NC_FAST, W_>(), st>>>(h->d_model, a)
+#define CEMK_LAUNCH_ROLLOUT(W_) do {                                                                                             \
+    if constexpr (SCENE) k_rollout_scene<KM_NC_FAST, W_, false, STATES, CONTACTS><<<grid, (W_) * 32, rollout_smem<KM_NC_FAST, W_>(), st>>>(h->d_model, a, sc); \
+    else k_rollout<KM_NC_FAST, W_, false, STATES, CONTACTS><<<grid, (W_) * 32, rollout_smem<KM_NC_FAST, W_>(), st>>>(h->d_model, a);                      \
+  } while (0)
   const int need = (B + nsm - 1) / nsm;                            // samples per SM
   if (need <= cap) {
     a.n_hi = 0; a.w_hi = a.w_lo = need; grid = (B + need - 1) / need;
@@ -1004,9 +1030,26 @@ static int launch_rollout(cemk_handle* h, RolloutBatch& a, cudaStream_t st) {
   return CEMK_OK;
 }
 
+// shared-memory size of the three product widths of k_rollout_scene<.., STATES, CONTACTS>
+template <bool STATES, bool CONTACTS>
+static int rollout_smem_attrs() {
+  CK(cudaFuncSetAttribute(k_rollout_scene<KM_NC_FAST, ROLLOUT_WARPS, false, STATES, CONTACTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)rollout_smem<KM_NC_FAST, ROLLOUT_WARPS>()));
+  CK(cudaFuncSetAttribute(k_rollout_scene<KM_NC_FAST, 8, false, STATES, CONTACTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)rollout_smem<KM_NC_FAST, 8>()));
+  CK(cudaFuncSetAttribute(k_rollout_scene<KM_NC_FAST, 4, false, STATES, CONTACTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)rollout_smem<KM_NC_FAST, 4>()));
+  return CEMK_OK;
+}
+
+// The handle's own scene / start record: the blocks of its device table (what the launches without SCENE read)
+static const float* model_block(const cemk_handle* h, size_t offset) {
+  return reinterpret_cast<const float*>(reinterpret_cast<const char*>(h->d_model) + offset);
+}
+
 extern "C" {
 
-int cemk_version(void) { return 6; }
+int cemk_version(void) { return 7; }
 const char* cemk_last_error(void) { return g_err; }
 int cemk_sizeof_kmodel(void) { return (int)sizeof(KModel); }
 
@@ -1036,6 +1079,11 @@ int cemk_create(const void* kmodel, int kmodel_bytes, int device, cemk_handle** 
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 8, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 8>()));
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_FAST, 4, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rollout_smem<KM_NC_FAST, 4>()));
   CK(cudaFuncSetAttribute(k_rollout<KM_NC_BIG, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)rollout_smem<KM_NC_BIG, 1>()));
+  { const int rc = rollout_smem_attrs<false, false>(); if (rc) return rc; }     // the SCENE instantiations
+  { const int rc = rollout_smem_attrs<true, false>(); if (rc) return rc; }
+  { const int rc = rollout_smem_attrs<true, true>(); if (rc) return rc; }
+  CK(cudaFuncSetAttribute(k_rollout_scene<KM_NC_BIG, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                           (int)rollout_smem<KM_NC_BIG, 1>()));
   h->d_mc = nullptr;
   { const int rc = mc_alloc(h); if (rc) return rc; }
@@ -1143,11 +1191,14 @@ int cemk_project(cemk_handle* h, int B, int iters, const float* xi, const float*
   return CEMK_OK;
 }
 
-int cemk_rollout_cost(cemk_handle* h, int B, int T, const float* thetadot, const float* q0, const float* v0, const float* target_pos,
-                      const float* target_rot, float w_pos, float w_rot, float w_col, float* theta, float* cost4, float* eef_pos,
-                      float* eef_rot, float* collision, float* qacc, int* flags, void* stream) {
+int cemk_rollout_cost_scene(cemk_handle* h, int B, int T, const float* thetadot, const float* q0, const float* v0,
+                            const float* target_pos, const float* target_rot, float w_pos, float w_rot, float w_col, float* theta,
+                            float* cost4, float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags,
+                            const float* scene, int scene_stride, const float* start, void* stream) {
   if (!h || !thetadot || !q0 || !v0 || !target_pos || !target_rot || !theta || !cost4 || B <= 0 || T <= 0)
     return set_err(CEMK_ERR_ARG, "cemk_rollout_cost: bad argument");
+  if (scene_stride != 0 && scene_stride != KM_SCENE_FLOATS)
+    return set_err(CEMK_ERR_ARG, "cemk_rollout_cost_scene: scene_stride must be 0 or CEMK_SCENE_FLOATS");
   { const int rc = rollout_dof_check(h, "cemk_rollout_cost"); if (rc) return rc; }
   DevGuard guard(h->device);
   cudaStream_t st = (cudaStream_t)stream;
@@ -1155,23 +1206,37 @@ int cemk_rollout_cost(cemk_handle* h, int B, int T, const float* thetadot, const
   a.B = B; a.T = T; a.thetadot = thetadot; a.q0 = q0; a.v0 = v0; a.target_pos = target_pos; a.target_rot = target_rot;
   a.w_pos = w_pos; a.w_rot = w_rot; a.w_col = w_col;
   a.theta = theta; a.cost4 = cost4; a.eef_pos = eef_pos; a.eef_rot = eef_rot; a.collision = collision; a.qacc = qacc; a.flags = flags;
-  { const int rc = launch_rollout<false>(h, a, st); if (rc) return rc; }
+  // no record: the table's own (the launch without SCENE); one record: the table's block stands in for the other
+  const bool scn = scene || start;
+  SceneArgs sc;
+  sc.scene = scene ? scene : model_block(h, offsetof(KModel, sb_pos));
+  sc.stride = scene ? scene_stride : 0;
+  sc.start = start ? start : model_block(h, offsetof(KModel, qpos0));
+  { const int rc = scn ? launch_rollout<false, false, true>(h, a, st, sc) : launch_rollout<false>(h, a, st); if (rc) return rc; }
   // debug option: recompute every sample with the all-in-shared-memory instantiation (no spill area)
   if (h->force_rerun) {
     CK(cudaMemsetAsync(a.flags, 1, sizeof(int) * B, st));                      // 0x01010101: bit 0 set
     a.n_hi = 0; a.w_hi = a.w_lo = GPW;
-    k_rollout<KM_NC_BIG, 1, true><<<(B + GPW - 1) / GPW, 32, rollout_smem<KM_NC_BIG, 1>(), st>>>(h->d_model, a);
+    if (scn) k_rollout_scene<KM_NC_BIG, 1, true><<<(B + GPW - 1) / GPW, 32, rollout_smem<KM_NC_BIG, 1>(), st>>>(h->d_model, a, sc);
+    else k_rollout<KM_NC_BIG, 1, true><<<(B + GPW - 1) / GPW, 32, rollout_smem<KM_NC_BIG, 1>(), st>>>(h->d_model, a);
     h->launches += 1;
   }
   CK(cudaPeekAtLastError());
   return CEMK_OK;
 }
 
+int cemk_rollout_cost(cemk_handle* h, int B, int T, const float* thetadot, const float* q0, const float* v0, const float* target_pos,
+                      const float* target_rot, float w_pos, float w_rot, float w_col, float* theta, float* cost4, float* eef_pos,
+                      float* eef_rot, float* collision, float* qacc, int* flags, void* stream) {
+  return cemk_rollout_cost_scene(h, B, T, thetadot, q0, v0, target_pos, target_rot, w_pos, w_rot, w_col, theta, cost4, eef_pos,
+                                 eef_rot, collision, qacc, flags, nullptr, 0, nullptr, stream);
+}
+
 // force_rerun does not apply here: it re-reads the samples' inputs after the product launch, and with in-place outputs
 // those rows already hold the stepped states.
-// cemk_step_states and cemk_step_states_contacts: the checks and the launch; fn names the entry in error messages, and
-// with a.slot_map set the contact outputs are written too
-static int step_states(cemk_handle* h, RolloutBatch& a, void* stream, const char* fn) {
+// cemk_step_states[_contacts|_scene]: the checks and the launch; fn names the entry in error messages, with a.slot_map set the
+// contact outputs are written too, and with sc.scene set the static boxes come from the scene records
+static int step_states(cemk_handle* h, RolloutBatch& a, const SceneArgs& sc, void* stream, const char* fn) {
   if (!h || !a.q0 || !a.v0 || !a.warm || !a.qpos_out || !a.qvel_out || !a.warm_out || a.B <= 0 || a.T <= 0) {
     snprintf(g_err, sizeof g_err, "%s: bad argument", fn);
     return CEMK_ERR_ARG;
@@ -1182,7 +1247,11 @@ static int step_states(cemk_handle* h, RolloutBatch& a, void* stream, const char
   }
   { const int rc = rollout_dof_check(h, fn); if (rc) return rc; }
   DevGuard guard(h->device);
-  { const int rc = a.slot_map ? launch_rollout<true, true>(h, a, (cudaStream_t)stream) : launch_rollout<true>(h, a, (cudaStream_t)stream); if (rc) return rc; }
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc;
+  if (sc.scene) rc = a.slot_map ? launch_rollout<true, true, true>(h, a, st, sc) : launch_rollout<true, false, true>(h, a, st, sc);
+  else rc = a.slot_map ? launch_rollout<true, true>(h, a, st) : launch_rollout<true>(h, a, st);
+  if (rc) return rc;
   CK(cudaPeekAtLastError());
   return CEMK_OK;
 }
@@ -1194,22 +1263,36 @@ int cemk_step_states(cemk_handle* h, int N, int T, const float* qpos, const floa
   a.B = N; a.T = T; a.thetadot = thetadot; a.q0 = qpos; a.v0 = qvel; a.warm = warm;
   a.qpos_out = qpos_out; a.qvel_out = qvel_out; a.warm_out = warm_out;
   a.theta = theta; a.eef_pos = eef_pos; a.eef_rot = eef_rot; a.collision = collision; a.qacc = qacc; a.flags = flags;
-  return step_states(h, a, stream, "cemk_step_states");
+  return step_states(h, a, SceneArgs{}, stream, "cemk_step_states");
+}
+
+int cemk_step_states_scene(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm,
+                           const float* thetadot, float* qpos_out, float* qvel_out, float* warm_out, float* theta,
+                           float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags, const int* slot_map,
+                           float* qfrc_constraint, int* ncon, int* con_slot, float* con_rec, const float* scene, int scene_stride,
+                           void* stream) {
+  const int given = (slot_map ? 1 : 0) + (qfrc_constraint ? 1 : 0) + (ncon ? 1 : 0) + (con_slot ? 1 : 0) + (con_rec ? 1 : 0);
+  if (given != 0 && given != 5)
+    return set_err(CEMK_ERR_ARG, scene ? "cemk_step_states_scene: slot_map and the contact outputs are all given or all NULL"
+                                       : "cemk_step_states_contacts: slot_map and the contact outputs are all given or all NULL");
+  if (scene_stride != 0 && scene_stride != KM_SCENE_FLOATS)
+    return set_err(CEMK_ERR_ARG, "cemk_step_states_scene: scene_stride must be 0 or CEMK_SCENE_FLOATS");
+  RolloutBatch a = {};
+  a.B = N; a.T = T; a.thetadot = thetadot; a.q0 = qpos; a.v0 = qvel; a.warm = warm;
+  a.qpos_out = qpos_out; a.qvel_out = qvel_out; a.warm_out = warm_out;
+  a.theta = theta; a.eef_pos = eef_pos; a.eef_rot = eef_rot; a.collision = collision; a.qacc = qacc; a.flags = flags;
+  a.slot_map = slot_map; a.qfrc = qfrc_constraint; a.ncon = ncon; a.con_slot = con_slot; a.con_rec = con_rec;
+  SceneArgs sc = {};
+  sc.scene = scene; sc.stride = scene ? scene_stride : 0;
+  return step_states(h, a, sc, stream, scene ? "cemk_step_states_scene" : "cemk_step_states_contacts");
 }
 
 int cemk_step_states_contacts(cemk_handle* h, int N, int T, const float* qpos, const float* qvel, const float* warm,
                               const float* thetadot, float* qpos_out, float* qvel_out, float* warm_out, float* theta,
                               float* eef_pos, float* eef_rot, float* collision, float* qacc, int* flags, const int* slot_map,
                               float* qfrc_constraint, int* ncon, int* con_slot, float* con_rec, void* stream) {
-  const int given = (slot_map ? 1 : 0) + (qfrc_constraint ? 1 : 0) + (ncon ? 1 : 0) + (con_slot ? 1 : 0) + (con_rec ? 1 : 0);
-  if (given != 0 && given != 5)
-    return set_err(CEMK_ERR_ARG, "cemk_step_states_contacts: slot_map and the contact outputs are all given or all NULL");
-  RolloutBatch a = {};
-  a.B = N; a.T = T; a.thetadot = thetadot; a.q0 = qpos; a.v0 = qvel; a.warm = warm;
-  a.qpos_out = qpos_out; a.qvel_out = qvel_out; a.warm_out = warm_out;
-  a.theta = theta; a.eef_pos = eef_pos; a.eef_rot = eef_rot; a.collision = collision; a.qacc = qacc; a.flags = flags;
-  a.slot_map = slot_map; a.qfrc = qfrc_constraint; a.ncon = ncon; a.con_slot = con_slot; a.con_rec = con_rec;
-  return step_states(h, a, stream, "cemk_step_states_contacts");
+  return cemk_step_states_scene(h, N, T, qpos, qvel, warm, thetadot, qpos_out, qvel_out, warm_out, theta, eef_pos, eef_rot, collision,
+                                qacc, flags, slot_map, qfrc_constraint, ncon, con_slot, con_rec, nullptr, 0, stream);
 }
 
 int cemk_cost_batch(cemk_handle* h, int B, int T, int nslot, const float* eef_pos, const float* eef_rot, const float* collision,

@@ -64,3 +64,9 @@ struct KModel {
   int bp_type[KM_MAXBPAIR], bp_a[KM_MAXBPAIR];
   float qpos0[16], warm0[12], qvel0[12];   // snapshot every rollout starts from (mjx_planner.py:267)
 };
+
+// The two pose blocks a rollout may take per call instead of the table's (cemk_rollout_cost_scene, cemk_step_states_scene):
+// a scene record is exactly sb_pos | sb_mat | sb_size (static box poses, unused rows zero), a start record exactly
+// qpos0 | warm0 | qvel0.  The table's own blocks are the default records.
+#define KM_SCENE_FLOATS (KM_MAXSBOX * (4 + 12 + 4))   // 160
+#define KM_START_FLOATS (16 + 12 + 12)                // 40

@@ -1536,8 +1536,13 @@ KNOINLINE void solve_rows_spilled(const KModel& m, WarpSmemT<NC>& S, int ncon, i
 // Inputs: S.qpos, S.qvel, S.warm.  Outputs: S.qacc (= new warm start), link frames, and the
 // collision-cost contribution of this step added to R.cost_c (mjx_planner.py:287-296).
 // CON: also the contact keys and geometry of io.con_key / io.con_rec when they are set.
-template <int NC, bool CON = false>
-KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& io) {
+// SCENE: the static boxes' poses come from the sample's scene record `scene` (the table's sb_pos | sb_mat | sb_size block,
+// KM_SCENE_FLOATS floats), not from the table.
+template <int NC, bool CON = false, bool SCENE = false>
+KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& io, const float* scene = nullptr) {
+  const float (*sb_pos)[4] = SCENE ? reinterpret_cast<const float (*)[4]>(scene) : m.sb_pos;
+  const float (*sb_mat)[12] = SCENE ? reinterpret_cast<const float (*)[12]>(scene + 4 * KM_MAXSBOX) : m.sb_mat;
+  const float (*sb_size)[4] = SCENE ? reinterpret_cast<const float (*)[4]>(scene + 16 * KM_MAXSBOX) : m.sb_size;
   PHASE(W, 1);
   // ---- P1: joint chain as a parallel prefix of rigid transforms.  Lane 0 holds the static base frame, lane
   //      i = 1..6 the local transform of link i-1 (body quat x joint rotation, body offset); composition
@@ -1734,15 +1739,15 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
         const bool st = p < m.nsbox;
         float la[3], lb[3];
         bool far;
-        if (st && m.sb_size[p][3] != 0.f) {
+        if (st && sb_size[p][3] != 0.f) {
           // axis-aligned static box: its frame is a signed permutation of the world axes, so the box coordinates are
           // the world offsets up to order and sign and the test is the same arithmetic on (A - c, B - c) with the
           // permuted half sizes -- bit-identical decision without the change of frame
-          sub3(la, A, m.sb_pos[p]); sub3(lb, B, m.sb_pos[p]);
-          far = capbox_far(la, lb, r, m.sb_mat[p] + 9);
+          sub3(la, A, sb_pos[p]); sub3(lb, B, sb_pos[p]);
+          far = capbox_far(la, lb, r, sb_mat[p] + 9);
         } else {
-          capbox_local(A, B, st ? m.sb_pos[p] : S.qpos + KM_NL, st ? m.sb_mat[p] : S.bmat, la, lb);
-          far = capbox_far(la, lb, r, st ? m.sb_size[p] : m.fb_size);
+          capbox_local(A, B, st ? sb_pos[p] : S.qpos + KM_NL, st ? sb_mat[p] : S.bmat, la, lb);
+          far = capbox_far(la, lb, r, st ? sb_size[p] : m.fb_size);
         }
         const bool valid = KP_TYPE(m.rp[p * KW + lane]) == KP_CAP_BOX;
         if (valid) { if (far) farbits |= 1 << p; else nearbits |= 1 << p; }
@@ -1848,11 +1853,11 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
           if (i < ntot) {
             const int e = S.nlist[i] & 0x3fff, x = m.rp[e], a = KP_A(x), b = KP_B(x);
             const bool st = b < m.nsbox;
-            const float* bsz = st ? m.sb_size[b] : m.fb_size;
+            const float* bsz = st ? sb_size[b] : m.fb_size;
             // (the list holds exactly the pairs that failed the far test: straight to the near path)
             float la[3], lb[3], nf[3];
             CapBoxOut c;
-            capbox_local(S.capA[a], S.capB[a], st ? m.sb_pos[b] : S.qpos + KM_NL, st ? m.sb_mat[b] : S.bmat, la, lb);
+            capbox_local(S.capA[a], S.capB[a], st ? sb_pos[b] : S.qpos + KM_NL, st ? sb_mat[b] : S.bmat, la, lb);
             const int nout = capsule_box_near<true, false>(la, lb, m.cap_r[a], bsz, c, nf);
 #pragma unroll
             for (int k = 0; k < 3; ++k) { R.h[k] = c.pos[0][k]; R.h[3 + k] = c.nrm[0][k]; R.h[6 + k] = c.pos[1][k]; R.h[9 + k] = c.nrm[1][k]; }
@@ -1929,8 +1934,8 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
           if (i < ntot) {
             const int e = S.nlist[i] & 0x3fff, x = m.rp[e], a = KP_A(x), b = KP_B(x);
             const bool wasfar = (S.nlist[i] >> 15) != 0, pref = ((S.nlist[i] >> 14) & 1) != 0, st = b < m.nsbox;
-            const float* bpos = st ? m.sb_pos[b] : S.qpos + KM_NL;
-            const float* bmat = st ? m.sb_mat[b] : S.bmat;
+            const float* bpos = st ? sb_pos[b] : S.qpos + KM_NL;
+            const float* bmat = st ? sb_mat[b] : S.bmat;
             const float d0 = R.f0, d1 = R.f1;
             float cc = (d0 < 0.f ? 1.f : 0.f) + (d1 < 0.f ? 1.f : 0.f);
             float* pd = io.prevd + (2 * (e / KW)) * KW + (e & (KW - 1));       // the owner's slots: pass e / KW, capsule lane e % KW
@@ -1991,10 +1996,20 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
       // world AABBs (extent_i = sum_j |R_ij| size_j); disjoint boxes cannot have an active slot
       const int a = m.bp_a[q];
       bool overlap = true;
-      for (int i = 0; i < 3; ++i) {
-        const float ea = fabsf(m.sb_mat[a][3 * i]) * m.sb_size[a][0] + fabsf(m.sb_mat[a][3 * i + 1]) * m.sb_size[a][1] + fabsf(m.sb_mat[a][3 * i + 2]) * m.sb_size[a][2];
-        const float eb = fabsf(S.bmat[3 * i]) * m.fb_size[0] + fabsf(S.bmat[3 * i + 1]) * m.fb_size[1] + fabsf(S.bmat[3 * i + 2]) * m.fb_size[2];
-        if (fabsf(bp[i] - m.sb_pos[a][i]) > ea + eb) overlap = false;
+      // (the table's rows spelled out without SCENE: a closure that captured the views kept them in local memory)
+      if constexpr (SCENE) {
+        const float* ap = scene + 4 * a; const float* am = scene + 4 * KM_MAXSBOX + 12 * a; const float* as = scene + 16 * KM_MAXSBOX + 4 * a;
+        for (int i = 0; i < 3; ++i) {
+          const float ea = fabsf(am[3 * i]) * as[0] + fabsf(am[3 * i + 1]) * as[1] + fabsf(am[3 * i + 2]) * as[2];
+          const float eb = fabsf(S.bmat[3 * i]) * m.fb_size[0] + fabsf(S.bmat[3 * i + 1]) * m.fb_size[1] + fabsf(S.bmat[3 * i + 2]) * m.fb_size[2];
+          if (fabsf(bp[i] - ap[i]) > ea + eb) overlap = false;
+        }
+      } else {
+        for (int i = 0; i < 3; ++i) {
+          const float ea = fabsf(m.sb_mat[a][3 * i]) * m.sb_size[a][0] + fabsf(m.sb_mat[a][3 * i + 1]) * m.sb_size[a][1] + fabsf(m.sb_mat[a][3 * i + 2]) * m.sb_size[a][2];
+          const float eb = fabsf(S.bmat[3 * i]) * m.fb_size[0] + fabsf(S.bmat[3 * i + 1]) * m.fb_size[1] + fabsf(S.bmat[3 * i + 2]) * m.fb_size[2];
+          if (fabsf(bp[i] - m.sb_pos[a][i]) > ea + eb) overlap = false;
+        }
       }
       return overlap;
     });
@@ -2013,8 +2028,8 @@ KFN void step_forward(Warp& W, const KModel& m, WarpSmemT<NC>& S, const StepIO& 
       } else {
         // one call site (the routine is large and inlined): geom1 is the static box, or the free box when it has the lower geom id
         const bool sw = ty == KB_BOX_BOX_SWAP;
-        box_box_warp<NC>(W, S, mine, q, sw ? bp : m.sb_pos[a], sw ? S.bmat : m.sb_mat[a], sw ? m.fb_size : m.sb_size[a],
-                         sw ? m.sb_pos[a] : bp, sw ? m.sb_mat[a] : S.bmat, sw ? m.sb_size[a] : m.fb_size);
+        box_box_warp<NC>(W, S, mine, q, sw ? bp : sb_pos[a], sw ? S.bmat : sb_mat[a], sw ? m.fb_size : sb_size[a],
+                         sw ? sb_pos[a] : bp, sw ? sb_mat[a] : S.bmat, sw ? sb_size[a] : m.fb_size);
       }
     }
   }
@@ -2250,15 +2265,21 @@ KFN void contact_outputs(Warp& W, const KModel& m, WarpSmemT<NC>& S, const Rollo
 // STATES = true: the same steps from the sample's own state rows, which it writes back after the last step; thetadot
 // may be null with T = 1 (the sample keeps its own qvel[:6], a plain mjx.step), theta is optional, no cost, no target.
 // CONTACTS (with STATES): also the contacts and constraint forces of the last step (contact_outputs).
-template <int NC, bool STATES = false, bool CONTACTS = false>
-KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const RolloutArgs& A) {
+// SCENE: the static boxes from the sample's scene record `scene` (KM_SCENE_FLOATS) and, without STATES, the snapshot
+// from the start record `start` (qpos0 | warm0 | qvel0, KM_START_FLOATS) instead of the table's.
+template <int NC, bool STATES = false, bool CONTACTS = false, bool SCENE = false>
+KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const RolloutArgs& A, const float* scene = nullptr,
+                        const float* start = nullptr) {
+  const float* qpos0 = SCENE && !STATES ? start : m.qpos0;
+  const float* warm0 = SCENE && !STATES ? start + 16 : m.warm0;
+  const float* qvel0 = SCENE && !STATES ? start + 28 : m.qvel0;
   LANES(W, R)
     if (STATES) {
       if (lane < KM_NQ) S.qpos[lane] = A.q0[lane];
       if (lane < KM_NV) { S.qvel[lane] = A.v0[lane]; S.warm[lane] = A.warm0[lane]; }
     } else {
-      if (lane < KM_NQ) S.qpos[lane] = lane < KM_NL ? A.q0[lane] : m.qpos0[lane];
-      if (lane < KM_NV) { S.qvel[lane] = lane < KM_NL ? A.v0[lane] : m.qvel0[lane]; S.warm[lane] = m.warm0[lane]; }
+      if (lane < KM_NQ) S.qpos[lane] = lane < KM_NL ? A.q0[lane] : qpos0[lane];
+      if (lane < KM_NV) { S.qvel[lane] = lane < KM_NL ? A.v0[lane] : qvel0[lane]; S.warm[lane] = warm0[lane]; }
     }
     R.tri = tri_entries(lane);
     if (lane == 0) { S.flags = 0; S.ovf = A.ovf; }
@@ -2293,7 +2314,7 @@ KFN void rollout_sample(Warp& W, const KModel& m, WarpSmemT<NC>& S, const Rollou
       io.con_key = last ? A.con_slot : nullptr;
       io.con_rec = last ? A.con_rec : nullptr;
     }
-    step_forward<NC, CONTACTS>(W, m, S, io);
+    step_forward<NC, CONTACTS, SCENE>(W, m, S, io, scene);
     PHASE(W, 12);
     // pre-step observations (mjx_planner.py:259-261) and running cost (:277-285)
     {

@@ -12,7 +12,7 @@ import ctypes as C
 
 import numpy as np
 
-from .mjcf import GEOM_BOX, GEOM_CAPSULE, GEOM_PLANE, JNT_FREE, JNT_HINGE, ModelConsts, quat_mul, quat_to_mat
+from .mjcf import GEOM_BOX, GEOM_CAPSULE, GEOM_PLANE, JNT_FREE, JNT_HINGE, ModelConsts, quat_mul, quat_normalize, quat_to_mat
 
 NL, NV, NQ, MAXCAP, MAXSBOX, MAXRPAIR, MAXBPAIR, MAXNEAR = 6, 12, 13, 12, 8, 160, 8, 96
 LANE_GROUP = 16          # lanes per sample in the rollout kernel (csrc/warp_dsl.h KW); one collider pass = 16 pair entries
@@ -51,6 +51,16 @@ class KModel(C.Structure):
     ]
 
 
+# The records a rollout may take per call instead of the table's blocks (csrc/kmodel.h): a scene record is the
+# sb_pos | sb_mat | sb_size block, a start record the qpos0 | warm0 | qvel0 block, in floats.
+SCENE_FLOATS = MAXSBOX * (4 + 12 + 4)
+START_FLOATS = 16 + 12 + 12
+assert KModel.sb_mat.offset == KModel.sb_pos.offset + 4 * 4 * MAXSBOX and KModel.sb_size.offset == KModel.sb_pos.offset + 4 * 16 * MAXSBOX
+assert KModel.fb_size.offset == KModel.sb_pos.offset + 4 * SCENE_FLOATS
+assert KModel.warm0.offset == KModel.qpos0.offset + 4 * 16 and KModel.qvel0.offset == KModel.qpos0.offset + 4 * 28
+assert C.sizeof(KModel) == KModel.qpos0.offset + 4 * START_FLOATS
+
+
 def _set(dst, src):
     a = np.asarray(src, dtype=np.float64)
     flat = np.ctypeslib.as_array(dst).reshape(-1)
@@ -78,6 +88,108 @@ def _static_pose(mc, body):
         pos = pos + quat_to_mat(quat) @ mc.body_pos[b]
         quat = quat_mul(quat, mc.body_quat[b])
     return pos, quat
+
+
+def _quat_to_mat_n(q):
+    """mjcf.quat_to_mat over [N, 4] -> [N, 3, 3], the same float64 arithmetic per row."""
+    w, x, y, z = q[:, 0], q[:, 1], q[:, 2], q[:, 3]
+    return np.stack([
+        np.stack([w * w + x * x - y * y - z * z, 2 * (x * y - w * z), 2 * (x * z + w * y)], -1),
+        np.stack([2 * (x * y + w * z), w * w - x * x + y * y - z * z, 2 * (y * z - w * x)], -1),
+        np.stack([2 * (x * z - w * y), 2 * (y * z + w * x), w * w - x * x - y * y + z * z], -1)], -2)
+
+
+def _quat_mul_n(a, b):
+    """mjcf.quat_mul over [N, 4] (b may be [4])."""
+    b = np.broadcast_to(b, a.shape)
+    aw, ax, ay, az = a[:, 0], a[:, 1], a[:, 2], a[:, 3]
+    bw, bx, by, bz = b[:, 0], b[:, 1], b[:, 2], b[:, 3]
+    return np.stack([aw * bw - ax * bx - ay * by - az * bz, aw * bx + ax * bw + ay * bz - az * by,
+                     aw * by - ax * bz + ay * bw + az * bx, aw * bz + ax * by - ay * bx + az * bw], -1)
+
+
+def _mat_vec_n(R, v):
+    """R [N, 3, 3] @ v [3], one row at a time in a fixed order (the result of a row does not depend on N)."""
+    return R[:, :, 0] * v[0] + R[:, :, 1] * v[1] + R[:, :, 2] * v[2]
+
+
+def static_box_fields(body_pos, body_quat, geom_pos, geom_quat, size):
+    """World pose of the body carrying a static box geom -> that box's rows of the scene record, for N poses at once, in
+    float64: body_pos [N, 3], body_quat [N, 4] (unit), the geom's pose in the body and its half sizes [3] -> sb_pos [N, 4],
+    sb_mat [N, 12], sb_size [N, 4] (csrc/kmodel.h).  An axis-aligned box (frame = signed permutation of the world axes, in
+    float32) gets its half sizes along the world axes in sb_mat[9:12] and the flag sb_size[3] = 1: its far-field test runs
+    on world coordinates with the permuted half sizes, no change of frame (rollout_core.h N1)."""
+    body_pos, body_quat = np.asarray(body_pos, dtype=np.float64), np.asarray(body_quat, dtype=np.float64)
+    geom_pos, size = np.asarray(geom_pos, dtype=np.float64), np.asarray(size, dtype=np.float64)
+    n = body_pos.shape[0]
+    gp = body_pos + _mat_vec_n(_quat_to_mat_n(body_quat), geom_pos)
+    gm = _quat_to_mat_n(_quat_mul_n(body_quat, np.asarray(geom_quat, dtype=np.float64)))
+    sb_pos, sb_mat, sb_size = np.zeros((n, 4)), np.zeros((n, 12)), np.zeros((n, 4))
+    sb_pos[:, :3] = gp
+    sb_mat[:, :9] = gm.reshape(n, 9)
+    sb_size[:, :3] = size
+    gm32 = gm.astype(np.float32)
+    aligned = np.all((gm32 == 0) | (np.abs(gm32) == 1), axis=(1, 2))
+    sb_mat[aligned, 9:12] = _mat_vec_n(np.abs(gm32[aligned].astype(np.float64)), size)
+    sb_size[aligned, 3] = 1.0
+    return sb_pos, sb_mat, sb_size
+
+
+def _static_box_geoms(mc):
+    """Collision box geoms on static bodies, in the kernel's static-box order (sb_* rows)."""
+    free = {int(mc.jnt_body[j]) for j in range(mc.njnt) if mc.jnt_type[j] == JNT_FREE}
+    return [g for g in range(mc.ngeom) if mc.geom_collides[g] and int(mc.geom_type[g]) == GEOM_BOX and int(mc.geom_body[g]) not in free
+            and int(mc.body_weldid[mc.geom_body[g]]) == 0]
+
+
+def movable_bodies(mc):
+    """Names of the bodies a scene record can move: static children of the world that carry static box geoms."""
+    bodies = sorted({int(mc.geom_body[g]) for g in _static_box_geoms(mc)})
+    # a body whose static descendants carry boxes too is not movable: a record moves only the boxes of the named body
+    nested = set()
+    for b in bodies:
+        c = int(mc.body_parent[b])
+        while c != 0:
+            nested.add(c)
+            c = int(mc.body_parent[c])
+    return [mc.body_names[b] for b in bodies if mc.body_parent[b] == 0 and mc.body_jntadr[b] < 0 and b not in nested]
+
+
+def scene_records(mc, body_pose):
+    """Scene records (csrc/kmodel.h, SCENE_FLOATS float32) with bodies moved: body_pose = {name: (pos [3], quat [4])}, either
+    array with a leading [N] allowed (broadcast against the others).  Bodies not named keep their model pose, so
+    ``scene_records(mc, {})`` is the table's own block.  Quaternions are normalised as the model compiler does.  Returns [N,
+    SCENE_FLOATS], N = 1 without a leading dimension.  ValueError for a body that is not movable, a non-finite pose or a
+    zero quaternion."""
+    movable = movable_bodies(mc)
+    poses, n = {}, 1
+    for name, pq in body_pose.items():
+        if name not in movable:
+            raise ValueError(f"{name!r} is not a movable body; the movable bodies are {movable}")
+        pos, quat = (np.asarray(a, dtype=np.float64) for a in pq)
+        if pos.shape[-1:] != (3,) or quat.shape[-1:] != (4,) or pos.ndim > 2 or quat.ndim > 2:
+            raise ValueError(f"{name}: pose must be pos [3] or [N, 3] and quat [4] or [N, 4], got {pos.shape} and {quat.shape}")
+        if not (np.all(np.isfinite(pos)) and np.all(np.isfinite(quat))):
+            raise ValueError(f"{name}: non-finite pose")
+        pos, quat = pos.reshape(-1, 3), quat.reshape(-1, 4)
+        if np.any(np.all(quat == 0, axis=1)):
+            raise ValueError(f"{name}: zero quaternion")
+        quat = np.array([quat_normalize(q) for q in quat])
+        poses[mc.body_id(name)] = (pos, quat)
+        n = max(n, pos.shape[0], quat.shape[0])
+    for b, (pos, quat) in poses.items():
+        if pos.shape[0] not in (1, n) or quat.shape[0] not in (1, n):
+            raise ValueError(f"{mc.body_names[b]}: leading dimensions of the poses disagree (N = {n})")
+        poses[b] = (np.broadcast_to(pos, (n, 3)), np.broadcast_to(quat, (n, 4)))
+    rec = np.zeros((n, SCENE_FLOATS), dtype=np.float32)
+    view = (rec[:, :4 * MAXSBOX].reshape(n, MAXSBOX, 4), rec[:, 4 * MAXSBOX:16 * MAXSBOX].reshape(n, MAXSBOX, 12),
+            rec[:, 16 * MAXSBOX:].reshape(n, MAXSBOX, 4))
+    for k, g in enumerate(_static_box_geoms(mc)):
+        b = int(mc.geom_body[g])
+        pos, quat = poses[b] if b in poses else (np.broadcast_to(p, (n, len(p))) for p in _static_pose(mc, b))
+        for dst, f in zip(view, static_box_fields(pos, quat, mc.geom_pos[g], mc.geom_quat[g], mc.geom_size[g])):
+            dst[:, k] = f
+    return rec
 
 
 def build_kmodel(mc: ModelConsts, timestep: float, robot_geom_names=None, tcp_site="tcp",
@@ -230,15 +342,10 @@ def build_kmodel(mc: ModelConsts, timestep: float, robot_geom_names=None, tcp_si
                 if k >= MAXSBOX:
                     raise NotImplementedError("too many static boxes")
                 sboxes[g] = k
-                m.sb_pos[k][:3] = list(gp)
-                m.sb_mat[k][:9] = list(gm.reshape(-1))
-                m.sb_size[k][:3] = list(mc.geom_size[g])
-                # axis-aligned box (frame = signed permutation of the world axes, in float32): its far-field test
-                # runs on world coordinates with the permuted half sizes, no change of frame (rollout_core.h N1)
-                gm32 = gm.astype(np.float32)
-                if np.all((gm32 == 0) | (np.abs(gm32) == 1)):
-                    m.sb_mat[k][9:12] = list(np.abs(gm32.astype(np.float64)) @ np.asarray(mc.geom_size[g], dtype=np.float64))
-                    m.sb_size[k][3] = 1.0
+                sp, sm, ss = static_box_fields(pos[None], quat[None], mc.geom_pos[g], mc.geom_quat[g], mc.geom_size[g])
+                m.sb_pos[k][:] = list(sp[0])
+                m.sb_mat[k][:] = list(sm[0])
+                m.sb_size[k][:] = list(ss[0])
             else:
                 raise NotImplementedError("static geoms must be planes or boxes")
     m.ncap, m.nsbox = len(caps), len(sboxes)

@@ -25,6 +25,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .kmodel import SCENE_FLOATS, scene_records
 from .planner import cem_planner
 
 
@@ -58,6 +59,19 @@ class PlantSim:
         self._td, self._q0, self._v0 = f(6).reshape(1, 6), f(6), f(6)
         self._tp, self._tr = f(3), torch.tensor([1.0, 0, 0, 0], device=dev)
         self._theta, self._cost4, self._qacc = f(6).reshape(1, 6), f(4).reshape(1, 4), f(12).reshape(1, 1, 12)
+        self._moves = {}
+        self.scene = scene_records(self.mc, {})[0]           # the plant's scene record (its table's static box block)
+
+    def set_body_pose(self, name, pos, quat):
+        """Move a static body of the plant (one of ``cem.scene_bodies``): rewrites the static box block of the plant's own
+        table with the derivation of the model table (kmodel.scene_records); ``self.scene`` is the new scene record."""
+        self._moves[name] = (np.asarray(pos, dtype=np.float64), np.asarray(quat, dtype=np.float64))
+        self.scene = scene_records(self.mc, self._moves)[0]
+        C.memmove(C.addressof(self._km) + type(self._km).sb_pos.offset, self.scene.ctypes.data, 4 * SCENE_FLOATS)
+
+    def state(self):
+        """The plant's state as ``compute_cem(state=...)`` takes it."""
+        return dict(qpos=self.qpos.copy(), qvel=self.qvel.copy(), qacc_warmstart=self.warm.copy())
 
     def close(self):
         if self._h:
@@ -101,7 +115,11 @@ def run_cem_planner(num_dof=None, num_batch=None, num_steps=None, maxiter_cem=No
                     w_col=None, num_elite=None, timestep=None, initial_qpos=None, target_names=None, show_viewer=None,
                     cam_distance=None, show_contact_points=None, position_threshold=None, rotation_threshold=None, save_data=None,
                     data_dir=None, stop_at_final_target=None, *, max_ticks=200, realtime=False, verbose=True, device=None,
-                    contact_exclude=None):
+                    contact_exclude=None, plan_from_plant=False, body_moves=None):
+    """``body_moves`` = {tick: {body name: (pos, quat)}} moves static bodies of the plant at the start of those ticks
+    (``PlantSim.set_body_pose``).  ``plan_from_plant=True`` plans every tick in the plant's scene from its full state
+    (``compute_cem(scene=..., state=...)``): the free box where the plant has it, moved obstacles where they are.  With the
+    default the planner plans in the model's scene from its snapshot, as the reference does."""
     if show_viewer:
         raise NotImplementedError("no MuJoCo viewer in this build: call with show_viewer=False (headless loop, max_ticks)")
     if save_data:
@@ -129,12 +147,15 @@ def run_cem_planner(num_dof=None, num_batch=None, num_steps=None, maxiter_cem=No
 
     thetadot = np.zeros(num_dof)
     cost_g_list, cost_list, cost_r_list, cost_c_list, thetadot_list, theta_list, tick_ms = [], [], [], [], [], [], []
-    dist_list, switch_ticks = [], []
+    dist_list, switch_ticks, plant_states = [], [], []
     target_idx = 0
     current_target = target_names[target_idx]
     reached_final = False
     for _tick in range(max_ticks):
         start_time = time.time()
+        for name, (pos, quat) in (body_moves or {}).get(_tick, {}).items():
+            plant.set_body_pose(name, pos, quat)
+        plant_kw = dict(scene=plant.scene, state=plant.state()) if plan_from_plant else {}
         if current_target != "home":
             target_pos = model.body(name=current_target).pos
             target_rot = model.body(name=current_target).quat
@@ -144,11 +165,12 @@ def run_cem_planner(num_dof=None, num_batch=None, num_steps=None, maxiter_cem=No
             model.body(name="target_0").pos[:] = data.site_xpos[cem.tcp_id]
             model.body(name="target_0").quat[:] = data.xquat[cem.hande_id]
         cost, best_cost_g, best_cost_r, best_cost_c, best_vels, best_traj, xi_mean, _, _ = cem.compute_cem(
-            xi_mean, data.qpos[:num_dof], data.qvel[:num_dof], data.qacc[:num_dof], target_pos, target_rot)
+            xi_mean, data.qpos[:num_dof], data.qvel[:num_dof], data.qacc[:num_dof], target_pos, target_rot, **plant_kw)
         plan_ms = (time.time() - start_time) * 1e3
         if not reached_final:
             thetadot = np.mean(best_vels[1:num_steps - 2], axis=0)           # mpc_planner.py:178
         plant.step(thetadot)
+        plant_states.append(plant.state())
         data.qpos[:], data.qvel[:], data.qacc[:] = plant.qpos, plant.qvel, plant.qacc
         data.forward()
         current_cost_g = np.linalg.norm(data.site_xpos[cem.tcp_id] - target_pos)
@@ -201,6 +223,6 @@ def run_cem_planner(num_dof=None, num_batch=None, num_steps=None, maxiter_cem=No
         np.savetxt(f'{data_dir}/cost_c.csv', cost_c_list, delimiter=",")
     return {'cost_g': cost_g_list, 'cost_r': cost_r_list, 'cost_c': cost_c_list, 'cost': cost_list, 'thetadot': thetadot_list,
             'theta': theta_list, 'tick_ms': tick_ms, 'final_target': current_target, 'reached_final': reached_final,
-            'dist': dist_list, 'switch_ticks': switch_ticks, 'cem': cem,
+            'dist': dist_list, 'switch_ticks': switch_ticks, 'cem': cem, 'plant_states': plant_states, 'plant_scene': plant.scene,
             'last': dict(xi_mean=xi_mean, qpos=data.qpos.copy(), qvel=data.qvel.copy(), qacc=data.qacc.copy(),
                          target_pos=np.array(target_pos), target_rot=np.array(target_rot))}

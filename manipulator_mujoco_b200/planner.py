@@ -38,7 +38,7 @@ import torch
 
 from . import _lib, jax_prng, parallel
 from .bernstein import bernstein_coeff_ordern_new
-from .kmodel import build_kmodel
+from .kmodel import SCENE_FLOATS, START_FLOATS, build_kmodel, movable_bodies, scene_records
 from .mjcf import ModelConsts, exclude_body_pairs, host_kinematics, load_model, quat_mul, quat_normalize
 
 _VP = C.c_void_p
@@ -215,6 +215,7 @@ class cem_planner:
         parallel.check_index_range(self.num_batch)
         self._ws = {}
         self._iter_out = None
+        self._iter_rec = None
         self._key_seen, self._key_tuple = None, None
         self._graph, self._graph_out, self._graph_key, self._eager_ticks = None, None, None, 0
         self.overflow_samples, self._warned_overflow = 0, False
@@ -458,7 +459,8 @@ class cem_planner:
         """mjx_planner.py:234-249 -> primal_sol [B, nvar]."""
         return self._project(xi_samples, state_term, False)[0]
 
-    def _rollout(self, thetadot, init_pos, init_vel, target_pos, target_rot, dumps, out_theta=None):
+    def _rollout(self, thetadot, init_pos, init_vel, target_pos, target_rot, dumps, out_theta=None, scene=None, start=None):
+        """scene: device scene record(s) [160] or [B, 160], start: device start record [40]; None = the handle's own."""
         td = self._t(thetadot)
         B, T = td.shape[0], self.num
         dev = self.device
@@ -472,20 +474,63 @@ class cem_planner:
         # keep every converted argument referenced until the launch is enqueued (a temporary tensor
         # would hand its storage to the next allocation before the kernel reads it)
         q0, v0, tp, tr = self._t(init_pos), self._t(init_vel), self._t(target_pos), self._t(target_rot)
-        _lib.check(self._lib.cemk_rollout_cost(
+        scene, stride = self._scene_tensor(scene, B)
+        _lib.check(self._lib.cemk_rollout_cost_scene(
             self._h, B, T, _ptr(td), _ptr(q0), _ptr(v0), _ptr(tp), _ptr(tr), float(w['w_pos']), float(w['w_rot']),
             float(w['w_col']), _ptr(theta), _ptr(cost4), _ptr(eef_pos), _ptr(eef_rot), _ptr(collision), None, _ptr(flags),
-            self._stream()), self._lib)
-        self._keep = (td, q0, v0, tp, tr)
+            _ptr(scene), stride, _ptr(start), self._stream()), self._lib)
+        self._keep = (td, q0, v0, tp, tr, scene, start)
         return theta, cost4, eef_pos, eef_rot, collision
 
-    def compute_rollout_batch(self, thetadot, init_pos, init_vel):
-        """mjx_planner.py:123,266-274 -> theta [B,6T], eef_pos [B,T,3], eef_rot [B,T,4], collision [B,T,187]."""
+    def compute_rollout_batch(self, thetadot, init_pos, init_vel, *, scene=None, state=None):
+        """mjx_planner.py:123,266-274 -> theta [B,6T], eef_pos [B,T,3], eef_rot [B,T,4], collision [B,T,187].
+        ``scene`` (``make_scene``, [160] shared or [B, 160]) and ``state`` (as in ``compute_cem``) replace the model's static
+        box poses and the free box's start state for this call."""
         self._require_rollout_dof("compute_rollout_batch")
         tp = torch.zeros(3, device=self.device)
         tr = torch.tensor([1.0, 0, 0, 0], device=self.device)
-        theta, _c, eef_pos, eef_rot, collision = self._rollout(thetadot, init_pos, init_vel, tp, tr, True)
+        start = None if state is None else self._t(self.start_record(state))
+        theta, _c, eef_pos, eef_rot, collision = self._rollout(thetadot, init_pos, init_vel, tp, tr, True, scene=scene, start=start)
         return theta, eef_pos, eef_rot, collision
+
+    # ------------------------------------------------------------------ scenes and start states given per call
+    @property
+    def scene_bodies(self):
+        """Names of the bodies ``make_scene`` can move (static children of the world carrying boxes).  Read-only."""
+        return tuple(movable_bodies(self._mc))
+
+    def make_scene(self, body_pose):
+        """Scene record for ``compute_cem`` / ``compute_rollout_batch`` / ``step_batch``: ``body_pose`` = {name: (pos [3],
+        quat [4])}, a leading [N] allowed on the arrays.  Bodies not named keep their model pose; the floor, box sizes,
+        robot and topology are the model's.  Returns a CUDA tensor [160], or [N, 160] with a leading dimension."""
+        batched = any(np.ndim(a) > 1 for pq in body_pose.values() for a in pq)
+        rec = scene_records(self._mc, body_pose)
+        t = torch.as_tensor(rec, device=self.device)
+        return t if batched else t[0]
+
+    @staticmethod
+    def start_record(state):
+        """Start record [40] (float32, host) of a state dict qpos [13], qvel [12], qacc_warmstart [12] (``mjx_data``,
+        ``jit_step``'s input and output, one row of ``step_batch``'s outputs): the rollouts start the free box and the warm
+        start from it."""
+        f = lambda k, n: np.asarray(state[k].detach().cpu() if torch.is_tensor(state[k]) else state[k], dtype=np.float32).reshape(-1)
+        qpos, qvel, warm = f("qpos", 13), f("qvel", 12), f("qacc_warmstart", 12)
+        if qpos.size != 13 or qvel.size != 12 or warm.size != 12:
+            raise ValueError(f"state needs qpos [13], qvel [12], qacc_warmstart [12], got {qpos.size}, {qvel.size}, {warm.size}")
+        rec = np.zeros(START_FLOATS, dtype=np.float32)
+        rec[:13], rec[16:28], rec[28:40] = qpos, warm, qvel
+        return rec
+
+    def _scene_tensor(self, scene, n):
+        """(device scene tensor, stride in floats) of a scene argument [160] (shared) or [n, 160]; (None, 0) for None."""
+        if scene is None:
+            return None, 0
+        t = self._t(scene)
+        if t.shape == (SCENE_FLOATS,):
+            return t, 0
+        if t.shape == (n, SCENE_FLOATS):
+            return t, SCENE_FLOATS
+        raise ValueError(f"scene must be [{SCENE_FLOATS}] or [{n}, {SCENE_FLOATS}] (make_scene), got {tuple(t.shape)}")
 
     @property
     def contact_slot_geoms(self):
@@ -498,7 +543,7 @@ class cem_planner:
         g.flags.writeable = False
         return g
 
-    def step_batch(self, qpos, qvel, qacc_warmstart, thetadot=None, contacts=False):
+    def step_batch(self, qpos, qvel, qacc_warmstart, thetadot=None, contacts=False, scene=None):
         """``jax.vmap(jit_step, in_axes=(None, 0))``: N environments, each stepped from its own state in one launch
         (``cemk_step_states``); the planner's model snapshot is not used or changed.  qpos [N, 13], qvel [N, 12],
         qacc_warmstart [N, 12] (numpy or torch).  ``thetadot`` [N, 6T] (dof-major, the rollout's layout) chains T steps with
@@ -511,7 +556,10 @@ class cem_planner:
         slot and padded with slot -1 and zeros: contact_slot [N, 48] (int32; geoms in ``contact_slot_geoms``), contact_dist
         [N, 48], contact_pos [N, 48, 3], contact_normal [N, 48, 3] (first row of the contact frame) and contact_force
         [N, 48, 3] (normal, tangent 1, tangent 2 in the contact frame, mju_decodePyramid of the four pyramid rows).  The
-        state outputs are the same bits as with ``contacts=False``."""
+        state outputs are the same bits as with ``contacts=False``.
+
+        ``scene`` (``make_scene``): [160], one scene for all environments, or [N, 160], one per environment
+        (``cemk_step_states_scene``); None = the model's own."""
         self._require_rollout_dof("step_batch")
         qp, qv, wm = self._t(qpos), self._t(qvel), self._t(qacc_warmstart)
         if qp.dim() != 2 or qp.shape[1] != 13 or qp.shape[0] == 0:
@@ -531,9 +579,21 @@ class cem_planner:
             # the library grows its rollout scratch to N samples and frees the old one, which the captured tick points at
             torch.cuda.current_stream(dev).synchronize()
             self._graph, self._graph_out, self._eager_ticks = None, None, 0
+        scene, stride = self._scene_tensor(scene, N)
         qpos_out, qvel_out, warm_out = torch.empty(N, 13, device=dev), torch.empty(N, 12, device=dev), torch.empty(N, 12, device=dev)
         flags = torch.empty(N, dtype=torch.int32, device=dev)
-        if not contacts:
+        if scene is not None:
+            qfrc = ncon = slot = rec = None
+            if contacts:
+                if self._key_slot_dev is None:
+                    self._key_slot_dev = torch.as_tensor(self._key_slot, dtype=torch.int32, device=dev)
+                qfrc, ncon = torch.empty(N, 12, device=dev), torch.empty(N, dtype=torch.int32, device=dev)
+                slot, rec = torch.empty(N, 48, dtype=torch.int32, device=dev), torch.empty(N, 48, 12, device=dev)
+            _lib.check(self._lib.cemk_step_states_scene(
+                self._h, N, T, _ptr(qp), _ptr(qv), _ptr(wm), _ptr(td), _ptr(qpos_out), _ptr(qvel_out), _ptr(warm_out), _ptr(theta),
+                None, None, None, None, _ptr(flags), _ptr(self._key_slot_dev if contacts else None), _ptr(qfrc), _ptr(ncon), _ptr(slot),
+                _ptr(rec), _ptr(scene), stride, self._stream()), self._lib)
+        elif not contacts:
             _lib.check(self._lib.cemk_step_states(self._h, N, T, _ptr(qp), _ptr(qv), _ptr(wm), _ptr(td), _ptr(qpos_out), _ptr(qvel_out),
                                                   _ptr(warm_out), _ptr(theta), None, None, None, None, _ptr(flags), self._stream()), self._lib)
         else:
@@ -545,7 +605,7 @@ class cem_planner:
                 self._h, N, T, _ptr(qp), _ptr(qv), _ptr(wm), _ptr(td), _ptr(qpos_out), _ptr(qvel_out), _ptr(warm_out), _ptr(theta),
                 None, None, None, None, _ptr(flags), _ptr(self._key_slot_dev), _ptr(qfrc), _ptr(ncon), _ptr(slot), _ptr(rec),
                 self._stream()), self._lib)
-        self._keep_sb = (qp, qv, wm, td)
+        self._keep_sb = (qp, qv, wm, td, scene)
         out = dict(qpos=qpos_out, qvel=qvel_out, qacc=warm_out.clone(), qacc_warmstart=warm_out, overflow=(flags & 1).bool())
         if theta is not None:
             out["theta"] = theta
@@ -640,7 +700,8 @@ class cem_planner:
         xi_filtered, thetadot = self._project(xi_samples, state_term, True, out_thetadot=out_td)
         tp = self._t(target_pos).reshape(-1, 3)[0]
         tr = self._t(target_rot).reshape(-1, 4)[0]
-        theta, cost4, _, _, _ = self._rollout(thetadot, init_pos, init_vel, tp, tr, False, out_theta=out_th)
+        scene, start = self._iter_rec if self._iter_rec is not None else (None, None)      # compute_cem's records
+        theta, cost4, _, _, _ = self._rollout(thetadot, init_pos, init_vel, tp, tr, False, out_theta=out_th, scene=scene, start=start)
         xi_ellite, cost_ellite, gidx = self._select_elites(cost4, xi_samples)
         xi_mean, xi_cov = self.compute_mean_cov(cost_ellite, xi_mean_prev, xi_cov_prev, xi_ellite)
         self._last_elite = (cost_ellite, gidx)
@@ -648,10 +709,11 @@ class cem_planner:
         carry = (init_pos, init_vel, target_pos, target_rot, xi_mean, xi_cov, key, state_term)
         return carry, (cost4[:, 0], cost4[:, 1], cost4[:, 2], cost4[:, 3], thetadot, theta)
 
-    def _cem_device(self, pin, pout):
+    def _cem_device(self, pin, pout, has_scene=False, has_state=False):
         """Everything a planning tick does on the device: H2D of the packed inputs, maxiter_cem
         iterations, best-sample extraction, D2H of the packed results (stream-ordered, no sync).
-        pin = [xi_mean | q0 v0 a0 0 0 (the state row, :374-384) | target_pos | target_rot]."""
+        pin = [xi_mean | q0 v0 a0 0 0 (the state row, :374-384) | target_pos | target_rot | scene record, if any |
+        start record, if any]."""
         dev = self.device
         Bl, T, nd, nv, m = self.num_batch_local, self.num, self.num_dof, self.nvar, self.maxiter_cem
         d_in = self._buf("d_in", (pin.numel(),))
@@ -663,6 +725,10 @@ class cem_planner:
         xi_cov = self._const("cov0", lambda: 10 * torch.eye(nv, device=dev))               # :386 (read-only)
         key = self._split0(self.key)                                                       # :388
         carry = (q0, v0, tp, tr, xi_mean_d, xi_cov, key, state_term)
+        o = nv + 37
+        scene_d = d_in[o:o + SCENE_FLOATS] if has_scene else None
+        o += SCENE_FLOATS if has_scene else 0
+        start_d = d_in[o:o + START_FLOATS] if has_state else None
         both = torch.empty(2, m, Bl, nd * T, device=dev)
         thetadot_all, theta_all = both[0], both[1]
         out_d = self._buf("tick_out", (pout.numel(),))
@@ -670,10 +736,11 @@ class cem_planner:
         flags = self._buf("flags", (Bl,), torch.int32)
         for i in range(m):                                                                 # :390-392
             self._iter_out = (thetadot_all[i], theta_all[i])
+            self._iter_rec = (scene_d, start_d)
             try:
                 carry, out = self.cem_iter(carry, None)
             finally:
-                self._iter_out = None
+                self._iter_out = self._iter_rec = None
             cost_e, gidx = self._last_elite
             # min over the (global) batch, overflow count, and (last iteration, :395-402) the best sample = head of the
             # (merged) sorted list and the new mean, straight into the packed result
@@ -689,20 +756,35 @@ class cem_planner:
         return thetadot_all, theta_all
 
     def compute_cem(self, xi_mean, init_pos=np.array([1.5, -1.8, 1.75, -1.25, -1.6, 0]), init_vel=np.zeros(6),
-                    init_acc=np.zeros(6), target_pos=np.zeros(3), target_rot=np.zeros(4)):
+                    init_acc=np.zeros(6), target_pos=np.zeros(3), target_rot=np.zeros(4), *, scene=None, state=None):
+        """mjx_planner.py:366-406.  ``scene``: a scene record [160] (``make_scene``; host or device) the rollouts of this tick
+        run against instead of the model's static box poses.  ``state``: dict qpos [13], qvel [12], qacc_warmstart [12]
+        (``mjx_data``, ``jit_step``, a row of ``step_batch``) the rollouts start the free box and the warm start from; the arm
+        still starts from init_pos / init_vel.  Nothing is kept: a call without them plans in the model's own scene."""
         self._require_rollout_dof("compute_cem")
         dev = self.device
         Bl, T, nd, nv = self.num_batch_local, self.num, self.num_dof, self.nvar
-        # one packed host->device copy for the per-tick inputs
-        pin = self._ws.get("pin_in")
+        has_scene, has_state = scene is not None, state is not None
+        # one packed host->device copy for the per-tick inputs, records included (a graph replays them without re-capture)
+        pkey = "pin_in" if not (has_scene or has_state) else ("pin_in", has_scene, has_state)
+        pin = self._ws.get(pkey)
         if pin is None:
-            pin = torch.zeros(nv + 37, dtype=torch.float32).pin_memory()
-            self._ws["pin_in"] = pin
-            self._ws["pin_in_np"] = pin.numpy()                       # a view: written in place every tick
-        host = self._ws["pin_in_np"]
+            pin = torch.zeros(nv + 37 + (SCENE_FLOATS if has_scene else 0) + (START_FLOATS if has_state else 0), dtype=torch.float32).pin_memory()
+            self._ws[pkey] = pin
+            self._ws[("np", pkey)] = pin.numpy()                      # a view: written in place every tick
+        host = self._ws[("np", pkey)]
         host[:nv] = np.asarray(xi_mean.detach().cpu() if torch.is_tensor(xi_mean) else xi_mean, dtype=np.float32).reshape(-1)
         host[nv:nv + 6], host[nv + 6:nv + 12], host[nv + 12:nv + 18] = np.asarray(init_pos).reshape(-1), np.asarray(init_vel).reshape(-1), np.asarray(init_acc).reshape(-1)
         host[nv + 30:nv + 33], host[nv + 33:nv + 37] = np.asarray(target_pos).reshape(-1), np.asarray(target_rot).reshape(-1)
+        o = nv + 37
+        if has_scene:
+            rec = np.asarray(scene.detach().cpu() if torch.is_tensor(scene) else scene, dtype=np.float32)
+            if rec.shape != (SCENE_FLOATS,):
+                raise ValueError(f"scene must be one scene record [{SCENE_FLOATS}] (make_scene), got {rec.shape}")
+            host[o:o + SCENE_FLOATS] = rec
+            o += SCENE_FLOATS
+        if has_state:
+            host[o:o + START_FLOATS] = self.start_record(state)
         m = self.maxiter_cem
         nout = m + 2 * nd * T + 3 + self.nvar + 1
         # The device side of a tick is a fixed sequence of launches on fixed buffers: after two eager
@@ -715,7 +797,7 @@ class cem_planner:
         if self._key_seen is not self.key:                              # (the reference never reassigns its key)
             self._key_seen, self._key_tuple = self.key, tuple(int(x) for x in jax_prng.as_key(self.key))
         gkey = (m, int(self.maxiter_projection), float(w['w_pos']), float(w['w_rot']), float(w['w_col']),
-                self._key_tuple, self._partitionable, T, Bl, int(self.ellite_num), nv)
+                self._key_tuple, self._partitionable, T, Bl, int(self.ellite_num), nv, has_scene, has_state)
         if self._graph is not None and gkey != self._graph_key:
             torch.cuda.current_stream(dev).synchronize()
             self._graph, self._graph_out, self._eager_ticks = None, None, 0
@@ -731,12 +813,12 @@ class cem_planner:
             g = torch.cuda.CUDAGraph()
             # thread_local: NCCL's watchdog thread polls events while this thread captures
             with torch.cuda.graph(g, capture_error_mode="thread_local" if self.world > 1 else "global"):
-                out = self._cem_device(pin, pout)
+                out = self._cem_device(pin, pout, has_scene, has_state)
             self._graph, self._graph_out, self._graph_key = g, out, gkey
             g.replay()
             thetadot_all, theta_all = out
         else:
-            thetadot_all, theta_all = self._cem_device(pin, pout)
+            thetadot_all, theta_all = self._cem_device(pin, pout, has_scene, has_state)
             self._eager_ticks += 1
         torch.cuda.current_stream(dev).synchronize()
         res = pout.numpy().copy()
